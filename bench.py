@@ -6,6 +6,7 @@ score + traceback (boss -V/-A) for every pair of the batch.  Metric (BASELINE.js
 updates per second, in GCUPS, summed over both sweeps and over all ranks; pairs/s beside it.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--pairs P] [--len L] [--impl reference] [--no-configs]
+                  [--dump-outputs DIR]
 
 N > 1: launched by torchrun, one rank per GPU; every rank processes its own P pairs (weak scaling,
 no data-path collective; the E-step's count all-reduce is timed separately as "em").  Times are
@@ -21,6 +22,9 @@ Beside the headline line's own keys the JSON carries
 
 --impl reference times the reference's own CPU implementation (oracle/_ref/refdrv, the unmodified
 reference sources; falls back to the C restatement if that binary is absent) on the host cores.
+
+--dump-outputs DIR writes what the last timed step computed on rank 0 as float64 .npy files (see dump_outputs), so
+that two builds can be compared output for output: the inputs depend on the arguments only.
 """
 from __future__ import annotations
 
@@ -282,7 +286,12 @@ def main():
     ap.add_argument("--cfg3-pairs", type=int, default=100000)
     ap.add_argument("--cfg4-pairs", type=int, default=1000)
     ap.add_argument("--cfg5-reads", type=int, default=131072)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results here as .npy files")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm keeps no results")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -464,9 +473,42 @@ def main():
             out["cpu_baseline"] = {"value": g, "unit": UNIT, "cores": threads, "kind": kind, "seconds": secs,
                                    "sample": "%d of the same synthetic %dx%d pairs, Forward (rolling) + Viterbi with traceback, %d threads"
                                              % (n, args.len, args.len, threads)}
+        if args.dump_outputs:      # the paths of the last timed step are still held by its batch
+            dump_outputs(args.dump_outputs, ll, sc, plen, *capi.viterbi_paths(batch, plen))
         print(json.dumps(out))
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_LIMIT = 60 << 20      # bytes of array data: with the .npy headers the files stay under 64 MB
+DUMP_PATHS = 256           # pairs whose Viterbi paths are written
+
+
+def dump_outputs(out_dir: str, ll, sc, plen, trans, off):
+    """Write the headline step's results to out_dir as float64 .npy files:
+      pairs, forward_loglike, viterbi_score, viterbi_path_length   per pair (every pair, or a seeded sample of them when
+                                                                   the batch is too large for DUMP_LIMIT; `pairs` names them)
+      viterbi_path_pairs, viterbi_path_offsets, viterbi_paths      the paths (global transition ids) of a seeded sample of
+                                                                   DUMP_PATHS pairs, concatenated, within what is left"""
+    n = len(ll)
+    rng = np.random.default_rng(SEED)
+    cap = DUMP_LIMIT // 2 // (4 * 8)
+    pairs = np.arange(n) if n <= cap else np.sort(rng.choice(n, cap, replace=False))
+    arrays = {"pairs": pairs, "forward_loglike": ll[pairs], "viterbi_score": sc[pairs], "viterbi_path_length": plen[pairs]}
+    budget = DUMP_LIMIT - 8 * 4 * len(pairs)
+    path_pairs, paths = [], []
+    for k in np.sort(rng.choice(n, min(n, DUMP_PATHS), replace=False)):
+        budget -= 8 * (int(off[k + 1] - off[k]) + 2)
+        if budget < 0:
+            break
+        path_pairs.append(k)
+        paths.append(trans[off[k]:off[k + 1]])
+    arrays["viterbi_path_pairs"] = np.array(path_pairs)
+    arrays["viterbi_path_offsets"] = np.concatenate([[0], np.cumsum([len(p) for p in paths])])
+    arrays["viterbi_paths"] = np.concatenate(paths) if paths else np.zeros(0)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def machine_groups(mj: dict):

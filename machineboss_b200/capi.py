@@ -325,13 +325,20 @@ def viterbi(m: Machine, b: Batch, paths: bool = True, packed: bool = False):
         _check(lib().mb_viterbi(m.h, b.h, _ptr(score), None))
         return score
     score, plen = viterbi_lengths(m, b)
+    trans, off = viterbi_paths(b, plen)
+    if packed:
+        return score, (trans, off)
+    return score, [trans[off[k]:off[k + 1]] for k in range(b.n_pairs)]
+
+
+def viterbi_paths(b: Batch, plen: np.ndarray):
+    """The paths of the batch's last Viterbi call (path lengths `plen`), copied from the device: (all ids
+    concatenated as int32, offsets[nPairs+1])."""
     off = np.concatenate([[0], np.cumsum(plen)]).astype(np.int64)
     trans = np.empty(int(off[-1]), dtype=np.int32)
     if off[-1]:
         _check(lib().mb_viterbi_paths(b.h, _ptr(trans), _ptr(off)))
-    if packed:
-        return score, (trans, off)
-    return score, [trans[off[k]:off[k + 1]] for k in range(b.n_pairs)]
+    return trans, off
 
 
 def forward_into(m: Machine, b: Batch, out: np.ndarray) -> None:
