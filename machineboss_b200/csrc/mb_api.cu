@@ -182,6 +182,21 @@ int paths_reserve (mb_batch* b, int64_t need) {
   return 0;
 }
 
+int paths_place (mb_batch* b, const int64_t* pairs, int64_t n, const int64_t* dLen, int64_t* dOutOff) {
+  std::vector<int64_t> len ((size_t) n), off ((size_t) n);
+  MB_CUDA (cudaMemcpyAsync (len.data(), dLen, (size_t) n * 8, cudaMemcpyDeviceToHost, b->stream));
+  MB_CUDA (cudaStreamSynchronize (b->stream));
+  for (int64_t q = 0; q < n; ++q) {
+    off[q] = b->pathsPacked;
+    b->pathStart[pairs[q]] = b->pathsPacked;
+    b->pathLen[pairs[q]] = len[q];
+    b->pathsPacked += len[q];
+  }
+  if (paths_reserve (b, b->pathsPacked)) return 1;
+  MB_CUDA (cudaMemcpyAsync (dOutOff, off.data(), (size_t) n * 8, cudaMemcpyHostToDevice, b->stream));
+  return 0;
+}
+
 // Stable counting sort of the transitions into token-indexed lists (see DevCsr).
 static void build_csr (const mb_machine* m, bool incoming, HostCsr& c) {
   const int64_t T = m->T;
@@ -392,7 +407,7 @@ int mb_machine_create (mb_machine** out, int32_t nStates, int32_t nInTok, int32_
     // engine (mb_lane.cu) sweeps whatever the number of states; the two-dimensional strip sweep needs
     // a cell to fit in shared memory
     bool ok = true;
-    if (wide_supported (m, &why)) ok = wide_prepare (m) == 0;      // (wide_prepare cleans up after itself on failure)
+    if (wide_supported (m, &why)) { ok = wide_prepare (m) == 0; if (!ok) wide_destroy (m); }
     else if (m->nIn != 0) { set_error ("mb_set_engine(WIDE): " + why); mb_machine_destroy (m); return 1; }
     if (ok) { m->engine = MB_ENGINE_WIDE; chosen = true; }
     else if (!automatic && m->nIn != 0) { mb_machine_destroy (m); return 1; }
@@ -411,9 +426,13 @@ int mb_machine_update_weights (mb_machine* m, const double* logWeight) {
     MB_CUDA (cudaMemcpy ((char*) m->dBlob + m->incLwOffset, m->hInc.lw.data(), m->hInc.lw.size() * 8, cudaMemcpyHostToDevice));
     MB_CUDA (cudaMemcpy ((char*) m->dBlob + m->outLwOffset, m->hOut.lw.data(), m->hOut.lw.size() * 8, cudaMemcpyHostToDevice));
   }
-  if ((m->wide || m->lane || m->big) && wide_update_weights (m)) return 1;
-  if (m->engine == MB_ENGINE_JIT) return jit_update_weights (m);
-  return 0;
+  if (lane_update_weights (m) || col_update_weights (m)) return 1;
+  const int rc = big_update_weights (m);
+  if (rc == 2) {      // the new weights' ratios changed which insert groups are proportional: generate the big engine again
+    big_destroy (m);
+    if (big_supported (m, nullptr) && big_prepare (m)) big_destroy (m);      // (without it the wide engine's sweeps serve)
+  } else if (rc) return 1;
+  return wide_update_weights (m) || jit_update_weights (m);
 }
 
 int mb_machine_info (const mb_machine* m, int32_t* nStates, int64_t* nTrans, int32_t* engine) {
@@ -429,6 +448,9 @@ void mb_machine_destroy (mb_machine* m) {
   cudaSetDevice (m->device);
   jit_destroy (m);
   wide_destroy (m);
+  lane_destroy (m);
+  col_destroy (m);
+  big_destroy (m);
   if (m->dBlob) cudaFree (m->dBlob);
   delete m;
 }
@@ -565,37 +587,104 @@ static int check_call (const mb_machine* m, const mb_batch* b) {
   return 0;
 }
 
-// The strip kernels sweep full matrices; a batch carrying envelopes runs on the generic engine.
-static bool use_jit (const mb_machine* m, const mb_batch* b) { return m->engine == MB_ENGINE_JIT && !b->hasEnv; }
-// 1: the wide engine takes the call, 0: the generic engine does, -1: error
-static int use_wide (mb_machine* m, const mb_batch* b) {
-  if (m->engine == MB_ENGINE_WIDE) return 1;
-  if (m->engine == MB_ENGINE_JIT && b->hasEnv && wide_supported (m, nullptr)) {
-    if (!m->wide && wide_prepare (m)) return -1;      // (a failed preparation leaves m->wide null)
-    return 1;
+enum Pass { PASS_FORWARD, PASS_VITERBI_PATHS, PASS_VITERBI_SCORES, PASS_BACKWARD, PASS_COUNTS, PASS_MATRIX };
+enum Route { ROUTE_ERROR = -1, ROUTE_NONE, ROUTE_JIT, ROUTE_BIG, ROUTE_COL, ROUTE_LANE, ROUTE_WIDE, ROUTE_GENERIC };
+
+// The engine that serves a call, after any lazy preparation it needs (ROUTE_NONE: nothing to do; ROUTE_ERROR: a preparation
+// failed, error set).  A failed preparation destroys what it built, so the engine's handle is null again.
+static int route_of (mb_machine* m, mb_batch* b, Pass pass) {
+  const bool sweep = pass == PASS_FORWARD || pass == PASS_VITERBI_PATHS || pass == PASS_VITERBI_SCORES;
+  if (pass == PASS_MATRIX || m->engine == MB_ENGINE_GENERIC) return ROUTE_GENERIC;
+  if (m->engine == MB_ENGINE_JIT) {
+    // the strip kernels sweep full matrices; with envelopes the wide engine takes the sweeps it can, the generic engine the rest
+    if (!b->hasEnv) return ROUTE_JIT;
+    if (!sweep || !wide_supported (m, nullptr)) return ROUTE_GENERIC;
+    if (!m->wide && wide_prepare (m)) { wide_destroy (m); return ROUTE_ERROR; }
+    return ROUTE_WIDE;
   }
-  return 0;
+  if (!sweep) return ROUTE_GENERIC;
+  if (b->nPairs == 0) return ROUTE_NONE;
+  if (lane_wanted (m, b)) {      // no input sequences: a read per lane, or the column engine for periodic generators
+    if (!m->lane) {
+      if (lane_prepare (m)) { lane_destroy (m); return ROUTE_ERROR; }
+      if (col_prepare (m, false)) {      // (if it cannot be built, the lane sweeps serve)
+        if (m->opt.get ("verbose", 0)) fprintf (stderr, "lane engine: the column engine could not be prepared (%s); using the lane sweeps\n", mb_last_error());
+        col_destroy (m);
+      }
+    }
+    const bool colTraces = !(pass == PASS_VITERBI_PATHS && m->opt.get ("col_no_traceback", 0));
+    return col_usable (m, pass == PASS_FORWARD) && colTraces ? ROUTE_COL : ROUTE_LANE;
+  }
+  if (!m->wide) return ROUTE_GENERIC;      // too large for the two-dimensional strip sweep
+  if (!b->hasEnv) {      // full matrices of a mid-size machine: the generated thread-per-cell sweep (mb_big.cu)
+    if (!m->bigTried) {      // a machine the generator cannot handle after all (NVRTC out of resources, ...) stays with the table-driven sweep
+      m->bigTried = true;
+      if (big_supported (m, nullptr) && big_prepare (m)) {
+        if (m->opt.get ("verbose", 0)) fprintf (stderr, "big engine: not available for this machine (%s); using the wide engine\n", mb_last_error());
+        big_destroy (m);
+      }
+    }
+    if (pass == PASS_FORWARD ? big_wanted (m, b) : big_wanted_viterbi (m, b)) return ROUTE_BIG;
+  }
+  return ROUTE_WIDE;
+}
+
+// route_of, and with the verbose option one line on stderr naming the pass and the engine
+static int route (mb_machine* m, mb_batch* b, Pass pass) {
+  const int r = route_of (m, b, pass);
+  if (r != ROUTE_ERROR && m->opt.get ("verbose", 0)) {
+    static const char* const passNames[] = { "mb_forward", "mb_viterbi", "mb_viterbi (scores)", "mb_backward", "mb_counts", "mb_matrix" };
+    static const char* const engineNames[] = { "no engine (empty batch)", "jit engine", "big engine", "column engine", "lane engine", "wide engine", "generic engine" };
+    fprintf (stderr, "%s: %s\n", passNames[pass], engineNames[r]);
+  }
+  return r;
 }
 
 int mb_forward (mb_machine* m, mb_batch* b, double* loglike) {
   if (check_call (m, b)) return 1;
-  if (use_jit (m, b)) return jit_forward (m, b, loglike, false);
-  const int w = use_wide (m, b);
-  return w < 0 ? 1 : w ? wide_forward (m, b, loglike) : generic_forward (m, b, loglike, false);
+  if (m->engine == MB_ENGINE_WIDE) b->lastRedo = 0;      // (the generic engine, which re-runs nothing, does not set it)
+  switch (route (m, b, PASS_FORWARD)) {
+    case ROUTE_NONE: return 0;
+    case ROUTE_JIT: return jit_forward (m, b, loglike, false);
+    case ROUTE_BIG: return big_forward (m, b, loglike);
+    case ROUTE_COL: return col_forward (m, b, loglike);
+    case ROUTE_LANE: return lane_forward (m, b, loglike);
+    case ROUTE_WIDE: return wide_forward (m, b, loglike);
+    case ROUTE_GENERIC: return generic_forward (m, b, loglike, false);
+    default: return 1;
+  }
 }
 
 int mb_backward (mb_machine* m, mb_batch* b, double* loglike) {
   if (check_call (m, b)) return 1;
-  return use_jit (m, b) ? jit_forward (m, b, loglike, true) : generic_forward (m, b, loglike, true);
+  return route (m, b, PASS_BACKWARD) == ROUTE_JIT ? jit_forward (m, b, loglike, true) : generic_forward (m, b, loglike, true);
 }
 
 int mb_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen) {
   if (check_call (m, b)) return 1;
   if (b->copyStream) MB_CUDA (cudaStreamSynchronize (b->copyStream));      // paths of the previous call still on their way out
   b->pathIdLimit = m->T;
-  if (use_jit (m, b)) return jit_viterbi (m, b, score, pathLen);
-  const int w = use_wide (m, b);
-  return w < 0 ? 1 : w ? wide_viterbi (m, b, score, pathLen) : generic_viterbi (m, b, score, pathLen);
+  b->pathStart.clear();
+  b->pathLen.clear();
+  const int r = route (m, b, pathLen ? PASS_VITERBI_PATHS : PASS_VITERBI_SCORES);
+  if (pathLen) {      // the engine places each pair's path with paths_place
+    b->pathStart.assign ((size_t) b->nPairs, 0);
+    b->pathLen.assign ((size_t) b->nPairs, 0);
+    b->pathsPacked = 0;
+  }
+  int rc = 1;
+  switch (r) {
+    case ROUTE_NONE: rc = 0; break;
+    case ROUTE_JIT: rc = jit_viterbi (m, b, score, pathLen); break;
+    case ROUTE_BIG: rc = big_viterbi (m, b, score, pathLen); break;
+    case ROUTE_COL: rc = col_viterbi (m, b, score, pathLen); break;
+    case ROUTE_LANE: rc = lane_viterbi (m, b, score, pathLen); break;
+    case ROUTE_WIDE: rc = wide_viterbi (m, b, score, pathLen); break;
+    case ROUTE_GENERIC: rc = generic_viterbi (m, b, score, pathLen); break;
+  }
+  if (rc) { b->pathStart.clear(); b->pathLen.clear(); return 1; }      // no traceback stored
+  if (pathLen) for (int64_t k = 0; k < b->nPairs; ++k) pathLen[k] = b->pathLen[k];
+  return 0;
 }
 
 int mb_viterbi_paths (mb_batch* b, int32_t* pathTrans, const int64_t* pathOff) {
@@ -691,12 +780,13 @@ int mb_batch_wait (mb_batch* b) {
 
 int mb_counts (mb_machine* m, mb_batch* b, double* counts, double* loglike) {
   if (check_call (m, b)) return 1;
-  return use_jit (m, b) ? jit_counts (m, b, counts, loglike) : generic_counts (m, b, counts, loglike);
+  return route (m, b, PASS_COUNTS) == ROUTE_JIT ? jit_counts (m, b, counts, loglike) : generic_counts (m, b, counts, loglike);
 }
 
 int mb_matrix (mb_machine* m, mb_batch* b, int64_t pair, int32_t kind, double* cells) {
   if (check_call (m, b)) return 1;
   if (!cells) { set_error ("mb_matrix: null output"); return 1; }
+  route (m, b, PASS_MATRIX);
   return generic_matrix (m, b, pair, kind, cells);
 }
 

@@ -578,17 +578,8 @@ __global__ void big_traceback_kernel (BigTbPlan p, DevBatch b, const int64_t* __
   if (!out) lenOut[n] = len;
 }
 
-struct BigBuf {
-  void* p = nullptr;
-  ~BigBuf() { if (p) cudaFree (p); }
-  int alloc (size_t bytes) { MB_CUDA (cudaMalloc (&p, bytes ? bytes : 8)); return 0; }
-  template<class T> T* as() { return (T*) p; }
-};
-
 int big_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen) {
   BigEngine& B = *be (m);
-  b->pathStart.clear();
-  b->pathLen.clear();
   if (b->nPairs == 0) return 0;
   const bool trace = pathLen != nullptr;
   std::vector<int64_t> order ((size_t) b->nPairs);
@@ -641,9 +632,7 @@ int big_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen) {
     tp.type = q; q += G; tp.source = q; q += G; tp.idOff = q; q += G; tp.ids = q;
     tp.S = S; tp.nOut = m->nOut; tp.nWords = B.nPtrWords;
   }
-  b->pathStart.assign ((size_t) b->nPairs, 0);
-  b->pathLen.assign ((size_t) b->nPairs, 0);
-  int64_t packed = 0, launches = 0;
+  int64_t launches = 0;
   double ms = 0;
   for (size_t c0 = 0; c0 < order.size();) {
     std::vector<int64_t> chunk, bpOff;
@@ -671,7 +660,7 @@ int big_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen) {
       }
     }
     c0 = c1;
-    BigBuf dBp, dBpOff, dOrder, dLen, dOutOff;
+    DevBuf dBp, dBpOff, dOrder, dLen, dOutOff;
     if (dBp.alloc ((size_t) words * 4) || dBpOff.alloc (bpOff.size() * 8) || dOrder.alloc (chunk.size() * 8) || dLen.alloc (chunk.size() * 8) || dOutOff.alloc (chunk.size() * 8)) return 1;
     MB_CUDA (cudaMemcpyAsync (dBpOff.p, bpOff.data(), bpOff.size() * 8, cudaMemcpyHostToDevice, b->stream));
     MB_CUDA (cudaMemcpyAsync (dOrder.p, chunk.data(), chunk.size() * 8, cudaMemcpyHostToDevice, b->stream));
@@ -682,12 +671,7 @@ int big_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen) {
     const unsigned tg = (unsigned) ((nWork + 63) / 64);
     big_traceback_kernel<<<tg, 64, 0, b->stream>>> (tp, b->dev, dOrder.as<int64_t>(), nWork, dBp.as<unsigned>(), dBpOff.as<int64_t>(), dRes, dLen.as<int64_t>(), nullptr, nullptr);
     MB_CUDA (cudaGetLastError());
-    std::vector<int64_t> len (chunk.size()), off (chunk.size());
-    MB_CUDA (cudaMemcpyAsync (len.data(), dLen.p, len.size() * 8, cudaMemcpyDeviceToHost, b->stream));
-    MB_CUDA (cudaStreamSynchronize (b->stream));
-    for (size_t n = 0; n < len.size(); ++n) { off[n] = packed; b->pathStart[chunk[n]] = packed; b->pathLen[chunk[n]] = len[n]; packed += len[n]; }
-    if (paths_reserve (b, packed)) return 1;
-    MB_CUDA (cudaMemcpyAsync (dOutOff.p, off.data(), off.size() * 8, cudaMemcpyHostToDevice, b->stream));
+    if (paths_place (b, chunk.data(), nWork, dLen.as<int64_t>(), dOutOff.as<int64_t>())) return 1;
     big_traceback_kernel<<<tg, 64, 0, b->stream>>> (tp, b->dev, dOrder.as<int64_t>(), nWork, dBp.as<unsigned>(), dBpOff.as<int64_t>(), dRes, dLen.as<int64_t>(), b->dPaths, dOutOff.as<int64_t>());
     MB_CUDA (cudaGetLastError());
     launches += 3;
@@ -697,7 +681,6 @@ int big_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen) {
   b->lastMs = ms;
   b->lastLaunches = launches;
   MB_CUDA (cudaMemcpy (score, dRes, (size_t) b->nPairs * 8, cudaMemcpyDeviceToHost));
-  for (int64_t k = 0; k < b->nPairs; ++k) pathLen[k] = b->pathLen[k];
   return 0;
 }
 

@@ -614,7 +614,7 @@ struct MBColArgsHost {      // must match struct MBColArgs in the skeleton
 };
 
 // order: reads, longest first.  sums: Forward (flags set for the reads whose result must not be trusted); else Viterbi scores.
-int col_launch (mb_machine* m, mb_batch* b, const std::vector<int64_t>& order, bool sums, double* dResult, int32_t* dFlag, int64_t* launches) {
+static int col_launch (mb_machine* m, mb_batch* b, const std::vector<int64_t>& order, bool sums, double* dResult, int32_t* dFlag, int64_t* launches) {
   ColEngine& E = *ce (m);
   const ColProg& p = E.prog;
   const int brow = p.nLL + 1;
@@ -750,7 +750,7 @@ __global__ void __launch_bounds__(64) col_traceback_kernel (ColTbPlan p, const u
 }
 
 // scores (dResult, by read) and paths (b->dPaths, b->pathStart / pathLen) of every read in `order`; *ms receives the device time
-int col_viterbi_paths (mb_machine* m, mb_batch* b, const std::vector<int64_t>& order, double* dResult, int64_t* launches, double* msOut) {
+static int col_viterbi_paths (mb_machine* m, mb_batch* b, const std::vector<int64_t>& order, double* dResult, int64_t* launches, double* msOut) {
   ColEngine& E = *ce (m);
   const ColProg& p = E.prog;
   const int brow = p.nLL + 1;
@@ -759,7 +759,6 @@ int col_viterbi_paths (mb_machine* m, mb_batch* b, const std::vector<int64_t>& o
   MB_CUDA (cudaMemGetInfo (&freeB, &totalB));
   const double budget = std::min (0.6 * (double) freeB, (double) m->opt.get ("col_bp_budget_mb", 1 << 20) * 1048576.);
   const int warps = E.threads / 32;
-  int64_t packed = 0;
   double ms = 0;
   ColTbPlan T;
   const int32_t* base = E.dTbPlan;
@@ -822,18 +821,7 @@ int col_viterbi_paths (mb_machine* m, mb_batch* b, const std::vector<int64_t>& o
     const unsigned tbGrid = (unsigned) ((nWork + 63) / 64);
     col_traceback_kernel<<<tbGrid, 64, 0, b->stream>>> (T, b->dY, b->dYOff, dOrder, nWork, dBp, dOffs + nWork, dPreP, dSufP, dResult, dLen, nullptr, nullptr);
     MB_CUDA (cudaGetLastError());
-    std::vector<int64_t> len ((size_t) nWork), outOff ((size_t) nWork);
-    MB_CUDA (cudaMemcpyAsync (len.data(), dLen, (size_t) nWork * 8, cudaMemcpyDeviceToHost, b->stream));
-    MB_CUDA (cudaStreamSynchronize (b->stream));
-    for (int64_t q = 0; q < nWork; ++q) {
-      const int64_t k = order[c0 + q];
-      outOff[q] = packed;
-      b->pathStart[k] = packed;
-      b->pathLen[k] = len[q];
-      packed += len[q];
-    }
-    if (paths_reserve (b, packed)) return 1;
-    MB_CUDA (cudaMemcpyAsync (dOutOff, outOff.data(), (size_t) nWork * 8, cudaMemcpyHostToDevice, b->stream));
+    if (paths_place (b, order.data() + c0, nWork, dLen, dOutOff)) return 1;
     col_traceback_kernel<<<tbGrid, 64, 0, b->stream>>> (T, b->dY, b->dYOff, dOrder, nWork, dBp, dOffs + nWork, dPreP, dSufP, dResult, dLen, b->dPaths, dOutOff);
     MB_CUDA (cudaGetLastError());
     if (launches) *launches += 5;
@@ -844,6 +832,56 @@ int col_viterbi_paths (mb_machine* m, mb_batch* b, const std::vector<int64_t>& o
     c0 = c1;
   }
   if (msOut) *msOut = ms;
+  return 0;
+}
+
+int col_forward (mb_machine* m, mb_batch* b, double* loglike) {
+  b->lastRedo = 0;
+  if (b->nPairs == 0) return 0;
+  const std::vector<int64_t> order = lane_order (b, nullptr);
+  DevBuf dRes, dFlag;
+  if (dRes.alloc ((size_t) b->nPairs * 8) || dFlag.alloc ((size_t) b->nPairs * 4)) return 1;
+  MB_CUDA (cudaMemsetAsync (dFlag.p, 0, (size_t) b->nPairs * 4, b->stream));
+  if (timing_begin (b)) return 1;
+  // the linear sweep; reads it flags, or that come out without any path, are decided by the lane engine's log-domain sweep
+  int64_t launches = 0;
+  if (col_launch (m, b, order, true, dRes.as<double>(), dFlag.as<int32_t>(), &launches)) return 1;
+  std::vector<int32_t> flag ((size_t) b->nPairs);
+  std::vector<double> res ((size_t) b->nPairs);
+  MB_CUDA (cudaMemcpyAsync (flag.data(), dFlag.p, flag.size() * 4, cudaMemcpyDeviceToHost, b->stream));
+  MB_CUDA (cudaMemcpyAsync (res.data(), dRes.p, res.size() * 8, cudaMemcpyDeviceToHost, b->stream));
+  MB_CUDA (cudaStreamSynchronize (b->stream));
+  std::vector<int64_t> redo;
+  for (int64_t k = 0; k < b->nPairs; ++k) if (flag[k] || !(res[k] > -INFINITY)) redo.push_back (k);
+  if (!redo.empty()) {
+    if (lane_forward_log_subset (m, b, redo, dRes.as<double>(), dFlag.as<int32_t>())) return 1;
+    ++launches;
+  }
+  b->lastRedo = (int64_t) redo.size();
+  if (timing_end (b, launches)) return 1;
+  MB_CUDA (cudaMemcpy (loglike, dRes.p, (size_t) b->nPairs * 8, cudaMemcpyDeviceToHost));
+  return 0;
+}
+
+// scores only: the max-plus sweep; with pathLen: the sweep with pointers and the column engine's own walk back
+int col_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen) {
+  if (b->nPairs == 0) return 0;
+  const std::vector<int64_t> order = lane_order (b, nullptr);
+  DevBuf dRes;
+  if (dRes.alloc ((size_t) b->nPairs * 8)) return 1;
+  if (!pathLen) {
+    if (timing_begin (b)) return 1;
+    int64_t launches = 0;
+    if (col_launch (m, b, order, false, dRes.as<double>(), nullptr, &launches)) return 1;
+    if (timing_end (b, launches)) return 1;
+  } else {
+    int64_t launches = 0;
+    double ms = 0;
+    if (col_viterbi_paths (m, b, order, dRes.as<double>(), &launches, &ms)) return 1;
+    b->lastMs = ms;
+    b->lastLaunches = launches;
+  }
+  MB_CUDA (cudaMemcpy (score, dRes.p, (size_t) b->nPairs * 8, cudaMemcpyDeviceToHost));
   return 0;
 }
 

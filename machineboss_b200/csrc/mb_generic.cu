@@ -246,13 +246,6 @@ static int plan_chunks (const mb_batch* b, int S, bool rolling, int copies, std:
   return 0;
 }
 
-struct DevBuf {
-  void* p = nullptr;
-  ~DevBuf() { if (p) cudaFree (p); }
-  int alloc (size_t bytes) { MB_CUDA (cudaMalloc (&p, bytes ? bytes : 8)); return 0; }
-  template<class T> T* as() { return (T*) p; }
-};
-
 static int upload (DevBuf& d, const std::vector<int64_t>& v, cudaStream_t st) {
   if (d.alloc (v.size() * 8)) return 1;
   MB_CUDA (cudaMemcpyAsync (d.p, v.data(), v.size() * 8, cudaMemcpyHostToDevice, st));
@@ -304,16 +297,13 @@ int generic_matrix (mb_machine* m, mb_batch* b, int64_t pair, int kind, double* 
 }
 
 int generic_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen) {
-  b->pathStart.clear();
-  b->pathLen.clear();
   if (b->nPairs == 0) return 0;
   const bool trace = pathLen != nullptr;
   std::vector<Chunk> chunks;
   if (plan_chunks (b, m->S, !trace, 1, chunks)) return 1;
   DevBuf dRes;
   if (dRes.alloc ((size_t) b->nPairs * 8)) return 1;
-  if (trace) { b->pathStart.assign ((size_t) b->nPairs, 0); b->pathLen.assign ((size_t) b->nPairs, 0); }
-  int64_t packed = 0, launches = 0;
+  int64_t launches = 0;
   double ms = 0;
   for (auto& ch: chunks) {
     DevBuf dPairs, dOff, dWs, dLen, dOutOff;
@@ -326,21 +316,11 @@ int generic_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen
     if (trace) {
       DevBatch cb = b->dev;
       cb.nPairs = (int64_t) ch.pairs.size();
-      if (dLen.alloc (ch.pairs.size() * 8)) return 1;
+      if (dLen.alloc (ch.pairs.size() * 8) || dOutOff.alloc (ch.pairs.size() * 8)) return 1;
       const unsigned tg = (unsigned) ((ch.pairs.size() + 63) / 64);
       traceback_kernel<<<tg, 64, 0, b->stream>>> (m->dev, cb, dPairs.as<int64_t>(), dOff.as<int64_t>(), dWs.as<double>(), dRes.as<double>(), dLen.as<int64_t>(), nullptr, nullptr);
       MB_CUDA (cudaGetLastError());
-      std::vector<int64_t> len (ch.pairs.size()), off (ch.pairs.size());
-      MB_CUDA (cudaMemcpyAsync (len.data(), dLen.p, len.size() * 8, cudaMemcpyDeviceToHost, b->stream));
-      MB_CUDA (cudaStreamSynchronize (b->stream));
-      for (size_t n = 0; n < len.size(); ++n) {
-        off[n] = packed;
-        b->pathStart[ch.pairs[n]] = packed;
-        b->pathLen[ch.pairs[n]] = len[n];
-        packed += len[n];
-      }
-      if (paths_reserve (b, packed)) return 1;
-      if (upload (dOutOff, off, b->stream)) return 1;
+      if (paths_place (b, ch.pairs.data(), (int64_t) ch.pairs.size(), dLen.as<int64_t>(), dOutOff.as<int64_t>())) return 1;
       traceback_kernel<<<tg, 64, 0, b->stream>>> (m->dev, cb, dPairs.as<int64_t>(), dOff.as<int64_t>(), dWs.as<double>(), dRes.as<double>(), dLen.as<int64_t>(), b->dPaths, dOutOff.as<int64_t>());
       MB_CUDA (cudaGetLastError());
       launches += 2;
@@ -351,7 +331,6 @@ int generic_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen
   b->lastMs = ms;
   b->lastLaunches = launches;
   MB_CUDA (cudaMemcpy (score, dRes.p, (size_t) b->nPairs * 8, cudaMemcpyDeviceToHost));
-  if (trace) for (int64_t k = 0; k < b->nPairs; ++k) pathLen[k] = b->pathLen[k];
   return 0;
 }
 

@@ -80,6 +80,14 @@ bool cuda_ok (cudaError_t e, const char* what);
 
 #define MB_CUDA(call) do { if (!mb::cuda_ok ((call), #call)) return 1; } while (0)
 
+// scratch device memory owned by one scope: cudaMalloc on alloc, cudaFree when the scope ends
+struct DevBuf {
+  void* p = nullptr;
+  ~DevBuf() { if (p) cudaFree (p); }
+  int alloc (size_t bytes) { MB_CUDA (cudaMalloc (&p, bytes ? bytes : 8)); return 0; }
+  template<class T> T* as() { return (T*) p; }
+};
+
 }  // namespace mb
 
 // ---- handles ----
@@ -104,12 +112,12 @@ struct mb_machine {
   void* jit = nullptr;
   // wide engine (mb_wide.cu)
   void* wide = nullptr;
-  // lane engine (mb_lane.cu): the wide engine's path for batches without input sequences
+  // lane engine (mb_lane.cu): batches without input sequences on a WIDE machine
   void* lane = nullptr;
-  // big engine (mb_big.cu): generated straight-line Forward sweep for mid-size machines, reached through the wide engine
+  // big engine (mb_big.cu): generated straight-line Forward sweep for mid-size machines on full matrices
   void* big = nullptr;
   bool bigTried = false;
-  // column engine (mb_col.cu): periodic generators swept as column = period, row = read position; reached through the lane engine
+  // column engine (mb_col.cu): periodic generators swept as column = period, row = read position; prepared with the lane engine
   void* col = nullptr;
 };
 
@@ -144,6 +152,7 @@ struct mb_batch {
   // result of the last mb_viterbi with traceback: packed paths on the device
   int32_t* dPaths = nullptr;
   std::vector<int64_t> pathStart, pathLen;   // per pair: offset into dPaths and length
+  int64_t pathsPacked = 0;             // entries of dPaths the current mb_viterbi call has placed (paths_place)
   int64_t pathsCapacity = 0;
   size_t pathsBytes = 0;               // size of the pooled block behind dPaths
   int64_t pathIdLimit = 0;             // transition ids of the stored paths are below this (the machine's nTrans)
@@ -177,25 +186,28 @@ int wide_update_weights (mb_machine* m);
 int wide_forward (mb_machine* m, mb_batch* b, double* loglike);
 int wide_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen);
 
-// ---- lane engine (mb_lane.cu): a read per lane, for batches without input sequences; reached through the wide engine ----
+// ---- lane engine (mb_lane.cu): a read per lane, for batches without input sequences ----
 int lane_prepare (mb_machine* m);
 void lane_destroy (mb_machine* m);
 int lane_update_weights (mb_machine* m);
 bool lane_wanted (const mb_machine* m, const mb_batch* b);      // no input sequences, no envelopes
 int lane_forward (mb_machine* m, mb_batch* b, double* loglike);
 int lane_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen);
+// the log-domain sweep over a subset of the batch, results into dResult[pair] (device): where the column engine sends the reads it flags
+int lane_forward_log_subset (mb_machine* m, mb_batch* b, const std::vector<int64_t>& pairs, double* dResult, int32_t* dFlag);
+std::vector<int64_t> lane_order (const mb_batch* b, const std::vector<int64_t>* subset);      // the pairs (all, or a subset), longest read first
 // the windowed program of the lane engine, executed for one read on the host (diagnostic; op 0 sum, 1 max, 2 log-sum-exp)
 int lane2_emulate (const mb_machine* m, const uint8_t* y, int64_t Lo, int op, double* result, std::vector<uint32_t>* bpOut);
 int lane2_info (const mb_machine* m, int32_t* info);      // { usable, window states, ring slots, hub sources, hub destinations, live states, records, back-pointer bytes }
 
 // ---- column engine (mb_col.cu): generators without input whose states repeat with a period (profile HMMs), swept as
-// a two-dimensional recurrence by a generated strip kernel; the lane engine calls it and keeps what it declines ----
+// a two-dimensional recurrence by a generated strip kernel; the lane engine serves the sweeps it declines ----
 int col_prepare (mb_machine* m, bool hostOnly);      // 0 also when the machine has no such structure (m->col stays null)
 void col_destroy (mb_machine* m);
 int col_update_weights (mb_machine* m);
 bool col_usable (const mb_machine* m, bool sums);
-int col_launch (mb_machine* m, mb_batch* b, const std::vector<int64_t>& order, bool sums, double* dResult, int32_t* dFlag, int64_t* launches);
-int col_viterbi_paths (mb_machine* m, mb_batch* b, const std::vector<int64_t>& order, double* dResult, int64_t* launches, double* ms);      // scores + paths into the batch
+int col_forward (mb_machine* m, mb_batch* b, double* loglike);
+int col_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen);
 int col_compile_check (const mb_machine* m, std::string* log);
 int col_info (const mb_machine* m, int32_t* info);      // { usable, period, first state, columns, prefix, suffix, carried, accumulators, groups, weight slots, left-going, up }
 int col_emulate (const mb_machine* m, const uint8_t* y, int64_t Lo, int op, double* result, std::vector<int64_t>* path);      // op 0 log-sum-exp, 1 max (path: the traceback, may be null)
@@ -232,6 +244,9 @@ size_t ws_bytes (const mb_batch* b, int slot);
 size_t ws_pool_bytes (int device);
 bool ws_pool_fits (int device, size_t bytes);   // a pooled block would serve this request   // freed blocks kept for reuse; released when an allocation fails
 int paths_reserve (mb_batch* b, int64_t need);   // room for `need` packed path entries in b->dPaths (pooled; keeps the content)
+// Viterbi paths of pairs[0..n), after those the call has placed so far: copies their lengths (dLen, device) to the host,
+// sets pathStart / pathLen, grows dPaths to hold them and writes each pair's start into dOutOff (device) for the id pass
+int paths_place (mb_batch* b, const int64_t* pairs, int64_t n, const int64_t* dLen, int64_t* dOutOff);
 
 // timing helpers
 int timing_begin (mb_batch* b);

@@ -924,6 +924,7 @@ static int upload_row_tables (const mb_machine* m, JitEngine& J) {
 }
 
 int jit_update_weights (mb_machine* m) {
+  if (!m->jit) return 0;
   JitEngine& J = *(JitEngine*) m->jit;
   std::vector<double> ef, eb;
   fill_weights (m, J, ef, eb);
@@ -1171,13 +1172,6 @@ struct MBArgsHost {   // must match struct MBArgs in the skeleton
   unsigned* F32; const int64_t* f32Off;
   int32_t* ef; const int64_t* efOff;
   const int64_t* items; const int64_t* itemBnd; int* prog;
-};
-
-struct DevBuf {
-  void* p = nullptr;
-  ~DevBuf() { if (p) cudaFree (p); }
-  int alloc (size_t bytes) { MB_CUDA (cudaMalloc (&p, bytes ? bytes : 8)); return 0; }
-  template<class T> T* as() { return (T*) p; }
 };
 
 static std::vector<int64_t> cost_order (const mb_batch* b, const std::vector<int64_t>& pairs) {
@@ -1474,8 +1468,6 @@ static double memory_budget (const mb_machine* m, const mb_batch* b, int slot, d
 
 int jit_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen) {
   JitEngine& J = *(JitEngine*) m->jit;
-  b->pathStart.clear();
-  b->pathLen.clear();
   if (b->nPairs == 0) return 0;
   const bool trace = pathLen != nullptr;
   const int useC = choose_width (m, J, b, full_order (b), trace ? 1 : 2);
@@ -1521,7 +1513,6 @@ int jit_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen) {
   int64_t* dOutOff = (int64_t*) ws_reserve (b, WS_OUTOFF, (size_t) b->nPairs * 8);
   if (!dTb || !dRes || !dTbOff || !dPairs || !dLen || !dOutOff) return 1;
   MB_CUDA (cudaMemcpyAsync (dTbOff, tbOffHost.data(), (size_t) b->nPairs * 8, cudaMemcpyHostToDevice, b->stream));
-  if (trace) { b->pathStart.assign ((size_t) b->nPairs, 0); b->pathLen.assign ((size_t) b->nPairs, 0); }
   char* plan = (char*) J.dTbPlan;
   const size_t nSlots = J.fwd.slots.size();
   TbPlan tp;
@@ -1534,7 +1525,7 @@ int jit_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen) {
   tp.idTab = tp.bits + m->S;
   tp.S = m->S; tp.nOut = m->nOut; tp.tbBytes = J.tbBytes; tp.W = W;
   tp.C = useC; tp.laneBytes = padded ? 16 : laneBytes;
-  int64_t packed = 0, launches = 0;
+  int64_t launches = 0;
   double ms = 0;
   for (size_t c = 0; c < chunks.size(); ++c) {
     std::vector<int64_t> chunkOrder;
@@ -1561,17 +1552,7 @@ int jit_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen) {
       const unsigned tg = (unsigned) ((n + 63) / 64);
       jit_traceback_kernel<<<tg, 64, 0, b->stream>>> (tp, (int) nSlots, b->dev, dPairs, (int64_t) n, dTb, dTbOff, dRes, dLen, dTmp, dTmpOff);
       MB_CUDA (cudaGetLastError());
-      std::vector<int64_t> len (n), off (n);
-      MB_CUDA (cudaMemcpyAsync (len.data(), dLen, n * 8, cudaMemcpyDeviceToHost, b->stream));
-      MB_CUDA (cudaStreamSynchronize (b->stream));
-      for (size_t q = 0; q < n; ++q) {
-        off[q] = packed;
-        b->pathStart[chunks[c][q]] = packed;
-        b->pathLen[chunks[c][q]] = len[q];
-        packed += len[q];
-      }
-      if (paths_reserve (b, packed)) return 1;
-      MB_CUDA (cudaMemcpyAsync (dOutOff, off.data(), n * 8, cudaMemcpyHostToDevice, b->stream));
+      if (paths_place (b, chunks[c].data(), (int64_t) n, dLen, dOutOff)) return 1;
       jit_path_ids_kernel<<<(unsigned) ((n * 32 + 255) / 256), 256, 0, b->stream>>> (tp, (int) nSlots, b->dev, dPairs, (int64_t) n, dLen, dTmp, dTmpOff, b->dPaths, dOutOff);
       MB_CUDA (cudaGetLastError());
       launches += 2;
@@ -1582,7 +1563,6 @@ int jit_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen) {
   b->lastMs = ms;
   b->lastLaunches = launches;
   MB_CUDA (cudaMemcpy (score, dRes, (size_t) b->nPairs * 8, cudaMemcpyDeviceToHost));
-  if (trace) for (int64_t k = 0; k < b->nPairs; ++k) pathLen[k] = b->pathLen[k];
   if (ws_bytes (b, WS_TB) > kKeepScratchBytes) ws_release (b, WS_TB);
   return 0;
 }

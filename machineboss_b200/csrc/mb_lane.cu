@@ -330,7 +330,6 @@ static void lane_fill_weights (const mb_machine* m, LHost* h) {
 
 void lane_destroy (mb_machine* m) {
   LHost* h = lh (m);
-  col_destroy (m);
   if (!h) return;
   for (void* p: { (void*) h->dRecLin, (void*) h->dRecLog, (void*) h->dEmLin, (void*) h->dEmLog, (void*) h->dEmIdx, (void*) h->l2.dBlobLin, (void*) h->l2.dBlobLog }) if (p) cudaFree (p);
   delete h;
@@ -360,7 +359,7 @@ int lane_update_weights (mb_machine* m) {
   if (!h) return 0;
   lane_fill_weights (m, h);
   if (h->l2.ok) lane2_fill_weights (m, h);
-  return lane_upload (m, h, false) || lane2_upload (m, h, false) || col_update_weights (m);
+  return lane_upload (m, h, false) || lane2_upload (m, h, false);
 }
 
 // The transition program: destinations in index order; per destination the emitting terms (union
@@ -437,12 +436,8 @@ int lane_prepare (mb_machine* m) {
   lane_fill_weights (m, h);
   lane2_build (m, h);
   if (h->l2.ok) lane2_fill_weights (m, h);
-  if (m->opt.get ("lane_host_only", 0)) return col_prepare (m, true);      // (diagnostic: build the programs without touching a device)
+  if (m->opt.get ("lane_host_only", 0)) return 0;      // (diagnostic: build the programs without touching a device)
   if (lane_upload (m, h, true) || lane2_upload (m, h, true)) return 1;
-  if (col_prepare (m, false)) {      // periodic machines (profile HMMs): the column engine takes the sweeps it can; if it cannot be built, the sweeps here serve
-    if (m->opt.get ("verbose", 0)) fprintf (stderr, "lane engine: the column engine could not be prepared (%s); using the lane sweeps\n", mb_last_error());
-    col_destroy (m);
-  }
   MB_CUDA (cudaDeviceGetAttribute (&h->numSMs, cudaDevAttrMultiProcessorCount, m->device));
   if (m->opt.get ("verbose", 0))
     fprintf (stderr, "lane engine: S=%d records=%lld (emitting rows %zu x %d tokens), bp %d bytes\n", S, (long long) h->nRec, h->emPerm.size() / std::max (nOut, 1), nOut, h->bpBytes);
@@ -1081,13 +1076,6 @@ __global__ void __launch_bounds__(256) lane2_kernel (const __grid_constant__ L2P
   }
 }
 
-struct LBuf {
-  void* p = nullptr;
-  ~LBuf() { if (p) cudaFree (p); }
-  int alloc (size_t bytes) { MB_CUDA (cudaMalloc (&p, bytes ? bytes : 8)); return 0; }
-  template<class T> T* as() { return (T*) p; }
-};
-
 // reads per lane.  Measured on B200 (PF00516, reads of 275): with enough reads to give every SM some 40
 // warps, one read per lane is fastest (262 144 reads: 175 GCUPS Forward, 132 Viterbi); with fewer, a second
 // independent chain per thread makes up for the missing warps in the sums (65 536 reads: 40 -> 89 GCUPS),
@@ -1204,7 +1192,7 @@ static int lane_launch (mb_machine* m, mb_batch* b, int R, const std::vector<int
                 : lane_launch_r<OP, 1> (m, b, order, dResult, dFlag, dBp, dBpOff);
 }
 
-static std::vector<int64_t> lane_order (const mb_batch* b, const std::vector<int64_t>* subset) {
+std::vector<int64_t> lane_order (const mb_batch* b, const std::vector<int64_t>* subset) {
   std::vector<int64_t> order;
   if (subset) order = *subset;
   else { order.resize ((size_t) b->nPairs); for (int64_t k = 0; k < b->nPairs; ++k) order[k] = k; }
@@ -1218,34 +1206,23 @@ bool lane_wanted (const mb_machine* m, const mb_batch* b) {
   return true;
 }
 
+int lane_forward_log_subset (mb_machine* m, mb_batch* b, const std::vector<int64_t>& pairs, double* dResult, int32_t* dFlag) {
+  if (!m->lane) { set_error ("lane engine not prepared for this machine"); return 1; }
+  return lane_launch<L_LSE> (m, b, lane_reads_per_lane (m, lh (m), (int64_t) pairs.size(), L_LSE), lane_order (b, &pairs), dResult, dFlag, nullptr, nullptr);
+}
+
 int lane_forward (mb_machine* m, mb_batch* b, double* loglike) {
   b->lastRedo = 0;
   if (b->nPairs == 0) return 0;
   LHost* h = lh (m);
   const std::vector<int64_t> order = lane_order (b, nullptr);
-  LBuf dRes, dFlag;
+  DevBuf dRes, dFlag;
   if (dRes.alloc ((size_t) b->nPairs * 8) || dFlag.alloc ((size_t) b->nPairs * 4)) return 1;
   MB_CUDA (cudaMemsetAsync (dFlag.p, 0, (size_t) b->nPairs * 4, b->stream));
   if (timing_begin (b)) return 1;
   int64_t launches = 1;
   const int R = lane_reads_per_lane (m, h, b->nPairs, L_SUM);
-  if (col_usable (m, true)) {
-    // the column engine's linear sweep; reads it flags, or that come out without any path, are decided by the log-domain sweep here
-    launches = 0;
-    if (col_launch (m, b, order, true, dRes.as<double>(), dFlag.as<int32_t>(), &launches)) return 1;
-    std::vector<int32_t> flag ((size_t) b->nPairs);
-    std::vector<double> res ((size_t) b->nPairs);
-    MB_CUDA (cudaMemcpyAsync (flag.data(), dFlag.p, flag.size() * 4, cudaMemcpyDeviceToHost, b->stream));
-    MB_CUDA (cudaMemcpyAsync (res.data(), dRes.p, res.size() * 8, cudaMemcpyDeviceToHost, b->stream));
-    MB_CUDA (cudaStreamSynchronize (b->stream));
-    std::vector<int64_t> redo;
-    for (int64_t k = 0; k < b->nPairs; ++k) if (flag[k] || !(res[k] > -INFINITY)) redo.push_back (k);
-    if (!redo.empty()) {
-      if (lane_launch<L_LSE> (m, b, lane_reads_per_lane (m, h, (int64_t) redo.size(), L_LSE), lane_order (b, &redo), dRes.as<double>(), dFlag.as<int32_t>(), nullptr, nullptr)) return 1;
-      ++launches;
-    }
-    b->lastRedo = (int64_t) redo.size();
-  } else if (h->linearOk) {
+  if (h->linearOk) {
     if (lane_launch<L_SUM> (m, b, R, order, dRes.as<double>(), dFlag.as<int32_t>(), nullptr, nullptr)) return 1;
     std::vector<int32_t> flag ((size_t) b->nPairs);
     MB_CUDA (cudaMemcpyAsync (flag.data(), dFlag.p, flag.size() * 4, cudaMemcpyDeviceToHost, b->stream));
@@ -1253,7 +1230,7 @@ int lane_forward (mb_machine* m, mb_batch* b, double* loglike) {
     std::vector<int64_t> redo;
     for (int64_t k = 0; k < b->nPairs; ++k) if (flag[k]) redo.push_back (k);
     if (!redo.empty()) {
-      if (lane_launch<L_LSE> (m, b, lane_reads_per_lane (m, h, (int64_t) redo.size(), L_LSE), lane_order (b, &redo), dRes.as<double>(), dFlag.as<int32_t>(), nullptr, nullptr)) return 1;
+      if (lane_forward_log_subset (m, b, redo, dRes.as<double>(), dFlag.as<int32_t>())) return 1;
       ++launches;
     }
     b->lastRedo = (int64_t) redo.size();
@@ -1268,33 +1245,17 @@ int wide_traceback_launch (mb_machine* m, mb_batch* b, const int64_t* dOrder, in
                            int bpBytes, int laneLayout, const double* dScore, int64_t* dLen, int32_t* dOut, const int64_t* dOutOff);
 
 int lane_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen) {
-  b->pathStart.clear();
-  b->pathLen.clear();
   if (b->nPairs == 0) return 0;
   LHost* h = lh (m);
   const bool trace = pathLen != nullptr;
   const std::vector<int64_t> order = lane_order (b, nullptr);
-  LBuf dRes;
+  DevBuf dRes;
   if (dRes.alloc ((size_t) b->nPairs * 8)) return 1;
   if (!trace) {
     if (timing_begin (b)) return 1;
-    int64_t launches = 1;
-    if (col_usable (m, false)) { launches = 0; if (col_launch (m, b, order, false, dRes.as<double>(), nullptr, &launches)) return 1; }
-    else if (lane_launch<L_MAX> (m, b, lane_reads_per_lane (m, h, b->nPairs, L_MAX), order, dRes.as<double>(), nullptr, nullptr, nullptr)) return 1;
-    if (timing_end (b, launches)) return 1;
+    if (lane_launch<L_MAX> (m, b, lane_reads_per_lane (m, h, b->nPairs, L_MAX), order, dRes.as<double>(), nullptr, nullptr, nullptr)) return 1;
+    if (timing_end (b, 1)) return 1;
     MB_CUDA (cudaMemcpy (score, dRes.p, (size_t) b->nPairs * 8, cudaMemcpyDeviceToHost));
-    return 0;
-  }
-  if (col_usable (m, false) && !m->opt.get ("col_no_traceback", 0)) {      // periodic generators: the column engine's sweep with pointers and its own walk back
-    b->pathStart.assign ((size_t) b->nPairs, 0);
-    b->pathLen.assign ((size_t) b->nPairs, 0);
-    int64_t launches = 0;
-    double ms = 0;
-    if (col_viterbi_paths (m, b, order, dRes.as<double>(), &launches, &ms)) return 1;
-    b->lastMs = ms;
-    b->lastLaunches = launches;
-    MB_CUDA (cudaMemcpy (score, dRes.p, (size_t) b->nPairs * 8, cudaMemcpyDeviceToHost));
-    for (int64_t k = 0; k < b->nPairs; ++k) pathLen[k] = b->pathLen[k];
     return 0;
   }
   // chunks of whole tasks (LPT reads) whose back-pointers, (maxLo+1) * S * LPT bytes or half-words per task, fit in free memory
@@ -1303,9 +1264,7 @@ int lane_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen) {
   MB_CUDA (cudaMemGetInfo (&freeB, &totalB));
   const double vecBytes = (double) h->numSMs * 48 * 2 * h->S * LPT * 8;
   const double budget = 0.75 * ((double) freeB - vecBytes);
-  b->pathStart.assign ((size_t) b->nPairs, 0);
-  b->pathLen.assign ((size_t) b->nPairs, 0);
-  int64_t packed = 0, launches = 0;
+  int64_t launches = 0;
   double ms = 0;
   for (size_t c0 = 0; c0 < order.size();) {
     std::vector<int64_t> bpOff;
@@ -1324,8 +1283,9 @@ int lane_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen) {
     c0 = c1;
     std::vector<int64_t> bpOffRead (chunk.size());      // the traceback kernel indexes by read
     for (size_t n = 0; n < chunk.size(); ++n) bpOffRead[n] = bpOff[n / LPT];
-    LBuf dBp, dBpOff, dBpOffRead, dOrder, dLen, dOutOff;
-    if (dBp.alloc ((size_t) bytes) || dBpOff.alloc (bpOff.size() * 8) || dBpOffRead.alloc (chunk.size() * 8) || dOrder.alloc (chunk.size() * 8) || dLen.alloc (chunk.size() * 8)) return 1;
+    DevBuf dBp, dBpOff, dBpOffRead, dOrder, dLen, dOutOff;
+    if (dBp.alloc ((size_t) bytes) || dBpOff.alloc (bpOff.size() * 8) || dBpOffRead.alloc (chunk.size() * 8) || dOrder.alloc (chunk.size() * 8) || dLen.alloc (chunk.size() * 8)
+        || dOutOff.alloc (chunk.size() * 8)) return 1;
     MB_CUDA (cudaMemcpyAsync (dBpOff.p, bpOff.data(), bpOff.size() * 8, cudaMemcpyHostToDevice, b->stream));
     MB_CUDA (cudaMemcpyAsync (dBpOffRead.p, bpOffRead.data(), bpOffRead.size() * 8, cudaMemcpyHostToDevice, b->stream));
     MB_CUDA (cudaMemcpyAsync (dOrder.p, chunk.data(), chunk.size() * 8, cudaMemcpyHostToDevice, b->stream));
@@ -1334,18 +1294,7 @@ int lane_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen) {
     const int64_t nWork = (int64_t) chunk.size();
     if (wide_traceback_launch (m, b, dOrder.as<int64_t>(), nWork, dBp.as<unsigned char>(), dBpOffRead.as<int64_t>(), h->bpBytes, LPT,
                                dRes.as<double>(), dLen.as<int64_t>(), nullptr, nullptr)) return 1;
-    std::vector<int64_t> len (chunk.size()), off (chunk.size());
-    MB_CUDA (cudaMemcpyAsync (len.data(), dLen.p, len.size() * 8, cudaMemcpyDeviceToHost, b->stream));
-    MB_CUDA (cudaStreamSynchronize (b->stream));
-    for (size_t n = 0; n < len.size(); ++n) {
-      off[n] = packed;
-      b->pathStart[chunk[n]] = packed;
-      b->pathLen[chunk[n]] = len[n];
-      packed += len[n];
-    }
-    if (paths_reserve (b, packed)) return 1;
-    if (dOutOff.alloc (off.size() * 8)) return 1;
-    MB_CUDA (cudaMemcpyAsync (dOutOff.p, off.data(), off.size() * 8, cudaMemcpyHostToDevice, b->stream));
+    if (paths_place (b, chunk.data(), nWork, dLen.as<int64_t>(), dOutOff.as<int64_t>())) return 1;
     if (wide_traceback_launch (m, b, dOrder.as<int64_t>(), nWork, dBp.as<unsigned char>(), dBpOffRead.as<int64_t>(), h->bpBytes, LPT,
                                dRes.as<double>(), dLen.as<int64_t>(), b->dPaths, dOutOff.as<int64_t>())) return 1;
     launches += 3;
@@ -1355,7 +1304,6 @@ int lane_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen) {
   b->lastMs = ms;
   b->lastLaunches = launches;
   MB_CUDA (cudaMemcpy (score, dRes.p, (size_t) b->nPairs * 8, cudaMemcpyDeviceToHost));
-  for (int64_t k = 0; k < b->nPairs; ++k) pathLen[k] = b->pathLen[k];
   return 0;
 }
 

@@ -628,8 +628,6 @@ static void wide_fill_weights (const mb_machine* m, WHost* h) {
 }
 
 void wide_destroy (mb_machine* m) {
-  lane_destroy (m);
-  big_destroy (m);
   WHost* h = wh (m);
   if (!h) return;
   if (h->dLin) cudaFree (h->dLin);
@@ -639,14 +637,6 @@ void wide_destroy (mb_machine* m) {
 }
 
 int wide_update_weights (mb_machine* m) {
-  if (lane_update_weights (m)) return 1;
-  {
-    const int rc = big_update_weights (m);
-    if (rc == 2) {      // the new weights' ratios changed which insert groups are proportional: generate the big engine again
-      big_destroy (m);
-      if (big_supported (m, nullptr) && big_prepare (m)) big_destroy (m);      // (without it the table-driven sweeps here serve)
-    } else if (rc) return 1;
-  }
   WHost* h = wh (m);
   if (!h) return 0;
   wide_fill_weights (m, h);
@@ -656,7 +646,7 @@ int wide_update_weights (mb_machine* m) {
   return 0;
 }
 
-static int wide_prepare_tables (mb_machine* m) {
+int wide_prepare (mb_machine* m) {
   WHost* h = new WHost;
   m->wide = h;
   WBuilder B, best;
@@ -717,18 +707,6 @@ static int wide_prepare_tables (mb_machine* m) {
   return 0;
 }
 
-// A failed preparation leaves no half-built tables behind: m->wide is either complete or null.
-int wide_prepare (mb_machine* m) {
-  if (wide_prepare_tables (m) == 0) return 0;
-  if (WHost* h = wh (m)) {
-    if (h->dLin) cudaFree (h->dLin);
-    if (h->dLog) cudaFree (h->dLog);
-    delete h;
-    m->wide = nullptr;
-  }
-  return 1;
-}
-
 // launch shape: column warps per CTA (W), ring depth, where the tables live, CTAs per SM
 struct WShape { int W = 0, R = 2, tabInSmem = 0, ctasPerSM = 0; size_t smem = 0; bool oneD = false; const void* fn = nullptr; };
 
@@ -767,13 +745,6 @@ static int choose_shape (const WHost* h, bool oneD, int forceW, WShape& best) {
 }
 
 
-struct WBuf {
-  void* p = nullptr;
-  ~WBuf() { if (p) cudaFree (p); }
-  int alloc (size_t bytes) { MB_CUDA (cudaMalloc (&p, bytes ? bytes : 8)); return 0; }
-  template<class T> T* as() { return (T*) p; }
-};
-
 static std::vector<int64_t> cost_order (const mb_batch* b, const std::vector<int64_t>* subset) {
   std::vector<int64_t> order;
   if (subset) order = *subset;
@@ -797,7 +768,7 @@ static int wide_launch (mb_machine* m, mb_batch* b, const std::vector<int64_t>& 
   const int64_t nWork = (int64_t) order.size();
   const int64_t wantCtas = oneD ? (nWork + nWarps * CPW - 1) / (nWarps * CPW) : nWork;
   const int grid = (int) std::max<int64_t> (1, std::min<int64_t> (wantCtas, (int64_t) sh.ctasPerSM * h->numSMs));
-  WBuf dOrder, dCounter, dBnd, dBndFG;
+  DevBuf dOrder, dCounter, dBnd, dBndFG;
   if (dOrder.alloc (order.size() * 8) || dCounter.alloc (8)) return 1;
   MB_CUDA (cudaMemcpyAsync (dOrder.p, order.data(), order.size() * 8, cudaMemcpyHostToDevice, b->stream));
   MB_CUDA (cudaMemsetAsync (dCounter.p, 0, 8, b->stream));
@@ -824,7 +795,7 @@ static int wide_launch (mb_machine* m, mb_batch* b, const std::vector<int64_t>& 
 // the log-domain sweep over a subset of the batch, results into dResult[pair] (device): where the big engine sends the pairs it flags
 int wide_forward_log_subset (mb_machine* m, mb_batch* b, const std::vector<int64_t>& pairs, double* dResult) {
   if (!m->wide) { set_error ("wide engine not prepared for this machine"); return 1; }
-  WBuf dFlag;
+  DevBuf dFlag;
   if (dFlag.alloc ((size_t) b->nPairs * 4)) return 1;
   return wide_launch<OP_LSE> (m, b, cost_order (b, &pairs), dResult, dFlag.as<int32_t>(), nullptr, nullptr);
 }
@@ -832,24 +803,9 @@ int wide_forward_log_subset (mb_machine* m, mb_batch* b, const std::vector<int64
 int wide_forward (mb_machine* m, mb_batch* b, double* loglike) {
   b->lastRedo = 0;
   if (b->nPairs == 0) return 0;
-  if (lane_wanted (m, b)) {      // no input sequences: a read per lane (mb_lane.cu)
-    if (!m->lane && lane_prepare (m)) return 1;
-    return lane_forward (m, b, loglike);
-  }
-  if (m->wide && !b->hasEnv) {      // full matrices of a mid-size machine: the generated thread-per-cell sweep (mb_big.cu)
-    if (!m->bigTried) {      // a machine the generator cannot handle after all (NVRTC out of resources, ...) stays with the table-driven sweep
-      m->bigTried = true;
-      if (big_supported (m, nullptr) && big_prepare (m)) {
-        if (m->opt.get ("verbose", 0)) fprintf (stderr, "big engine: not available for this machine (%s); using the wide engine\n", mb_last_error());
-        big_destroy (m);
-      }
-    }
-    if (big_wanted (m, b)) return big_forward (m, b, loglike);
-  }
-  if (!m->wide) return generic_forward (m, b, loglike, false);      // too large for the two-dimensional strip sweep
   WHost* h = wh (m);
   const std::vector<int64_t> order = cost_order (b, nullptr);
-  WBuf dRes, dFlag;
+  DevBuf dRes, dFlag;
   if (dRes.alloc ((size_t) b->nPairs * 8) || dFlag.alloc ((size_t) b->nPairs * 4)) return 1;
   MB_CUDA (cudaMemsetAsync (dFlag.p, 0, (size_t) b->nPairs * 4, b->stream));
   if (timing_begin (b)) return 1;
@@ -874,28 +830,11 @@ int wide_forward (mb_machine* m, mb_batch* b, double* loglike) {
 }
 
 int wide_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen) {
-  b->pathStart.clear();
-  b->pathLen.clear();
   if (b->nPairs == 0) return 0;
-  if (lane_wanted (m, b)) {
-    if (!m->lane && lane_prepare (m)) return 1;
-    return lane_viterbi (m, b, score, pathLen);
-  }
-  if (m->wide && !b->hasEnv) {      // full matrices of a mid-size machine: the generated thread-per-cell sweep (mb_big.cu)
-    if (!m->bigTried) {      // a machine the generator cannot handle after all (NVRTC out of resources, ...) stays with the table-driven sweep
-      m->bigTried = true;
-      if (big_supported (m, nullptr) && big_prepare (m)) {
-        if (m->opt.get ("verbose", 0)) fprintf (stderr, "big engine: not available for this machine (%s); using the wide engine\n", mb_last_error());
-        big_destroy (m);
-      }
-    }
-    if (big_wanted_viterbi (m, b)) return big_viterbi (m, b, score, pathLen);
-  }
-  if (!m->wide) return generic_viterbi (m, b, score, pathLen);
   WHost* h = wh (m);
   const bool trace = pathLen != nullptr;
   const std::vector<int64_t> order = cost_order (b, nullptr);
-  WBuf dRes;
+  DevBuf dRes;
   if (dRes.alloc ((size_t) b->nPairs * 8)) return 1;
   if (!trace) {
     if (timing_begin (b)) return 1;
@@ -908,9 +847,7 @@ int wide_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen) {
   size_t freeB = 0, totalB = 0;
   MB_CUDA (cudaMemGetInfo (&freeB, &totalB));
   const double budget = 0.75 * (double) freeB;
-  b->pathStart.assign ((size_t) b->nPairs, 0);
-  b->pathLen.assign ((size_t) b->nPairs, 0);
-  int64_t packed = 0, launches = 0;
+  int64_t launches = 0;
   double ms = 0;
   for (size_t c0 = 0; c0 < order.size();) {
     std::vector<int64_t> chunk, bpOff;
@@ -926,8 +863,9 @@ int wide_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen) {
       bytes += (need + 15) - fmod (need + 15, 16);
     }
     c0 = c1;
-    WBuf dBp, dBpOff, dOrder, dLen, dOutOff;
-    if (dBp.alloc ((size_t) bytes) || dBpOff.alloc (bpOff.size() * 8) || dOrder.alloc (chunk.size() * 8) || dLen.alloc (chunk.size() * 8)) return 1;
+    DevBuf dBp, dBpOff, dOrder, dLen, dOutOff;
+    if (dBp.alloc ((size_t) bytes) || dBpOff.alloc (bpOff.size() * 8) || dOrder.alloc (chunk.size() * 8) || dLen.alloc (chunk.size() * 8)
+        || dOutOff.alloc (chunk.size() * 8)) return 1;
     MB_CUDA (cudaMemcpyAsync (dBpOff.p, bpOff.data(), bpOff.size() * 8, cudaMemcpyHostToDevice, b->stream));
     MB_CUDA (cudaMemcpyAsync (dOrder.p, chunk.data(), chunk.size() * 8, cudaMemcpyHostToDevice, b->stream));
     if (timing_begin (b)) return 1;
@@ -937,18 +875,7 @@ int wide_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen) {
     wide_traceback_kernel<<<tg, 32, 0, b->stream>>> (m->dev, b->dev, dOrder.as<int64_t>(), nWork, dBp.as<unsigned char>(), dBpOff.as<int64_t>(), h->t.bpBytes, 0,
                                                       dRes.as<double>(), dLen.as<int64_t>(), nullptr, nullptr);
     MB_CUDA (cudaGetLastError());
-    std::vector<int64_t> len (chunk.size()), off (chunk.size());
-    MB_CUDA (cudaMemcpyAsync (len.data(), dLen.p, len.size() * 8, cudaMemcpyDeviceToHost, b->stream));
-    MB_CUDA (cudaStreamSynchronize (b->stream));
-    for (size_t n = 0; n < len.size(); ++n) {
-      off[n] = packed;
-      b->pathStart[chunk[n]] = packed;
-      b->pathLen[chunk[n]] = len[n];
-      packed += len[n];
-    }
-    if (paths_reserve (b, packed)) return 1;
-    if (dOutOff.alloc (off.size() * 8)) return 1;
-    MB_CUDA (cudaMemcpyAsync (dOutOff.p, off.data(), off.size() * 8, cudaMemcpyHostToDevice, b->stream));
+    if (paths_place (b, chunk.data(), nWork, dLen.as<int64_t>(), dOutOff.as<int64_t>())) return 1;
     wide_traceback_kernel<<<tg, 32, 0, b->stream>>> (m->dev, b->dev, dOrder.as<int64_t>(), nWork, dBp.as<unsigned char>(), dBpOff.as<int64_t>(), h->t.bpBytes, 0,
                                                       dRes.as<double>(), dLen.as<int64_t>(), b->dPaths, dOutOff.as<int64_t>());
     MB_CUDA (cudaGetLastError());
@@ -959,8 +886,6 @@ int wide_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen) {
   b->lastMs = ms;
   b->lastLaunches = launches;
   MB_CUDA (cudaMemcpy (score, dRes.p, (size_t) b->nPairs * 8, cudaMemcpyDeviceToHost));
-  // paths were packed in chunk order; mb_viterbi_paths copies them out by pathStart
-  for (int64_t k = 0; k < b->nPairs; ++k) pathLen[k] = b->pathLen[k];
   return 0;
 }
 
