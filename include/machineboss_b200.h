@@ -142,6 +142,19 @@ int mb_counts (mb_machine* m, mb_batch* b, double* counts, double* loglike);
 #define MB_MATRIX_VITERBI  2
 int mb_matrix (mb_machine* m, mb_batch* b, int64_t pair, int32_t kind, double* cells);
 
+/* ---- ForwardMatrix::samplePath (src/forward.cpp:17-23) for every pair of the batch, nSamples paths each, drawn on the device ----
+ * Path j of pair k has length pathLen[k * nSamples + j] (0 when loglike[k] is -inf); loglike (may be NULL) receives the
+ * Forward log-likelihoods of the stored matrices (the generic engine's values).  Draws are keyed by (seed, k, j): the same
+ * triple gives the same path on any device and under any chunking.  Each step draws a candidate in proportion to
+ * exp (F(previous cell) + log-weight), shifted by the step's largest candidate so that long pairs do not underflow, with
+ * Philox4x32-10 (key = seed, counter = { step, j, k & 0xffffffff, k >> 32 }).  The reference's mt19937 stream is not
+ * reproduced (ForwardMatrix::samplePath in the host mirror does that).  The paths are kept apart from mb_viterbi's: neither
+ * call overwrites the other's.  A failed call leaves no samples stored. */
+int mb_sample_paths (mb_machine* m, mb_batch* b, int32_t nSamples, uint64_t seed, double* loglike, int64_t* pathLen);
+/* The ids of the last mb_sample_paths on this batch, narrowed to bytesPerId = 1, 2 or 4 as in mb_viterbi_paths_narrow:
+ * path r = k * nSamples + j goes to elements pathOff[r] .. pathOff[r] + pathLen[r]. */
+int mb_sampled_paths (mb_batch* b, void* pathTrans, int32_t bytesPerId, const int64_t* pathOff);
+
 /* ---- one list of pairs over several GPUs of a box (SURVEY.md 8e) ----
  * Replaces the reference's single-core loops over a SeqPairList: MachineCounts (counts.cpp:37-43) inside
  * MachineFitter::fit (fitter.cpp:23-47), and the -L / -A loops of the CLI (boss.cpp:796,826).  The pairs are

@@ -21,7 +21,7 @@ _lib = None
 SYMBOLS = ["mb_last_error", "mb_version", "mb_set_kernel_cache_dir", "mb_device_count", "mb_set_device", "mb_set_engine", "mb_set_option", "mb_machine_set_option",
            "mb_machine_create", "mb_machine_update_weights", "mb_machine_info", "mb_machine_destroy",
            "mb_batch_create", "mb_batch_destroy", "mb_batch_trim", "mb_batch_set_envelopes", "mb_forward", "mb_backward", "mb_viterbi",
-           "mb_viterbi_paths", "mb_viterbi_paths_narrow", "mb_viterbi_paths_start", "mb_batch_wait", "mb_counts", "mb_matrix", "mb_last_kernel_ms", "mb_last_redo", "mb_jit_compile_check", "mb_jit_host_tables", "mb_lane_emulate", "mb_col_emulate",
+           "mb_viterbi_paths", "mb_viterbi_paths_narrow", "mb_viterbi_paths_start", "mb_batch_wait", "mb_counts", "mb_matrix", "mb_sample_paths", "mb_sampled_paths", "mb_last_kernel_ms", "mb_last_redo", "mb_jit_compile_check", "mb_jit_host_tables", "mb_lane_emulate", "mb_col_emulate",
            "mb_shard_pairs", "mb_group_create", "mb_group_info", "mb_group_destroy", "mb_group_machine_create", "mb_group_machine_update_weights",
            "mb_group_machine_set_option", "mb_group_machine_info", "mb_group_machine_destroy", "mb_group_batch_create", "mb_group_batch_set_envelopes",
            "mb_group_batch_shard", "mb_group_batch_destroy", "mb_group_forward", "mb_group_backward", "mb_group_viterbi", "mb_group_viterbi_paths",
@@ -66,6 +66,8 @@ def lib():
         L.mb_batch_wait.argtypes = [P]
         L.mb_counts.argtypes = [P, P, P, P]
         L.mb_matrix.argtypes = [P, P, I64, I32, P]
+        L.mb_sample_paths.argtypes = [P, P, I32, ctypes.c_uint64, P, P]
+        L.mb_sampled_paths.argtypes = [P, P, I32, P]
         L.mb_jit_compile_check.argtypes = [I32, I32, I32, I64, P, P, P, P, ctypes.c_char_p, I64]
         L.mb_jit_host_tables.argtypes = [I32, I32, I32, I64, P, P, P, P, P, I32, P, I64, ctypes.POINTER(I64)]
         L.mb_lane_emulate.argtypes = [I32, I32, I32, I64, P, P, P, P, P, P, I64, I32, ctypes.POINTER(D), P, P]
@@ -387,6 +389,21 @@ def matrix(m: Machine, b: Batch, pair: int, kind: int = 0) -> np.ndarray:
     out = np.empty((lo + 1, li + 1, m.n_states), dtype=np.float64)
     _check(lib().mb_matrix(m.h, b.h, int(pair), int(kind), _ptr(out)))
     return out
+
+
+def sample_paths(m: Machine, b: Batch, n: int, seed: int, bytes_per_id: int = 4):
+    """ForwardMatrix::samplePath for every pair, n paths each, drawn on the device (mb_sample_paths).  Returns (loglike[nPairs],
+    lengths[nPairs, n], offsets[nPairs * n + 1], ids): path j of pair k is ids[offsets[k * n + j]:offsets[k * n + j + 1]], ids
+    int32, or uint8 / uint16 with bytes_per_id 1 / 2."""
+    ll = np.empty(max(b.n_pairs, 1), dtype=np.float64)
+    plen = np.zeros(max(b.n_pairs * n, 1), dtype=np.int64)
+    _check(lib().mb_sample_paths(m.h, b.h, int(n), int(seed) & 0xFFFFFFFFFFFFFFFF, ll.ctypes.data, plen.ctypes.data))
+    plen = plen[: b.n_pairs * n]
+    off = np.concatenate([[0], np.cumsum(plen)]).astype(np.int64)
+    ids = np.empty(int(off[-1]), dtype={1: np.uint8, 2: np.uint16, 4: np.int32}[bytes_per_id])
+    if off[-1]:
+        _check(lib().mb_sampled_paths(b.h, _ptr(ids), int(bytes_per_id), _ptr(off)))
+    return ll[: b.n_pairs], plen.reshape(b.n_pairs, n), off, ids
 
 
 def counts(m: Machine, b: Batch):

@@ -164,35 +164,35 @@ static void pooled_free (int device, void* p, size_t bytes) {
   } else cudaFree (p);
 }
 
-// room for `need` packed path entries in b->dPaths, keeping what is already there (chunked tracebacks append)
-int paths_reserve (mb_batch* b, int64_t need) {
-  if (need <= b->pathsCapacity) return 0;
-  const int64_t want = std::max<int64_t> (need, 2 * b->pathsCapacity);
+// room for `need` packed path entries in ps.dPaths, keeping what is already there (chunked tracebacks append)
+int paths_reserve (mb_batch* b, PathStore& ps, int64_t need) {
+  if (need <= ps.pathsCapacity) return 0;
+  const int64_t want = std::max<int64_t> (need, 2 * ps.pathsCapacity);
   size_t got = 0;
   int32_t* p = (int32_t*) pooled_alloc (b->device, (size_t) want * 4, &got);
   if (!p) return 1;
-  if (b->dPaths) {
-    MB_CUDA (cudaMemcpyAsync (p, b->dPaths, (size_t) b->pathsCapacity * 4, cudaMemcpyDeviceToDevice, b->stream));
+  if (ps.dPaths) {
+    MB_CUDA (cudaMemcpyAsync (p, ps.dPaths, (size_t) ps.pathsCapacity * 4, cudaMemcpyDeviceToDevice, b->stream));
     MB_CUDA (cudaStreamSynchronize (b->stream));
-    pooled_free (b->device, b->dPaths, b->pathsBytes);
+    pooled_free (b->device, ps.dPaths, ps.pathsBytes);
   }
-  b->dPaths = p;
-  b->pathsBytes = got;
-  b->pathsCapacity = (int64_t) (got / 4);
+  ps.dPaths = p;
+  ps.pathsBytes = got;
+  ps.pathsCapacity = (int64_t) (got / 4);
   return 0;
 }
 
-int paths_place (mb_batch* b, const int64_t* pairs, int64_t n, const int64_t* dLen, int64_t* dOutOff) {
+int paths_place (mb_batch* b, PathStore& ps, const int64_t* rows, int64_t n, const int64_t* dLen, int64_t* dOutOff) {
   std::vector<int64_t> len ((size_t) n), off ((size_t) n);
   MB_CUDA (cudaMemcpyAsync (len.data(), dLen, (size_t) n * 8, cudaMemcpyDeviceToHost, b->stream));
   MB_CUDA (cudaStreamSynchronize (b->stream));
   for (int64_t q = 0; q < n; ++q) {
-    off[q] = b->pathsPacked;
-    b->pathStart[pairs[q]] = b->pathsPacked;
-    b->pathLen[pairs[q]] = len[q];
-    b->pathsPacked += len[q];
+    off[q] = ps.pathsPacked;
+    ps.pathStart[rows[q]] = ps.pathsPacked;
+    ps.pathLen[rows[q]] = len[q];
+    ps.pathsPacked += len[q];
   }
-  if (paths_reserve (b, b->pathsPacked)) return 1;
+  if (paths_reserve (b, ps, ps.pathsPacked)) return 1;
   MB_CUDA (cudaMemcpyAsync (dOutOff, off.data(), (size_t) n * 8, cudaMemcpyHostToDevice, b->stream));
   return 0;
 }
@@ -555,7 +555,8 @@ void mb_batch_destroy (mb_batch* b) {
   cudaSetDevice (b->device);
   if (b->dEnv) cudaFree (b->dEnv);
   pooled_free (b->device, b->dTokBlock, b->tokBytes);
-  pooled_free (b->device, b->dPaths, b->pathsBytes);
+  pooled_free (b->device, b->viterbiPaths.dPaths, b->viterbiPaths.pathsBytes);
+  pooled_free (b->device, b->sampledPaths.dPaths, b->sampledPaths.pathsBytes);
   ws_release_all (b);
   if (b->copyStream) { cudaStreamSynchronize (b->copyStream); cudaStreamDestroy (b->copyStream); }
   if (b->evCopy) cudaEventDestroy (b->evCopy);
@@ -587,14 +588,15 @@ static int check_call (const mb_machine* m, const mb_batch* b) {
   return 0;
 }
 
-enum Pass { PASS_FORWARD, PASS_VITERBI_PATHS, PASS_VITERBI_SCORES, PASS_BACKWARD, PASS_COUNTS, PASS_MATRIX };
+enum Pass { PASS_FORWARD, PASS_VITERBI_PATHS, PASS_VITERBI_SCORES, PASS_BACKWARD, PASS_COUNTS, PASS_MATRIX, PASS_SAMPLE };
 enum Route { ROUTE_ERROR = -1, ROUTE_NONE, ROUTE_JIT, ROUTE_BIG, ROUTE_COL, ROUTE_LANE, ROUTE_WIDE, ROUTE_GENERIC };
 
 // The engine that serves a call, after any lazy preparation it needs (ROUTE_NONE: nothing to do; ROUTE_ERROR: a preparation
 // failed, error set).  A failed preparation destroys what it built, so the engine's handle is null again.
 static int route_of (mb_machine* m, mb_batch* b, Pass pass) {
   const bool sweep = pass == PASS_FORWARD || pass == PASS_VITERBI_PATHS || pass == PASS_VITERBI_SCORES;
-  if (pass == PASS_MATRIX || m->engine == MB_ENGINE_GENERIC) return ROUTE_GENERIC;
+  // stored matrices (a pair's whole matrix, sampled paths) exist only in the generic engine
+  if (pass == PASS_MATRIX || pass == PASS_SAMPLE || m->engine == MB_ENGINE_GENERIC) return ROUTE_GENERIC;
   if (m->engine == MB_ENGINE_JIT) {
     // the strip kernels sweep full matrices; with envelopes the wide engine takes the sweeps it can, the generic engine the rest
     if (!b->hasEnv) return ROUTE_JIT;
@@ -633,7 +635,7 @@ static int route_of (mb_machine* m, mb_batch* b, Pass pass) {
 static int route (mb_machine* m, mb_batch* b, Pass pass) {
   const int r = route_of (m, b, pass);
   if (r != ROUTE_ERROR && m->opt.get ("verbose", 0)) {
-    static const char* const passNames[] = { "mb_forward", "mb_viterbi", "mb_viterbi (scores)", "mb_backward", "mb_counts", "mb_matrix" };
+    static const char* const passNames[] = { "mb_forward", "mb_viterbi", "mb_viterbi (scores)", "mb_backward", "mb_counts", "mb_matrix", "mb_sample_paths" };
     static const char* const engineNames[] = { "no engine (empty batch)", "jit engine", "big engine", "column engine", "lane engine", "wide engine", "generic engine" };
     fprintf (stderr, "%s: %s\n", passNames[pass], engineNames[r]);
   }
@@ -663,14 +665,15 @@ int mb_backward (mb_machine* m, mb_batch* b, double* loglike) {
 int mb_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen) {
   if (check_call (m, b)) return 1;
   if (b->copyStream) MB_CUDA (cudaStreamSynchronize (b->copyStream));      // paths of the previous call still on their way out
-  b->pathIdLimit = m->T;
-  b->pathStart.clear();
-  b->pathLen.clear();
+  PathStore& ps = b->viterbiPaths;
+  ps.pathIdLimit = m->T;
+  ps.pathStart.clear();
+  ps.pathLen.clear();
   const int r = route (m, b, pathLen ? PASS_VITERBI_PATHS : PASS_VITERBI_SCORES);
   if (pathLen) {      // the engine places each pair's path with paths_place
-    b->pathStart.assign ((size_t) b->nPairs, 0);
-    b->pathLen.assign ((size_t) b->nPairs, 0);
-    b->pathsPacked = 0;
+    ps.pathStart.assign ((size_t) b->nPairs, 0);
+    ps.pathLen.assign ((size_t) b->nPairs, 0);
+    ps.pathsPacked = 0;
   }
   int rc = 1;
   switch (r) {
@@ -682,72 +685,85 @@ int mb_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen) {
     case ROUTE_WIDE: rc = wide_viterbi (m, b, score, pathLen); break;
     case ROUTE_GENERIC: rc = generic_viterbi (m, b, score, pathLen); break;
   }
-  if (rc) { b->pathStart.clear(); b->pathLen.clear(); return 1; }      // no traceback stored
-  if (pathLen) for (int64_t k = 0; k < b->nPairs; ++k) pathLen[k] = b->pathLen[k];
+  if (rc) { ps.pathStart.clear(); ps.pathLen.clear(); return 1; }      // no traceback stored
+  if (pathLen) for (int64_t k = 0; k < b->nPairs; ++k) pathLen[k] = ps.pathLen[k];
   return 0;
 }
 
 int mb_viterbi_paths (mb_batch* b, int32_t* pathTrans, const int64_t* pathOff) {
   if (!b) { set_error ("null batch"); return 1; }
-  if ((int64_t) b->pathLen.size() != b->nPairs) { set_error ("mb_viterbi_paths: no traceback stored; call mb_viterbi with pathLen first"); return 1; }
+  const PathStore& ps = b->viterbiPaths;
+  if ((int64_t) ps.pathLen.size() != b->nPairs) { set_error ("mb_viterbi_paths: no traceback stored; call mb_viterbi with pathLen first"); return 1; }
   MB_CUDA (cudaSetDevice (b->device));
   // paths are packed on the device in pair order; one D2H copy, then scatter to the caller's offsets
   int64_t total = 0;
-  for (int64_t k = 0; k < b->nPairs; ++k) total += b->pathLen[k];
+  for (int64_t k = 0; k < b->nPairs; ++k) total += ps.pathLen[k];
   if (!total) return 0;
   bool contiguous = true;
-  for (int64_t k = 0; k < b->nPairs && contiguous; ++k) contiguous = (pathOff[k] - pathOff[0] == b->pathStart[k]);
+  for (int64_t k = 0; k < b->nPairs && contiguous; ++k) contiguous = (pathOff[k] - pathOff[0] == ps.pathStart[k]);
   if (contiguous) {
-    MB_CUDA (cudaMemcpy (pathTrans + pathOff[0], b->dPaths, (size_t) total * 4, cudaMemcpyDeviceToHost));
+    MB_CUDA (cudaMemcpy (pathTrans + pathOff[0], ps.dPaths, (size_t) total * 4, cudaMemcpyDeviceToHost));
     return 0;
   }
   std::vector<int32_t> tmp ((size_t) total);
-  MB_CUDA (cudaMemcpy (tmp.data(), b->dPaths, (size_t) total * 4, cudaMemcpyDeviceToHost));
+  MB_CUDA (cudaMemcpy (tmp.data(), ps.dPaths, (size_t) total * 4, cudaMemcpyDeviceToHost));
   for (int64_t k = 0; k < b->nPairs; ++k)
-    memcpy (pathTrans + pathOff[k], tmp.data() + b->pathStart[k], (size_t) b->pathLen[k] * 4);
+    memcpy (pathTrans + pathOff[k], tmp.data() + ps.pathStart[k], (size_t) ps.pathLen[k] * 4);
+  return 0;
+}
+
+// The stored paths of ps (as many as ps.pathLen holds) with ids of bytesPerId = 1, 2 or 4 bytes, path r to pathTrans[pathOff[r] ..)
+static int copy_paths (mb_batch* b, const PathStore& ps, void* pathTrans, int32_t bytesPerId, const int64_t* pathOff) {
+  MB_CUDA (cudaSetDevice (b->device));
+  const int64_t n = (int64_t) ps.pathLen.size();
+  int64_t total = 0;
+  for (int64_t r = 0; r < n; ++r) total += ps.pathLen[r];
+  if (!total) return 0;
+  bool contiguous = true;      // the engines pack in their own order (JIT: pair order; wide, lane: longest first)
+  for (int64_t r = 0; r < n && contiguous; ++r) contiguous = (pathOff[r] - pathOff[0] == ps.pathStart[r]);
+  const void* src = ps.dPaths;
+  if (bytesPerId < 4) {
+    void* tmp = ws_reserve (b, WS_PATHNARROW, (size_t) total * bytesPerId);
+    if (!tmp) return 1;
+    const unsigned grid = (unsigned) std::min<int64_t> ((total + 255) / 256, 148 * 16);
+    if (bytesPerId == 1) narrow_ids_kernel<uint8_t><<<grid, 256, 0, b->stream>>> (ps.dPaths, (uint8_t*) tmp, total);
+    else narrow_ids_kernel<uint16_t><<<grid, 256, 0, b->stream>>> (ps.dPaths, (uint16_t*) tmp, total);
+    MB_CUDA (cudaGetLastError());
+    src = tmp;
+  }
+  if (contiguous) {
+    MB_CUDA (cudaMemcpyAsync ((char*) pathTrans + pathOff[0] * bytesPerId, src, (size_t) total * bytesPerId, cudaMemcpyDeviceToHost, b->stream));
+    MB_CUDA (cudaStreamSynchronize (b->stream));
+    return 0;
+  }
+  std::vector<char> host ((size_t) total * bytesPerId);
+  MB_CUDA (cudaMemcpyAsync (host.data(), src, host.size(), cudaMemcpyDeviceToHost, b->stream));
+  MB_CUDA (cudaStreamSynchronize (b->stream));
+  for (int64_t r = 0; r < n; ++r)
+    memcpy ((char*) pathTrans + pathOff[r] * bytesPerId, host.data() + ps.pathStart[r] * bytesPerId, (size_t) ps.pathLen[r] * bytesPerId);
   return 0;
 }
 
 int mb_viterbi_paths_narrow (mb_batch* b, void* pathTrans, int32_t bytesPerId, const int64_t* pathOff) {
   if (!b) { set_error ("null batch"); return 1; }
-  if ((int64_t) b->pathLen.size() != b->nPairs) { set_error ("mb_viterbi_paths_narrow: no traceback stored; call mb_viterbi with pathLen first"); return 1; }
+  const PathStore& ps = b->viterbiPaths;
+  if ((int64_t) ps.pathLen.size() != b->nPairs) { set_error ("mb_viterbi_paths_narrow: no traceback stored; call mb_viterbi with pathLen first"); return 1; }
   if (bytesPerId == 4) return mb_viterbi_paths (b, (int32_t*) pathTrans, pathOff);
   if (bytesPerId != 1 && bytesPerId != 2) { set_error ("mb_viterbi_paths_narrow: bytesPerId must be 1, 2 or 4"); return 1; }
-  if (b->pathIdLimit > (bytesPerId == 1 ? 256 : 65536)) { set_error ("mb_viterbi_paths_narrow: the machine's transition ids do not fit in " + std::to_string (bytesPerId) + " byte(s)"); return 1; }
-  MB_CUDA (cudaSetDevice (b->device));
-  int64_t total = 0;
-  for (int64_t k = 0; k < b->nPairs; ++k) total += b->pathLen[k];
-  if (!total) return 0;
-  bool contiguous = true;      // the engines pack in their own order (JIT: pair order; wide, lane: longest first)
-  for (int64_t k = 0; k < b->nPairs && contiguous; ++k) contiguous = (pathOff[k] - pathOff[0] == b->pathStart[k]);
-  void* tmp = ws_reserve (b, WS_PATHNARROW, (size_t) total * bytesPerId);
-  if (!tmp) return 1;
-  const unsigned grid = (unsigned) std::min<int64_t> ((total + 255) / 256, 148 * 16);
-  if (bytesPerId == 1) narrow_ids_kernel<uint8_t><<<grid, 256, 0, b->stream>>> (b->dPaths, (uint8_t*) tmp, total);
-  else narrow_ids_kernel<uint16_t><<<grid, 256, 0, b->stream>>> (b->dPaths, (uint16_t*) tmp, total);
-  MB_CUDA (cudaGetLastError());
-  if (contiguous) {
-    MB_CUDA (cudaMemcpyAsync ((char*) pathTrans + pathOff[0] * bytesPerId, tmp, (size_t) total * bytesPerId, cudaMemcpyDeviceToHost, b->stream));
-    MB_CUDA (cudaStreamSynchronize (b->stream));
-    return 0;
-  }
-  std::vector<char> host ((size_t) total * bytesPerId);
-  MB_CUDA (cudaMemcpyAsync (host.data(), tmp, host.size(), cudaMemcpyDeviceToHost, b->stream));
-  MB_CUDA (cudaStreamSynchronize (b->stream));
-  for (int64_t k = 0; k < b->nPairs; ++k)
-    memcpy ((char*) pathTrans + pathOff[k] * bytesPerId, host.data() + b->pathStart[k] * bytesPerId, (size_t) b->pathLen[k] * bytesPerId);
-  return 0;
+  if (ps.pathIdLimit > (bytesPerId == 1 ? 256 : 65536)) { set_error ("mb_viterbi_paths_narrow: the machine's transition ids do not fit in " + std::to_string (bytesPerId) + " byte(s)"); return 1; }
+  return copy_paths (b, ps, pathTrans, bytesPerId, pathOff);
 }
 
 int mb_viterbi_paths_start (mb_batch* b, void* pathTrans, int32_t bytesPerId, const int64_t* pathOff) {
   if (!b) { set_error ("null batch"); return 1; }
-  if ((int64_t) b->pathLen.size() != b->nPairs) { set_error ("mb_viterbi_paths_start: no traceback stored; call mb_viterbi with pathLen first"); return 1; }
+  const PathStore& ps = b->viterbiPaths;
+  if ((int64_t) ps.pathLen.size() != b->nPairs) { set_error ("mb_viterbi_paths_start: no traceback stored; call mb_viterbi with pathLen first"); return 1; }
   if (bytesPerId != 1 && bytesPerId != 2 && bytesPerId != 4) { set_error ("mb_viterbi_paths_start: bytesPerId must be 1, 2 or 4"); return 1; }
-  if (bytesPerId < 4 && b->pathIdLimit > (bytesPerId == 1 ? 256 : 65536)) { set_error ("mb_viterbi_paths_start: the machine's transition ids do not fit in " + std::to_string (bytesPerId) + " byte(s)"); return 1; }
+  if (bytesPerId < 4 && ps.pathIdLimit > (bytesPerId == 1 ? 256 : 65536)) { set_error ("mb_viterbi_paths_start: the machine's transition ids do not fit in " + std::to_string (bytesPerId) + " byte(s)"); return 1; }
   int64_t total = 0;
-  for (int64_t k = 0; k < b->nPairs; ++k) total += b->pathLen[k];
+  for (int64_t k = 0; k < b->nPairs; ++k) total += ps.pathLen[k];
   bool contiguous = true;
-  for (int64_t k = 0; k < b->nPairs && contiguous; ++k) contiguous = (pathOff[k] - pathOff[0] == b->pathStart[k]);
+  for (int64_t k = 0; k < b->nPairs && contiguous; ++k) contiguous = (pathOff[k] - pathOff[0] == ps.pathStart[k]);
   if (!contiguous) return mb_viterbi_paths_narrow (b, pathTrans, bytesPerId, pathOff);      // scattered offsets: the blocking path
   if (!total) return 0;
   MB_CUDA (cudaSetDevice (b->device));
@@ -755,13 +771,13 @@ int mb_viterbi_paths_start (mb_batch* b, void* pathTrans, int32_t bytesPerId, co
     MB_CUDA (cudaStreamCreateWithFlags (&b->copyStream, cudaStreamNonBlocking));
     MB_CUDA (cudaEventCreateWithFlags (&b->evCopy, cudaEventDisableTiming));
   }
-  const void* src = b->dPaths;
+  const void* src = ps.dPaths;
   if (bytesPerId < 4) {
     void* tmp = ws_reserve (b, WS_PATHNARROW, (size_t) total * bytesPerId);
     if (!tmp) return 1;
     const unsigned grid = (unsigned) std::min<int64_t> ((total + 255) / 256, 148 * 16);
-    if (bytesPerId == 1) narrow_ids_kernel<uint8_t><<<grid, 256, 0, b->stream>>> (b->dPaths, (uint8_t*) tmp, total);
-    else narrow_ids_kernel<uint16_t><<<grid, 256, 0, b->stream>>> (b->dPaths, (uint16_t*) tmp, total);
+    if (bytesPerId == 1) narrow_ids_kernel<uint8_t><<<grid, 256, 0, b->stream>>> (ps.dPaths, (uint8_t*) tmp, total);
+    else narrow_ids_kernel<uint16_t><<<grid, 256, 0, b->stream>>> (ps.dPaths, (uint16_t*) tmp, total);
     MB_CUDA (cudaGetLastError());
     src = tmp;
   }
@@ -788,6 +804,32 @@ int mb_matrix (mb_machine* m, mb_batch* b, int64_t pair, int32_t kind, double* c
   if (!cells) { set_error ("mb_matrix: null output"); return 1; }
   route (m, b, PASS_MATRIX);
   return generic_matrix (m, b, pair, kind, cells);
+}
+
+int mb_sample_paths (mb_machine* m, mb_batch* b, int32_t nSamples, uint64_t seed, double* loglike, int64_t* pathLen) {
+  if (check_call (m, b)) return 1;
+  b->samplesPerPair = 0;      // a failed call leaves no samples stored
+  if (nSamples < 1) { set_error ("mb_sample_paths: nSamples must be at least 1"); return 1; }
+  PathStore& ps = b->sampledPaths;
+  const size_t nPaths = (size_t) b->nPairs * (size_t) nSamples;
+  ps.pathIdLimit = m->T;
+  ps.pathStart.assign (nPaths, 0);      // placed by paths_place, path k * nSamples + j
+  ps.pathLen.assign (nPaths, 0);
+  ps.pathsPacked = 0;
+  route (m, b, PASS_SAMPLE);
+  if (generic_sample_paths (m, b, nSamples, seed, loglike)) { ps.pathStart.clear(); ps.pathLen.clear(); return 1; }      // no samples stored
+  b->samplesPerPair = nSamples;
+  if (pathLen) for (size_t r = 0; r < nPaths; ++r) pathLen[r] = ps.pathLen[r];
+  return 0;
+}
+
+int mb_sampled_paths (mb_batch* b, void* pathTrans, int32_t bytesPerId, const int64_t* pathOff) {
+  if (!b) { set_error ("null batch"); return 1; }
+  const PathStore& ps = b->sampledPaths;
+  if (b->samplesPerPair == 0) { set_error ("mb_sampled_paths: no samples stored; call mb_sample_paths first"); return 1; }
+  if (bytesPerId != 1 && bytesPerId != 2 && bytesPerId != 4) { set_error ("mb_sampled_paths: bytesPerId must be 1, 2 or 4"); return 1; }
+  if (bytesPerId < 4 && ps.pathIdLimit > (bytesPerId == 1 ? 256 : 65536)) { set_error ("mb_sampled_paths: the machine's transition ids do not fit in " + std::to_string (bytesPerId) + " byte(s)"); return 1; }
+  return copy_paths (b, ps, pathTrans, bytesPerId, pathOff);
 }
 
 int mb_jit_compile_check (int32_t nStates, int32_t nInTok, int32_t nOutTok, int64_t nTrans,

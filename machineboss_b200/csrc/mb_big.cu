@@ -671,8 +671,8 @@ int big_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen) {
     const unsigned tg = (unsigned) ((nWork + 63) / 64);
     big_traceback_kernel<<<tg, 64, 0, b->stream>>> (tp, b->dev, dOrder.as<int64_t>(), nWork, dBp.as<unsigned>(), dBpOff.as<int64_t>(), dRes, dLen.as<int64_t>(), nullptr, nullptr);
     MB_CUDA (cudaGetLastError());
-    if (paths_place (b, chunk.data(), nWork, dLen.as<int64_t>(), dOutOff.as<int64_t>())) return 1;
-    big_traceback_kernel<<<tg, 64, 0, b->stream>>> (tp, b->dev, dOrder.as<int64_t>(), nWork, dBp.as<unsigned>(), dBpOff.as<int64_t>(), dRes, dLen.as<int64_t>(), b->dPaths, dOutOff.as<int64_t>());
+    if (paths_place (b, b->viterbiPaths, chunk.data(), nWork, dLen.as<int64_t>(), dOutOff.as<int64_t>())) return 1;
+    big_traceback_kernel<<<tg, 64, 0, b->stream>>> (tp, b->dev, dOrder.as<int64_t>(), nWork, dBp.as<unsigned>(), dBpOff.as<int64_t>(), dRes, dLen.as<int64_t>(), b->viterbiPaths.dPaths, dOutOff.as<int64_t>());
     MB_CUDA (cudaGetLastError());
     launches += 3;
     if (timing_end (b, launches)) return 1;

@@ -749,7 +749,7 @@ __global__ void __launch_bounds__(64) col_traceback_kernel (ColTbPlan p, const u
   if (!out) lenOut[n] = len;
 }
 
-// scores (dResult, by read) and paths (b->dPaths, b->pathStart / pathLen) of every read in `order`; *ms receives the device time
+// scores (dResult, by read) and paths (b->viterbiPaths) of every read in `order`; *ms receives the device time
 static int col_viterbi_paths (mb_machine* m, mb_batch* b, const std::vector<int64_t>& order, double* dResult, int64_t* launches, double* msOut) {
   ColEngine& E = *ce (m);
   const ColProg& p = E.prog;
@@ -821,8 +821,8 @@ static int col_viterbi_paths (mb_machine* m, mb_batch* b, const std::vector<int6
     const unsigned tbGrid = (unsigned) ((nWork + 63) / 64);
     col_traceback_kernel<<<tbGrid, 64, 0, b->stream>>> (T, b->dY, b->dYOff, dOrder, nWork, dBp, dOffs + nWork, dPreP, dSufP, dResult, dLen, nullptr, nullptr);
     MB_CUDA (cudaGetLastError());
-    if (paths_place (b, order.data() + c0, nWork, dLen, dOutOff)) return 1;
-    col_traceback_kernel<<<tbGrid, 64, 0, b->stream>>> (T, b->dY, b->dYOff, dOrder, nWork, dBp, dOffs + nWork, dPreP, dSufP, dResult, dLen, b->dPaths, dOutOff);
+    if (paths_place (b, b->viterbiPaths, order.data() + c0, nWork, dLen, dOutOff)) return 1;
+    col_traceback_kernel<<<tbGrid, 64, 0, b->stream>>> (T, b->dY, b->dYOff, dOrder, nWork, dBp, dOffs + nWork, dPreP, dSufP, dResult, dLen, b->viterbiPaths.dPaths, dOutOff);
     MB_CUDA (cudaGetLastError());
     if (launches) *launches += 5;
     if (timing_end (b, 5)) return 1;

@@ -14,6 +14,7 @@
 //   ViterbiMatrix::fill        viterbi.cpp:18-43      fill_kernel<OP_MAX, false>
 //   BackwardMatrix::fill       backward.cpp:18-46     fill_kernel<OP_SUM, true>
 //   DPMatrix::traceBack        dpmatrix.defs.h:82-110 traceback_kernel
+//   ForwardMatrix::samplePath  forward.cpp:17-23      sample_kernel
 //   BackwardMatrix::getCounts  backward.cpp:62-87     counts_kernel
 #include <algorithm>
 #include <cmath>
@@ -174,6 +175,90 @@ __global__ void traceback_kernel (DevMachine m, DevBatch b, const int64_t* __res
   if (!out) lenOut[slot] = n;
 }
 
+// Philox4x32-10 (Salmon, Moraes, Dror and Shaw, SC'11), as Random123's philox4x32 with 10 rounds: the counter-based generator
+// of sample_kernel.  Written out here, not taken from cuRAND, so that a host replay reproduces every draw bit for bit.
+__device__ __forceinline__ uint4 philox4x32_10 (uint4 c, uint2 key) {
+#pragma unroll
+  for (int r = 0; r < 10; ++r) {
+    if (r) { key.x += 0x9E3779B9u; key.y += 0xBB67AE85u; }
+    const uint32_t lo0 = 0xD2511F53u * c.x, hi0 = __umulhi (0xD2511F53u, c.x);
+    const uint32_t lo1 = 0xCD9E8D57u * c.z, hi1 = __umulhi (0xCD9E8D57u, c.z);
+    c = make_uint4 (hi1 ^ c.y ^ key.x, lo1, hi0 ^ c.w ^ key.y, lo0);
+  }
+  return c;
+}
+
+// ForwardMatrix::samplePath (forward.cpp:17-23, dpmatrix.defs.h:176-186) over stored Forward matrices: one thread per
+// (pair of the chunk, sample), thread q = slot * nSamples + j.  Each step rebuilds the candidates as traceback_kernel does
+// (match, delete, insert, silent; each by source state then transition index), weighs candidate n by
+// w_n = exp (v_n - max v), v_n = F(previous cell)[source] + log-weight (the reference's exp (v_n) underflows to all zeros once
+// Forward values fall below about -745), and takes the first candidate with w_n > 0 whose running sum exceeds u * sum w, or
+// failing that, after rounding, the last one with w_n > 0.  u is drawn with Philox4x32-10, key = seed, counter = (step, j, k):
+// a path depends only on (seed, pair index k, sample j) and the pair, never on the chunking.  With out == nullptr only the
+// length is computed; otherwise path q is written start -> end into out[outOff[q] ..).
+__global__ void sample_kernel (DevMachine m, DevBatch b, const int64_t* __restrict__ pairs, int64_t nSlots, int32_t nSamples, uint64_t seed,
+                               const int64_t* __restrict__ wsOff, const double* __restrict__ ws, const double* __restrict__ loglike,
+                               int64_t* __restrict__ lenOut, int32_t* __restrict__ out, const int64_t* __restrict__ outOff) {
+  const int64_t q = (int64_t) blockIdx.x * blockDim.x + threadIdx.x;
+  if (q >= nSlots * nSamples) return;
+  const int64_t slot = q / nSamples;
+  const uint32_t j = (uint32_t) (q - slot * nSamples);
+  const int64_t k = pairs[slot];
+  const uint8_t* x = b.x + b.xOff[k];
+  const uint8_t* y = b.y + b.yOff[k];
+  const int64_t Li = b.xOff[k + 1] - b.xOff[k], Lo = b.yOff[k + 1] - b.yOff[k];
+  const int S = m.S;
+  const Cells C = { const_cast<double*> (ws) + wsOff[slot], Li, S, 0 };
+  const uint2 key = make_uint2 ((uint32_t) seed, (uint32_t) (seed >> 32));
+  int64_t n = 0;
+  if (loglike[k] > neg_inf()) {
+    const int64_t total = out ? lenOut[q] : 0;
+    int64_t i = Li, o = Lo;
+    int s = S - 1;
+    while (i > 0 || o > 0 || s != 0) {
+      const int a = i ? x[i - 1] : 0, c = o ? y[o - 1] : 0;
+      const int64_t ks = (int64_t) s * m.nIn1;
+      auto visit = [&] (auto&& f) {      // f (list entry, value, type) over the candidates in order
+        auto list = [&] (int64_t listKey, const double* cell, int type) {
+          for (int64_t p = m.inc.off[listKey], e = m.inc.off[listKey + 1]; p < e; ++p) f (p, cell[m.inc.other[p]] + m.inc.lw[p], type);
+        };
+        if (i && o) list ((ks + a) * m.nOut1 + c, C.at (i - 1, o - 1), T_MATCH);
+        if (i) list ((ks + a) * m.nOut1, C.at (i - 1, o), T_DELETE);
+        if (o) list (ks * m.nOut1 + c, C.at (i, o - 1), T_INSERT);
+        list (ks * m.nOut1, C.at (i, o), T_SILENT);
+      };
+      double mx = neg_inf();
+      visit ([&] (int64_t, double v, int) { mx = fmax (mx, v); });
+      if (!(mx > neg_inf())) break;   // cannot happen on a path through finite cells
+      double norm = 0;
+      visit ([&] (int64_t, double v, int) { norm += exp (v - mx); });
+      const uint4 r = philox4x32_10 (make_uint4 ((uint32_t) n, j, (uint32_t) k, (uint32_t) ((uint64_t) k >> 32)), key);
+      const double thr = (double) (((uint64_t) r.x << 21) | (r.y >> 11)) * 0x1p-53 * norm;
+      double run = 0;
+      int64_t pick = -1, last = -1;
+      int pickType = 0, lastType = 0;
+      visit ([&] (int64_t p, double v, int type) {
+        if (pick >= 0) return;
+        const double w = exp (v - mx);
+        if (!(w > 0)) return;
+        run += w;
+        last = p; lastType = type;
+        if (run > thr) { pick = p; pickType = type; }
+      });
+      if (pick < 0) { pick = last; pickType = lastType; }
+      if (out) {
+        if (n >= total) break;   // cannot happen: the walk replays the length pass's
+        out[outOff[q] + total - 1 - n] = m.inc.id[pick];
+      }
+      ++n;
+      if (pickType == T_MATCH || pickType == T_DELETE) --i;
+      if (pickType == T_MATCH || pickType == T_INSERT) --o;
+      s = m.inc.other[pick];
+    }
+  }
+  if (!out) lenOut[q] = n;
+}
+
 // BackwardMatrix::getCounts (backward.cpp:62-87): count[t] += exp(F(src cell) - ll + w_t + B(dest cell)).
 // One CTA per pair; the CTA walks the transitions, each thread sums the cells where the
 // transition's labels match the tokens, then a block reduction and one atomic per transition.
@@ -320,8 +405,8 @@ int generic_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen
       const unsigned tg = (unsigned) ((ch.pairs.size() + 63) / 64);
       traceback_kernel<<<tg, 64, 0, b->stream>>> (m->dev, cb, dPairs.as<int64_t>(), dOff.as<int64_t>(), dWs.as<double>(), dRes.as<double>(), dLen.as<int64_t>(), nullptr, nullptr);
       MB_CUDA (cudaGetLastError());
-      if (paths_place (b, ch.pairs.data(), (int64_t) ch.pairs.size(), dLen.as<int64_t>(), dOutOff.as<int64_t>())) return 1;
-      traceback_kernel<<<tg, 64, 0, b->stream>>> (m->dev, cb, dPairs.as<int64_t>(), dOff.as<int64_t>(), dWs.as<double>(), dRes.as<double>(), dLen.as<int64_t>(), b->dPaths, dOutOff.as<int64_t>());
+      if (paths_place (b, b->viterbiPaths, ch.pairs.data(), (int64_t) ch.pairs.size(), dLen.as<int64_t>(), dOutOff.as<int64_t>())) return 1;
+      traceback_kernel<<<tg, 64, 0, b->stream>>> (m->dev, cb, dPairs.as<int64_t>(), dOff.as<int64_t>(), dWs.as<double>(), dRes.as<double>(), dLen.as<int64_t>(), b->viterbiPaths.dPaths, dOutOff.as<int64_t>());
       MB_CUDA (cudaGetLastError());
       launches += 2;
     }
@@ -331,6 +416,45 @@ int generic_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen
   b->lastMs = ms;
   b->lastLaunches = launches;
   MB_CUDA (cudaMemcpy (score, dRes.p, (size_t) b->nPairs * 8, cudaMemcpyDeviceToHost));
+  return 0;
+}
+
+// Per chunk: the full-storage Forward fill, the sampler's length pass, placement, the id pass (generic_viterbi's scheme).
+int generic_sample_paths (mb_machine* m, mb_batch* b, int32_t nSamples, uint64_t seed, double* loglike) {
+  b->lastMs = 0;
+  b->lastLaunches = 0;
+  if (b->nPairs == 0) return 0;
+  std::vector<Chunk> chunks;
+  if (plan_chunks (b, m->S, false, 1, chunks)) return 1;
+  DevBuf dRes;
+  if (dRes.alloc ((size_t) b->nPairs * 8)) return 1;
+  int64_t launches = 0;
+  double ms = 0;
+  for (auto& ch: chunks) {
+    const int64_t nSlots = (int64_t) ch.pairs.size(), nPaths = nSlots * nSamples;
+    std::vector<int64_t> rows ((size_t) nPaths);      // path q of the chunk is path k * nSamples + j of the batch
+    for (int64_t q = 0; q < nPaths; ++q) rows[q] = ch.pairs[q / nSamples] * nSamples + q % nSamples;
+    DevBuf dPairs, dOff, dWs, dLen, dOutOff;
+    if (upload (dPairs, ch.pairs, b->stream) || upload (dOff, ch.wsOff, b->stream) || dWs.alloc ((size_t) ch.doubles * 8)
+        || dLen.alloc ((size_t) nPaths * 8) || dOutOff.alloc ((size_t) nPaths * 8)) return 1;
+    if (timing_begin (b)) return 1;
+    fill_kernel<OP_SUM, false><<<(unsigned) nSlots, 256, 0, b->stream>>> (m->dev, b->dev, dPairs.as<int64_t>(), dOff.as<int64_t>(), dWs.as<double>(), 0, dRes.as<double>());
+    MB_CUDA (cudaGetLastError());
+    const unsigned sg = (unsigned) ((nPaths + 63) / 64);
+    sample_kernel<<<sg, 64, 0, b->stream>>> (m->dev, b->dev, dPairs.as<int64_t>(), nSlots, nSamples, seed, dOff.as<int64_t>(), dWs.as<double>(), dRes.as<double>(),
+                                             dLen.as<int64_t>(), nullptr, nullptr);
+    MB_CUDA (cudaGetLastError());
+    if (paths_place (b, b->sampledPaths, rows.data(), nPaths, dLen.as<int64_t>(), dOutOff.as<int64_t>())) return 1;
+    sample_kernel<<<sg, 64, 0, b->stream>>> (m->dev, b->dev, dPairs.as<int64_t>(), nSlots, nSamples, seed, dOff.as<int64_t>(), dWs.as<double>(), dRes.as<double>(),
+                                             dLen.as<int64_t>(), b->sampledPaths.dPaths, dOutOff.as<int64_t>());
+    MB_CUDA (cudaGetLastError());
+    launches += 3;
+    if (timing_end (b, launches)) return 1;
+    ms += b->lastMs;
+  }
+  b->lastMs = ms;
+  b->lastLaunches = launches;
+  if (loglike) MB_CUDA (cudaMemcpy (loglike, dRes.p, (size_t) b->nPairs * 8, cudaMemcpyDeviceToHost));
   return 0;
 }
 

@@ -80,6 +80,17 @@ bool cuda_ok (cudaError_t e, const char* what);
 
 #define MB_CUDA(call) do { if (!mb::cuda_ok ((call), #call)) return 1; } while (0)
 
+// Packed transition ids of a batch's stored paths (pooled device block) and where each path lies in it.  A batch keeps one
+// store for its Viterbi traceback and one for its sampled paths, so neither call overwrites the other's result.
+struct PathStore {
+  int32_t* dPaths = nullptr;
+  std::vector<int64_t> pathStart, pathLen;   // per path: offset into dPaths and length
+  int64_t pathsPacked = 0;             // entries of dPaths the current call has placed (paths_place)
+  int64_t pathsCapacity = 0;
+  size_t pathsBytes = 0;               // size of the pooled block behind dPaths
+  int64_t pathIdLimit = 0;             // transition ids of the stored paths are below this (the machine's nTrans)
+};
+
 // scratch device memory owned by one scope: cudaMalloc on alloc, cudaFree when the scope ends
 struct DevBuf {
   void* p = nullptr;
@@ -149,13 +160,9 @@ struct mb_batch {
   // grow-only device workspace, reused across calls on this batch so that steady-state calls do
   // no cudaMalloc / cudaFree (slots: see enum WsSlot)
   struct WsEntry { void* p = nullptr; size_t bytes = 0; } ws[24];
-  // result of the last mb_viterbi with traceback: packed paths on the device
-  int32_t* dPaths = nullptr;
-  std::vector<int64_t> pathStart, pathLen;   // per pair: offset into dPaths and length
-  int64_t pathsPacked = 0;             // entries of dPaths the current mb_viterbi call has placed (paths_place)
-  int64_t pathsCapacity = 0;
-  size_t pathsBytes = 0;               // size of the pooled block behind dPaths
-  int64_t pathIdLimit = 0;             // transition ids of the stored paths are below this (the machine's nTrans)
+  mb::PathStore viterbiPaths;          // result of the last mb_viterbi with traceback, a path per pair
+  mb::PathStore sampledPaths;          // result of the last mb_sample_paths, path k * nSamples + j
+  int32_t samplesPerPair = 0;          // nSamples of that call (0: no samples stored)
 };
 
 namespace mb {
@@ -166,6 +173,8 @@ int generic_forward (mb_machine* m, mb_batch* b, double* loglike, bool backward)
 int generic_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen);
 int generic_counts (mb_machine* m, mb_batch* b, double* counts, double* loglike);
 int generic_matrix (mb_machine* m, mb_batch* b, int64_t pair, int kind, double* cells);
+// nSamples paths per pair drawn from the stored Forward matrices into b->sampledPaths (pathLen / pathStart set by the caller's size)
+int generic_sample_paths (mb_machine* m, mb_batch* b, int32_t nSamples, uint64_t seed, double* loglike);
 
 // ---- jit engine (mb_jit.cu) ----
 bool jit_supported (const mb_machine* m, std::string* why);
@@ -243,10 +252,11 @@ void ws_release_all (mb_batch* b);
 size_t ws_bytes (const mb_batch* b, int slot);
 size_t ws_pool_bytes (int device);
 bool ws_pool_fits (int device, size_t bytes);   // a pooled block would serve this request   // freed blocks kept for reuse; released when an allocation fails
-int paths_reserve (mb_batch* b, int64_t need);   // room for `need` packed path entries in b->dPaths (pooled; keeps the content)
-// Viterbi paths of pairs[0..n), after those the call has placed so far: copies their lengths (dLen, device) to the host,
-// sets pathStart / pathLen, grows dPaths to hold them and writes each pair's start into dOutOff (device) for the id pass
-int paths_place (mb_batch* b, const int64_t* pairs, int64_t n, const int64_t* dLen, int64_t* dOutOff);
+int paths_reserve (mb_batch* b, PathStore& ps, int64_t need);   // room for `need` packed path entries in ps.dPaths (pooled; keeps the content)
+// paths rows[0..n) of the store (a pair's index for Viterbi paths), after those the call has placed so far: copies their lengths
+// (dLen, device) to the host, sets pathStart / pathLen, grows dPaths to hold them and writes each path's start into dOutOff
+// (device) for the id pass
+int paths_place (mb_batch* b, PathStore& ps, const int64_t* rows, int64_t n, const int64_t* dLen, int64_t* dOutOff);
 
 // timing helpers
 int timing_begin (mb_batch* b);

@@ -1552,8 +1552,8 @@ int jit_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen) {
       const unsigned tg = (unsigned) ((n + 63) / 64);
       jit_traceback_kernel<<<tg, 64, 0, b->stream>>> (tp, (int) nSlots, b->dev, dPairs, (int64_t) n, dTb, dTbOff, dRes, dLen, dTmp, dTmpOff);
       MB_CUDA (cudaGetLastError());
-      if (paths_place (b, chunks[c].data(), (int64_t) n, dLen, dOutOff)) return 1;
-      jit_path_ids_kernel<<<(unsigned) ((n * 32 + 255) / 256), 256, 0, b->stream>>> (tp, (int) nSlots, b->dev, dPairs, (int64_t) n, dLen, dTmp, dTmpOff, b->dPaths, dOutOff);
+      if (paths_place (b, b->viterbiPaths, chunks[c].data(), (int64_t) n, dLen, dOutOff)) return 1;
+      jit_path_ids_kernel<<<(unsigned) ((n * 32 + 255) / 256), 256, 0, b->stream>>> (tp, (int) nSlots, b->dev, dPairs, (int64_t) n, dLen, dTmp, dTmpOff, b->viterbiPaths.dPaths, dOutOff);
       MB_CUDA (cudaGetLastError());
       launches += 2;
     }

@@ -1294,9 +1294,9 @@ int lane_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen) {
     const int64_t nWork = (int64_t) chunk.size();
     if (wide_traceback_launch (m, b, dOrder.as<int64_t>(), nWork, dBp.as<unsigned char>(), dBpOffRead.as<int64_t>(), h->bpBytes, LPT,
                                dRes.as<double>(), dLen.as<int64_t>(), nullptr, nullptr)) return 1;
-    if (paths_place (b, chunk.data(), nWork, dLen.as<int64_t>(), dOutOff.as<int64_t>())) return 1;
+    if (paths_place (b, b->viterbiPaths, chunk.data(), nWork, dLen.as<int64_t>(), dOutOff.as<int64_t>())) return 1;
     if (wide_traceback_launch (m, b, dOrder.as<int64_t>(), nWork, dBp.as<unsigned char>(), dBpOffRead.as<int64_t>(), h->bpBytes, LPT,
-                               dRes.as<double>(), dLen.as<int64_t>(), b->dPaths, dOutOff.as<int64_t>())) return 1;
+                               dRes.as<double>(), dLen.as<int64_t>(), b->viterbiPaths.dPaths, dOutOff.as<int64_t>())) return 1;
     launches += 3;
     if (timing_end (b, launches)) return 1;
     ms += b->lastMs;

@@ -875,9 +875,9 @@ int wide_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen) {
     wide_traceback_kernel<<<tg, 32, 0, b->stream>>> (m->dev, b->dev, dOrder.as<int64_t>(), nWork, dBp.as<unsigned char>(), dBpOff.as<int64_t>(), h->t.bpBytes, 0,
                                                       dRes.as<double>(), dLen.as<int64_t>(), nullptr, nullptr);
     MB_CUDA (cudaGetLastError());
-    if (paths_place (b, chunk.data(), nWork, dLen.as<int64_t>(), dOutOff.as<int64_t>())) return 1;
+    if (paths_place (b, b->viterbiPaths, chunk.data(), nWork, dLen.as<int64_t>(), dOutOff.as<int64_t>())) return 1;
     wide_traceback_kernel<<<tg, 32, 0, b->stream>>> (m->dev, b->dev, dOrder.as<int64_t>(), nWork, dBp.as<unsigned char>(), dBpOff.as<int64_t>(), h->t.bpBytes, 0,
-                                                      dRes.as<double>(), dLen.as<int64_t>(), b->dPaths, dOutOff.as<int64_t>());
+                                                      dRes.as<double>(), dLen.as<int64_t>(), b->viterbiPaths.dPaths, dOutOff.as<int64_t>());
     MB_CUDA (cudaGetLastError());
     launches += 3;
     if (timing_end (b, launches)) return 1;

@@ -924,6 +924,36 @@ inline vector<double> viterbiLogLikes (const EvaluatedMachine& m, const SeqPairL
   return sc;
 }
 
+// nSamples paths per pair drawn from the posterior on the device (mb_sample_paths): path j of pair k is keyed by (seed, k, j), so a
+// list gives the same paths on every run and device.  (*loglike)[k] receives pair k's Forward log-likelihood; a pair without
+// a finite path gets nSamples empty paths.  One device: the list is not dealt over the box's GPUs.  The reference's
+// mt19937 draws are ForwardMatrix::samplePath's.
+inline vector<vector<MachinePath> > posteriorPaths (const EvaluatedMachine& m, const SeqPairList& l, int nSamples, uint64_t seed, vector<double>* loglike = nullptr) {
+  const size_t n = l.seqPairs.size();
+  DeviceBatch b (m, pairPointers (l));
+  vector<double> ll (n ? n : 1);
+  const size_t nPaths = nSamples > 0 ? n * (size_t) nSamples : 0;
+  vector<int64_t> len (nPaths ? nPaths : 1), off (nPaths + 1, 0);
+  mbCheck (mb_sample_paths (m.handle(), b.handle(), nSamples, seed, ll.data(), len.data()));
+  for (size_t r = 0; r < nPaths; ++r) off[r + 1] = off[r] + len[r];
+  if (loglike) loglike->assign (ll.begin(), ll.begin() + n);
+  vector<vector<MachinePath> > paths (n, vector<MachinePath> ((size_t) nSamples));
+  auto unpack = [&] (const auto& ids) {
+    for (size_t r = 0; r < nPaths; ++r)
+      for (int64_t q = off[r]; q < off[r + 1]; ++q) paths[r / nSamples][r % nSamples].trans.push_back (m.transition ((int32_t) ids[q]));
+  };
+  if (m.nTransitions <= 256) {      // byte ids: a quarter of the device-to-host copy
+    vector<uint8_t> ids ((size_t) off[nPaths] ? (size_t) off[nPaths] : 1);
+    if (off[nPaths]) mbCheck (mb_sampled_paths (b.handle(), ids.data(), 1, off.data()));
+    unpack (ids);
+  } else {
+    vector<int32_t> ids ((size_t) off[nPaths] ? (size_t) off[nPaths] : 1);
+    if (off[nPaths]) mbCheck (mb_sampled_paths (b.handle(), ids.data(), 4, off.data()));
+    unpack (ids);
+  }
+  return paths;
+}
+
 // api.h:25-31 equivalents taking an already-evaluated machine
 inline double forwardLogLike (const EvaluatedMachine& m, const SeqPair& sp) { return ForwardMatrix (m, sp).logLike(); }
 inline double viterbiLogLike (const EvaluatedMachine& m, const SeqPair& sp) { return ViterbiMatrix (m, sp).logLike(); }

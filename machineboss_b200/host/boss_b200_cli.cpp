@@ -17,6 +17,8 @@
 //   -A, --align     Viterbi alignments as a SeqPairList with meta.path       (boss.cpp:833,843-846)
 //   -C, --counts    raw expected transition counts, MachineCounts::writeJson (counts.cpp:73-78)
 //   --sample-paths SEED   one path per pair drawn from the posterior, ForwardMatrix::samplePath (forward.cpp:17-23)
+//   --posterior-paths N [--posterior-seed S]   N paths per pair drawn from the posterior for the whole list at once on the
+//                   device (posteriorPaths, default seed 1): [[[transition ids], ...N], ...], [] for a pair without a path
 //                   (boss -C prints PARAMETER counts, which needs the symbolic weight derivatives
 //                   of the Machine -- outside this path; see INTEGRATION.md)
 //   data: -D/--data pairs.json (a SeqPairList) | --input-fasta X --output-fasta Y |
@@ -88,6 +90,8 @@ int main (int argc, char** argv) {
     bool doL = false, doV = false, doA = false, doC = false, doSample = false, useApi = false;
     string envMode;
     long long sampleSeed = 1;
+    int posteriorN = 0;
+    unsigned long long posteriorSeed = 1;
     int postTransTop = 0;
     bool doDownsample = false;
     double downsampleSize = 1., downsampleProb = 0.;
@@ -118,6 +122,8 @@ int main (int argc, char** argv) {
       else if (f == "-C" || f == "--counts") doC = true;
       else if (f == "--envelope") envMode = next();      // full | path | <width>: print each pair's Envelope (t/src/testenv.cpp; no device needed)
       else if (f == "--sample-paths") { doSample = true; sampleSeed = atoll (next().c_str()); }
+      else if (f == "--posterior-paths") { posteriorN = atoi (next().c_str()); if (posteriorN < 1) throw runtime_error ("--posterior-paths needs a count of at least 1"); }
+      else if (f == "--posterior-seed") posteriorSeed = strtoull (next().c_str(), nullptr, 10);
       else if (f == "--downsample-size") { doDownsample = true; downsampleSize = atof (next().c_str()); }      // boss.cpp:487-490: which transitions Machine::downsample keeps
       else if (f == "--downsample-prob") { doDownsample = true; downsampleProb = atof (next().c_str()); }
       else if (f == "--downsample-path") { doDownsample = true; downsamplePaths = atoi (next().c_str()); }      // boss.cpp:491-493: sample this many paths (seed: --seed)
@@ -249,7 +255,7 @@ int main (int argc, char** argv) {
     for (const auto& i: inSeqs) for (const auto& o: outSeqs) { SeqPair sp; sp.input = i; sp.output = o; data.seqPairs.push_back (sp); }
     if (data.seqPairs.empty() && inputEmpty && outputEmpty) data.seqPairs.push_back (SeqPair());   // boss.cpp:769-770
     if (data.seqPairs.empty()) throw runtime_error ("no sequence data given");
-    if (!(doL || doV || doA || doC || doT || doSample || postTransTop)) throw runtime_error ("nothing to do: give -L, -V, -A, -C or -T");
+    if (!(doL || doV || doA || doC || doT || doSample || posteriorN || postTransTop)) throw runtime_error ("nothing to do: give -L, -V, -A, -C or -T");
 
     if (doT) {   // boss.cpp:776-787
       if (constraints.empty() && machine.cons.empty()) throw runtime_error ("To fit parameters, please specify a constraints file and (for machines with input/output) a data file");
@@ -365,6 +371,27 @@ int main (int argc, char** argv) {
         }
         cout << "]";
         ++k;
+      }
+      cout << "]\n";
+    }
+    if (posteriorN) {   // the whole list in one device call; pairs that cannot be tokenised print []
+      vector<double> ll;
+      const vector<vector<MachinePath> > paths = posteriorPaths (eval, ok, posteriorN, (uint64_t) posteriorSeed, &ll);
+      vector<int> okAt (data.seqPairs.size(), -1);
+      for (size_t q = 0; q < okIndex.size(); ++q) okAt[okIndex[q]] = (int) q;
+      cout << "[";
+      for (size_t k = 0; k < data.seqPairs.size(); ++k) {
+        cout << (k ? ",\n " : "") << "[";
+        if (okAt[k] >= 0 && ll[okAt[k]] > ninf) {
+          size_t j = 0;
+          for (const auto& p: paths[okAt[k]]) {
+            cout << (j++ ? "," : "") << "[";
+            size_t n = 0;
+            for (const auto& t: p.trans) cout << (n++ ? "," : "") << t.id;
+            cout << "]";
+          }
+        }
+        cout << "]";
       }
       cout << "]\n";
     }
