@@ -130,6 +130,15 @@ int mb_batch_wait (mb_batch* b);
  * log-likelihood is -inf contribute nothing. */
 int mb_counts (mb_machine* m, mb_batch* b, double* counts, double* loglike);
 
+/* ---- MachineCounts of each pair on its own (src/counts.cpp:37-64 over a list of one) ----
+ * Posterior counts of each pair: row k of counts ([nPairs][nTrans], row-major) is what mb_counts gives for a
+ * batch holding only pair k; loglike[k] (may be NULL) as mb_counts.  An impossible pair gets a zero row and -inf.
+ * Per pair: expected substitutions and gaps, use of a profile's states by each read, weighted EM, and the
+ * gradient of pair k's log-likelihood with respect to the log-weights (row k).  counts must not be NULL
+ * (mb_counts gives the log-likelihoods alone).  Same engines as mb_counts; the device holds the rows of one
+ * chunk of pairs at a time. */
+int mb_pair_counts (mb_machine* m, mb_batch* b, double* counts, double* loglike);
+
 /* ---- DPMatrix::cell of a ForwardMatrix / BackwardMatrix / ViterbiMatrix (src/dpmatrix.h:128-146) ----
  * The whole log-domain matrix of ONE pair of the batch, as the reference stores it (dpmatrix.h:86-95):
  * cells[((o * (inLen + 1)) + i) * nStates + s], state fastest; -inf outside the pair's envelope.  It is what
@@ -159,7 +168,7 @@ int mb_sampled_paths (mb_batch* b, void* pathTrans, int32_t bytesPerId, const in
  * Replaces the reference's single-core loops over a SeqPairList: MachineCounts (counts.cpp:37-43) inside
  * MachineFitter::fit (fitter.cpp:23-47), and the -L / -A loops of the CLI (boss.cpp:796,826).  The pairs are
  * dealt to the devices longest-processing-time first by cell count (Li+1)(Lo+1); the machine is replicated; one
- * host thread per device drives that device's share.  Forward / Viterbi: no communication, results gathered by
+ * host thread per device drives that device's share.  Forward / Viterbi / per-pair counts: no communication, results gathered by
  * pair index.  Counts: ncclAllReduce (sum, ncclDouble) of nTrans + 1 values over NVLink (libnccl.so.2, resolved
  * at run time; one device, or no NCCL: added on the host -- mb_group_info says which).  Results are those of
  * the single-device calls: identical for Forward and Viterbi, equal up to the order of summation for counts. */
@@ -188,6 +197,9 @@ int mb_group_viterbi (mb_gmachine* m, mb_gbatch* b, double* score, int64_t* path
 int mb_group_viterbi_paths (mb_gbatch* b, int32_t* pathTrans, const int64_t* pathOff);
 int mb_group_viterbi_paths_narrow (mb_gbatch* b, void* pathTrans, int32_t bytesPerId, const int64_t* pathOff);
 int mb_group_counts (mb_gmachine* m, mb_gbatch* b, double* counts, double* loglike);
+/* mb_pair_counts over the group: each device computes the rows of its pairs, the host places them in list order
+ * (no all-reduce; mb_group_last_loglike is left as it was) */
+int mb_group_pair_counts (mb_gmachine* m, mb_gbatch* b, double* counts, double* loglike);
 int mb_group_last_loglike (const mb_gmachine* m, double* total);      /* summed over all pairs by the last mb_group_counts' all-reduce */
 int mb_group_last_kernel_ms (const mb_gbatch* b, double* maxMs, int64_t* nLaunches);      /* slowest device, launches of all */
 
@@ -235,7 +247,7 @@ int mb_col_emulate (int32_t nStates, int32_t nInTok, int32_t nOutTok, int64_t nT
  * Device time, in milliseconds, of the kernels launched by the last compute call on this batch
  * (CUDA events on the launching stream), and how many kernels that was. */
 int mb_last_kernel_ms (const mb_batch* b, double* ms, int64_t* nLaunches);
-/* How many pairs of the last mb_forward / mb_backward / mb_counts on this batch the scaled
+/* How many pairs of the last mb_forward / mb_backward / mb_counts / mb_pair_counts on this batch the scaled
  * linear-domain sweep handed over to the log-domain kernel (dangerous dynamic range, or -inf). */
 int mb_last_redo (const mb_batch* b, int64_t* nPairs);
 

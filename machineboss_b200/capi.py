@@ -21,11 +21,11 @@ _lib = None
 SYMBOLS = ["mb_last_error", "mb_version", "mb_set_kernel_cache_dir", "mb_device_count", "mb_set_device", "mb_set_engine", "mb_set_option", "mb_machine_set_option",
            "mb_machine_create", "mb_machine_update_weights", "mb_machine_info", "mb_machine_destroy",
            "mb_batch_create", "mb_batch_destroy", "mb_batch_trim", "mb_batch_set_envelopes", "mb_forward", "mb_backward", "mb_viterbi",
-           "mb_viterbi_paths", "mb_viterbi_paths_narrow", "mb_viterbi_paths_start", "mb_batch_wait", "mb_counts", "mb_matrix", "mb_sample_paths", "mb_sampled_paths", "mb_last_kernel_ms", "mb_last_redo", "mb_jit_compile_check", "mb_jit_host_tables", "mb_lane_emulate", "mb_col_emulate",
+           "mb_viterbi_paths", "mb_viterbi_paths_narrow", "mb_viterbi_paths_start", "mb_batch_wait", "mb_counts", "mb_pair_counts", "mb_matrix", "mb_sample_paths", "mb_sampled_paths", "mb_last_kernel_ms", "mb_last_redo", "mb_jit_compile_check", "mb_jit_host_tables", "mb_lane_emulate", "mb_col_emulate",
            "mb_shard_pairs", "mb_group_create", "mb_group_info", "mb_group_destroy", "mb_group_machine_create", "mb_group_machine_update_weights",
            "mb_group_machine_set_option", "mb_group_machine_info", "mb_group_machine_destroy", "mb_group_batch_create", "mb_group_batch_set_envelopes",
            "mb_group_batch_shard", "mb_group_batch_destroy", "mb_group_forward", "mb_group_backward", "mb_group_viterbi", "mb_group_viterbi_paths",
-           "mb_group_viterbi_paths_narrow", "mb_group_counts", "mb_group_last_loglike", "mb_group_last_kernel_ms"]
+           "mb_group_viterbi_paths_narrow", "mb_group_counts", "mb_group_pair_counts", "mb_group_last_loglike", "mb_group_last_kernel_ms"]
 
 
 class MachineBossError(RuntimeError):
@@ -65,6 +65,7 @@ def lib():
         L.mb_viterbi_paths_start.argtypes = [P, P, I32, P]
         L.mb_batch_wait.argtypes = [P]
         L.mb_counts.argtypes = [P, P, P, P]
+        L.mb_pair_counts.argtypes = [P, P, P, P]
         L.mb_matrix.argtypes = [P, P, I64, I32, P]
         L.mb_sample_paths.argtypes = [P, P, I32, ctypes.c_uint64, P, P]
         L.mb_sampled_paths.argtypes = [P, P, I32, P]
@@ -96,6 +97,7 @@ def lib():
         L.mb_group_viterbi_paths.argtypes = [P, P, P]
         L.mb_group_viterbi_paths_narrow.argtypes = [P, P, I32, P]
         L.mb_group_counts.argtypes = [P, P, P, P]
+        L.mb_group_pair_counts.argtypes = [P, P, P, P]
         L.mb_group_last_loglike.argtypes = [P, ctypes.POINTER(D)]
         L.mb_group_last_kernel_ms.argtypes = [P, ctypes.POINTER(D), ctypes.POINTER(I64)]
         _lib = L
@@ -413,6 +415,16 @@ def counts(m: Machine, b: Batch):
     return c, ll
 
 
+def pair_counts(m: Machine, b: Batch, loglike: bool = False):
+    """Posterior counts of each pair on its own (mb_pair_counts): array [nPairs, nTrans], row k what counts() gives for a
+    batch of pair k alone.  With loglike=True also returns the Forward log-likelihoods."""
+    c = np.zeros(max(b.n_pairs * m.n_trans, 1), dtype=np.float64)
+    ll = np.empty(max(b.n_pairs, 1), dtype=np.float64)
+    _check(lib().mb_pair_counts(m.h, b.h, c.ctypes.data, ll.ctypes.data))
+    rows = c[: b.n_pairs * m.n_trans].reshape(b.n_pairs, m.n_trans)
+    return (rows, ll[: b.n_pairs]) if loglike else rows
+
+
 # ---------------------------------------------------------------------------------------------
 # several GPUs of one box (mb_group_*): the list dealt to the devices, one host thread per device
 # ---------------------------------------------------------------------------------------------
@@ -545,3 +557,12 @@ def group_counts(m: GroupMachine, b: GroupBatch):
     ll = np.empty(max(b.n_pairs, 1), dtype=np.float64)
     _check(lib().mb_group_counts(m.h, b.h, c.ctypes.data, ll.ctypes.data))
     return c[: m.n_trans], ll[: b.n_pairs]
+
+
+def group_pair_counts(m: GroupMachine, b: GroupBatch, loglike: bool = False):
+    """pair_counts over a group: [nPairs, nTrans] in list order (mb_group_pair_counts)."""
+    c = np.zeros(max(b.n_pairs * m.n_trans, 1), dtype=np.float64)
+    ll = np.empty(max(b.n_pairs, 1), dtype=np.float64)
+    _check(lib().mb_group_pair_counts(m.h, b.h, c.ctypes.data, ll.ctypes.data))
+    rows = c[: b.n_pairs * m.n_trans].reshape(b.n_pairs, m.n_trans)
+    return (rows, ll[: b.n_pairs]) if loglike else rows

@@ -588,7 +588,7 @@ static int check_call (const mb_machine* m, const mb_batch* b) {
   return 0;
 }
 
-enum Pass { PASS_FORWARD, PASS_VITERBI_PATHS, PASS_VITERBI_SCORES, PASS_BACKWARD, PASS_COUNTS, PASS_MATRIX, PASS_SAMPLE };
+enum Pass { PASS_FORWARD, PASS_VITERBI_PATHS, PASS_VITERBI_SCORES, PASS_BACKWARD, PASS_COUNTS, PASS_MATRIX, PASS_SAMPLE, PASS_PAIR_COUNTS };
 enum Route { ROUTE_ERROR = -1, ROUTE_NONE, ROUTE_JIT, ROUTE_BIG, ROUTE_COL, ROUTE_LANE, ROUTE_WIDE, ROUTE_GENERIC };
 
 // The engine that serves a call, after any lazy preparation it needs (ROUTE_NONE: nothing to do; ROUTE_ERROR: a preparation
@@ -635,7 +635,7 @@ static int route_of (mb_machine* m, mb_batch* b, Pass pass) {
 static int route (mb_machine* m, mb_batch* b, Pass pass) {
   const int r = route_of (m, b, pass);
   if (r != ROUTE_ERROR && m->opt.get ("verbose", 0)) {
-    static const char* const passNames[] = { "mb_forward", "mb_viterbi", "mb_viterbi (scores)", "mb_backward", "mb_counts", "mb_matrix", "mb_sample_paths" };
+    static const char* const passNames[] = { "mb_forward", "mb_viterbi", "mb_viterbi (scores)", "mb_backward", "mb_counts", "mb_matrix", "mb_sample_paths", "mb_pair_counts" };
     static const char* const engineNames[] = { "no engine (empty batch)", "jit engine", "big engine", "column engine", "lane engine", "wide engine", "generic engine" };
     fprintf (stderr, "%s: %s\n", passNames[pass], engineNames[r]);
   }
@@ -797,6 +797,12 @@ int mb_batch_wait (mb_batch* b) {
 int mb_counts (mb_machine* m, mb_batch* b, double* counts, double* loglike) {
   if (check_call (m, b)) return 1;
   return route (m, b, PASS_COUNTS) == ROUTE_JIT ? jit_counts (m, b, counts, loglike) : generic_counts (m, b, counts, loglike);
+}
+
+int mb_pair_counts (mb_machine* m, mb_batch* b, double* counts, double* loglike) {
+  if (check_call (m, b)) return 1;
+  if (!counts) { set_error ("mb_pair_counts: null counts (mb_counts gives the log-likelihoods alone)"); return 1; }
+  return route (m, b, PASS_PAIR_COUNTS) == ROUTE_JIT ? jit_counts (m, b, nullptr, loglike, counts) : generic_counts (m, b, nullptr, loglike, counts);
 }
 
 int mb_matrix (mb_machine* m, mb_batch* b, int64_t pair, int32_t kind, double* cells) {

@@ -262,10 +262,12 @@ __global__ void sample_kernel (DevMachine m, DevBatch b, const int64_t* __restri
 // BackwardMatrix::getCounts (backward.cpp:62-87): count[t] += exp(F(src cell) - ll + w_t + B(dest cell)).
 // One CTA per pair; the CTA walks the transitions, each thread sums the cells where the
 // transition's labels match the tokens, then a block reduction and one atomic per transition.
+// ROWS: the CTA of the chunk's pair blockIdx.x adds into that pair's own row, counts + blockIdx.x * rowStride.
+template<bool ROWS>
 __global__ void __launch_bounds__(256) counts_kernel (DevMachine m, DevBatch b, const int64_t* __restrict__ pairs,
                                                       const int64_t* __restrict__ wsOff, const double* __restrict__ wsF,
                                                       const double* __restrict__ wsB, const double* __restrict__ backLL,
-                                                      double* __restrict__ counts) {
+                                                      double* __restrict__ counts, int64_t rowStride) {
   __shared__ double red[256];
   const int64_t k = pairs[blockIdx.x];
   const double ll = backLL[k];   // backward.cpp:66 uses the Backward log-likelihood
@@ -277,6 +279,7 @@ __global__ void __launch_bounds__(256) counts_kernel (DevMachine m, DevBatch b, 
   const Cells F = { const_cast<double*> (wsF) + wsOff[blockIdx.x], Li, S, 0 }, B = { const_cast<double*> (wsB) + wsOff[blockIdx.x], Li, S, 0 };
   const int64_t nKeys = (int64_t) S * m.nIn1 * m.nOut1;
   const Env env = pair_env (b, k);
+  if (ROWS) counts += (int64_t) blockIdx.x * rowStride;
   for (int64_t key = 0; key < nKeys; ++key) {
     const int64_t p0 = m.out.off[key], p1 = m.out.off[key + 1];
     if (p0 == p1) continue;
@@ -313,16 +316,18 @@ struct Chunk {
   int64_t doubles = 0;
 };
 
-static int plan_chunks (const mb_batch* b, int S, bool rolling, int copies, std::vector<Chunk>& chunks) {
+// rowDoubles: a further buffer of that many doubles per pair of a chunk (per-pair counts), which shares the budget
+static int plan_chunks (const mb_batch* b, int S, bool rolling, int copies, std::vector<Chunk>& chunks, int64_t rowDoubles = 0) {
   size_t freeB = 0, totalB = 0;
   MB_CUDA (cudaMemGetInfo (&freeB, &totalB));
   const double budget = 0.80 * (double) freeB / 8.0 / copies;   // doubles per copy
+  const double rowShare = (double) rowDoubles / copies;
   Chunk cur;
   for (int64_t k = 0; k < b->nPairs; ++k) {
     const int64_t Li = b->xOff[k + 1] - b->xOff[k], Lo = b->yOff[k + 1] - b->yOff[k];
     const double need = rolling ? 3.0 * (double) (Li + 1) * S : (double) (Li + 1) * (double) (Lo + 1) * S;
-    if (need > budget) { set_error ("pair " + std::to_string (k) + " needs more device memory than is free (" + std::to_string (need * 8 * copies) + " bytes)"); return 1; }
-    if (!cur.pairs.empty() && ((double) cur.doubles + need > budget || cur.pairs.size() >= 65535 * 16)) { chunks.push_back (cur); cur = Chunk(); }
+    if (need + rowShare > budget) { set_error ("pair " + std::to_string (k) + " needs more device memory than is free (" + std::to_string ((need + rowShare) * 8 * copies) + " bytes)"); return 1; }
+    if (!cur.pairs.empty() && ((double) cur.doubles + need + rowShare * (double) (cur.pairs.size() + 1) > budget || cur.pairs.size() >= 65535 * 16)) { chunks.push_back (cur); cur = Chunk(); }
     cur.pairs.push_back (k);
     cur.wsOff.push_back (cur.doubles);
     cur.doubles += (int64_t) need;
@@ -458,13 +463,16 @@ int generic_sample_paths (mb_machine* m, mb_batch* b, int32_t nSamples, uint64_t
   return 0;
 }
 
-int generic_counts (mb_machine* m, mb_batch* b, double* counts, double* loglike) {
+int generic_counts (mb_machine* m, mb_batch* b, double* counts, double* loglike, double* rows) {
   if (b->nPairs == 0) { if (counts) for (int64_t t = 0; t < m->T; ++t) counts[t] = 0; return 0; }
   std::vector<Chunk> chunks;
-  if (plan_chunks (b, m->S, false, 2, chunks)) return 1;
+  if (plan_chunks (b, m->S, false, 2, chunks, rows ? m->T : 0)) return 1;
+  size_t maxPairs = 0;
+  for (auto& ch: chunks) maxPairs = std::max (maxPairs, ch.pairs.size());
+  const size_t T = (size_t) std::max<int64_t> (m->T, 1), countDoubles = rows ? maxPairs * T : T;      // rows: [chunk pairs][nTrans]
   DevBuf dF, dB, dCounts;
-  if (dF.alloc ((size_t) b->nPairs * 8) || dB.alloc ((size_t) b->nPairs * 8) || dCounts.alloc ((size_t) std::max<int64_t> (m->T, 1) * 8)) return 1;
-  MB_CUDA (cudaMemsetAsync (dCounts.p, 0, (size_t) std::max<int64_t> (m->T, 1) * 8, b->stream));
+  if (dF.alloc ((size_t) b->nPairs * 8) || dB.alloc ((size_t) b->nPairs * 8) || dCounts.alloc (countDoubles * 8)) return 1;
+  MB_CUDA (cudaMemsetAsync (dCounts.p, 0, T * 8, b->stream));
   int64_t launches = 0;
   double ms = 0;
   for (auto& ch: chunks) {
@@ -472,19 +480,24 @@ int generic_counts (mb_machine* m, mb_batch* b, double* counts, double* loglike)
     if (upload (dPairs, ch.pairs, b->stream) || upload (dOff, ch.wsOff, b->stream) || dWsF.alloc ((size_t) ch.doubles * 8) || dWsB.alloc ((size_t) ch.doubles * 8)) return 1;
     const unsigned grid = (unsigned) ch.pairs.size();
     if (timing_begin (b)) return 1;
+    if (rows) MB_CUDA (cudaMemsetAsync (dCounts.p, 0, ch.pairs.size() * T * 8, b->stream));
     fill_kernel<OP_SUM, false><<<grid, 256, 0, b->stream>>> (m->dev, b->dev, dPairs.as<int64_t>(), dOff.as<int64_t>(), dWsF.as<double>(), 0, dF.as<double>());
     fill_kernel<OP_SUM, true><<<grid, 256, 0, b->stream>>> (m->dev, b->dev, dPairs.as<int64_t>(), dOff.as<int64_t>(), dWsB.as<double>(), 0, dB.as<double>());
-    if (counts)
-      counts_kernel<<<grid, 256, 0, b->stream>>> (m->dev, b->dev, dPairs.as<int64_t>(), dOff.as<int64_t>(), dWsF.as<double>(), dWsB.as<double>(), dB.as<double>(), dCounts.as<double>());
+    if (rows)
+      counts_kernel<true><<<grid, 256, 0, b->stream>>> (m->dev, b->dev, dPairs.as<int64_t>(), dOff.as<int64_t>(), dWsF.as<double>(), dWsB.as<double>(), dB.as<double>(), dCounts.as<double>(), (int64_t) T);
+    else if (counts)
+      counts_kernel<false><<<grid, 256, 0, b->stream>>> (m->dev, b->dev, dPairs.as<int64_t>(), dOff.as<int64_t>(), dWsF.as<double>(), dWsB.as<double>(), dB.as<double>(), dCounts.as<double>(), 0);
     MB_CUDA (cudaGetLastError());
-    launches += counts ? 3 : 2;
+    launches += counts || rows ? 3 : 2;
     if (timing_end (b, launches)) return 1;
     ms += b->lastMs;
+    // a chunk's pairs are consecutive in the batch, so its rows are one block of the caller's array
+    if (rows && m->T) MB_CUDA (cudaMemcpy (rows + ch.pairs[0] * m->T, dCounts.p, ch.pairs.size() * T * 8, cudaMemcpyDeviceToHost));
   }
   b->lastMs = ms;
   b->lastLaunches = launches;
   if (loglike) MB_CUDA (cudaMemcpy (loglike, dF.p, (size_t) b->nPairs * 8, cudaMemcpyDeviceToHost));
-  if (counts) MB_CUDA (cudaMemcpy (counts, dCounts.p, (size_t) m->T * 8, cudaMemcpyDeviceToHost));
+  if (counts && !rows) MB_CUDA (cudaMemcpy (counts, dCounts.p, (size_t) m->T * 8, cudaMemcpyDeviceToHost));
   return 0;
 }
 

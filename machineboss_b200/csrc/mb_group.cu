@@ -444,6 +444,22 @@ int mb_group_counts (mb_gmachine* gm, mb_gbatch* gb, double* counts, double* log
   return 0;
 }
 
+int mb_group_pair_counts (mb_gmachine* gm, mb_gbatch* gb, double* counts, double* loglike) {
+  if (check_group_call (gm, gb)) return 1;
+  if (!counts) { set_error ("mb_group_pair_counts: null counts (mb_group_counts gives the log-likelihoods alone)"); return 1; }
+  const size_t T = (size_t) gm->T;
+  return gb->g->run ([&] (int d) {      // each device's rows, scattered into list order; nothing crosses devices
+    const std::vector<int64_t>& mine = gb->pairsOf[d];
+    std::vector<double> rows (mine.size() * T + 1), ll (mine.size() + 1);
+    if (mb_pair_counts (gm->m[d], gb->b[d], rows.data(), ll.data())) return 1;
+    for (size_t q = 0; q < mine.size(); ++q) {
+      if (T) memcpy (counts + mine[q] * (int64_t) T, rows.data() + q * T, T * 8);
+      if (loglike) loglike[mine[q]] = ll[q];
+    }
+    return 0;
+  });
+}
+
 int mb_group_last_loglike (const mb_gmachine* gm, double* total) {
   if (!gm) { set_error ("null machine"); return 1; }
   if (total) *total = gm->lastLogLike;

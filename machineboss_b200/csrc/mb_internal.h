@@ -171,7 +171,8 @@ namespace mb {
 // Each returns 0 on success.  Results are written to host arrays.
 int generic_forward (mb_machine* m, mb_batch* b, double* loglike, bool backward);
 int generic_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen);
-int generic_counts (mb_machine* m, mb_batch* b, double* counts, double* loglike);
+// rows == nullptr: counts[nTrans] summed over the batch (may be null); otherwise pair k's counts to rows[k * nTrans ..)
+int generic_counts (mb_machine* m, mb_batch* b, double* counts, double* loglike, double* rows = nullptr);
 int generic_matrix (mb_machine* m, mb_batch* b, int64_t pair, int kind, double* cells);
 // nSamples paths per pair drawn from the stored Forward matrices into b->sampledPaths (pathLen / pathStart set by the caller's size)
 int generic_sample_paths (mb_machine* m, mb_batch* b, int32_t nSamples, uint64_t seed, double* loglike);
@@ -185,7 +186,7 @@ void jit_destroy (mb_machine* m);
 int jit_update_weights (mb_machine* m);
 int jit_forward (mb_machine* m, mb_batch* b, double* loglike, bool backward);
 int jit_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen);
-int jit_counts (mb_machine* m, mb_batch* b, double* counts, double* loglike);
+int jit_counts (mb_machine* m, mb_batch* b, double* counts, double* loglike, double* rows = nullptr);      // as generic_counts
 
 // ---- wide engine (mb_wide.cu): Forward log-likelihood and Viterbi for mid-size and large machines ----
 bool wide_supported (const mb_machine* m, std::string* why);
@@ -245,7 +246,7 @@ int rt_prepare (void* fn, int threads, size_t smemBytes, int* blocksPerSM);
 int rt_launch (void* fn, unsigned grid, unsigned threads, size_t smemBytes, cudaStream_t stream, void** params);
 
 // per-batch workspace (mb_api.cu)
-enum WsSlot { WS_ORDER = 0, WS_BND, WS_RESULT, WS_RESULT2, WS_TB, WS_TBOFF, WS_F, WS_FOFF, WS_COUNTS, WS_PAIRS, WS_LEN, WS_OUTOFF, WS_COUNTER, WS_FLAG, WS_EF, WS_EFOFF, WS_PATHTMP, WS_PATHTMPOFF, WS_PATHNARROW, WS_ITEMS, WS_ITEMBND, WS_PROG, WS_NSLOTS };
+enum WsSlot { WS_ORDER = 0, WS_BND, WS_RESULT, WS_RESULT2, WS_TB, WS_TBOFF, WS_F, WS_FOFF, WS_COUNTS, WS_PAIRS, WS_LEN, WS_OUTOFF, WS_COUNTER, WS_FLAG, WS_EF, WS_EFOFF, WS_PATHTMP, WS_PATHTMPOFF, WS_PATHNARROW, WS_ITEMS, WS_ITEMBND, WS_PROG, WS_ROWOF, WS_NSLOTS };
 void* ws_reserve (mb_batch* b, int slot, size_t bytes);   // nullptr + error set on failure
 void ws_release (mb_batch* b, int slot);
 void ws_release_all (mb_batch* b);

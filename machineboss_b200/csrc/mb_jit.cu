@@ -251,6 +251,12 @@ struct JitEngine {
   bool splitTried = false;
   CUfunction kSplit[4] = { nullptr, nullptr, nullptr, nullptr };      // viterbi, forward_lin, backward_lin, viterbi_score
   int blocksPerSMS[4] = { 1, 1, 1, 1 };
+  // the per-pair count module (MB_PAIR_ROWS): built the first time a call asks for per-pair counts
+  std::string sourceR;
+  CUmodule modR = nullptr;
+  bool rowsTried = false;
+  CUfunction kRows[2] = { nullptr, nullptr };      // bcounts_rows (log domain), bcounts_lin_rows
+  int blocksPerSMR[2] = { 1, 1 };
   // E-step: Forward states kept per cell (those with an emitting transition group coming in, plus the
   // start state); the others follow from them inside the cell through the silent groups
   std::vector<int> stored;
@@ -739,6 +745,27 @@ static int ensure_split_module (mb_machine* m, JitEngine& J) {
   return 0;
 }
 
+// The per-pair count module, on first use.
+static int ensure_rows_module (mb_machine* m, JitEngine& J) {
+  if (J.modR) return 0;
+  if (J.rowsTried) { set_error ("jit engine: the per-pair count module could not be built"); return 1; }
+  J.rowsTried = true;
+  std::vector<char> cubin;
+  if (nvrtc_compile (J.sourceR, ".rows.cu", cubin, nullptr)) return 1;
+  if (!cu_ok (g_drv.ModuleLoadData (&J.modR, cubin.data()), "cuModuleLoadData")) return 1;
+  const char* names[2] = { "mb_k_bcounts_rows", "mb_k_bcounts_lin_rows" };
+  const int qOf[2] = { 4, 8 };
+  for (int q = 0; q < 2; ++q) {
+    if (!cu_ok (g_drv.ModuleGetFunction (&J.kRows[q], J.modR, names[q]), "cuModuleGetFunction")) return 1;
+    if (!cu_ok (g_drv.FuncSetAttribute (J.kRows[q], CU_FUNC_ATTRIBUTE_MAX_DYNAMIC_SHARED_SIZE_BYTES, (int) J.smemBytes[qOf[q]]), "cuFuncSetAttribute")) return 1;
+    int nb = 0;
+    if (!cu_ok (g_drv.OccupancyMaxActiveBlocksPerMultiprocessor (&nb, J.kRows[q], J.threads, J.smemBytes[qOf[q]]), "occupancy")) return 1;
+    J.blocksPerSMR[q] = std::max (1, nb);
+  }
+  if (m->opt.get ("verbose", 0)) fprintf (stderr, "[mb_jit] per-pair count module compiled\n");
+  return 0;
+}
+
 static std::string module_source (const mb_machine* m, JitEngine& J, int passC, int pass, int passMinBlocks, int passMinBlocksLin);
 
 // A fitted score module (MB_C = C), on first use.  Returns its index in J.fit, or -1 when it cannot be built (the caller
@@ -991,6 +1018,7 @@ static void generate (const mb_machine* m, JitEngine& J) {
   J.source = module_source (m, J, J.C, 0, J.minBlocks, J.minBlocksLin);
   J.sourceV = J.CV != J.C ? module_source (m, J, J.CV, 1, J.minBlocksV, J.minBlocksLinV) : std::string();
   J.sourceS = "#define MB_SPLIT 1\n" + (J.sourceV.empty() ? J.source : J.sourceV);
+  J.sourceR = "#define MB_PAIR_ROWS 1\n#define MB_NTRANS " + std::to_string (m->T) + "\n" + J.source;
 }
 
 // One module's source: every kernel at passC columns per lane.  pass 0: the first module (E-step and log-domain kernels, and
@@ -1093,6 +1121,9 @@ int jit_compile_check (const mb_machine* m, std::string* log) {
     if (nvrtc_compile (J.sourceV, ".viterbi.cu", cubin, &logV)) return 1;
     if (log) *log += "\n---- Viterbi module (MB_C = " + std::to_string (J.CV) + ") ----\n" + logV;
   }
+  std::string logR;
+  if (nvrtc_compile (J.sourceR, ".rows.cu", cubin, &logR)) return 1;
+  if (log) *log += "\n---- per-pair count module ----\n" + logR;
   if (m->opt.get ("jit_split", -1) > 0) {
     std::string logS;
     if (nvrtc_compile (J.sourceS, ".split.cu", cubin, &logS)) return 1;
@@ -1138,6 +1169,7 @@ void jit_destroy (mb_machine* m) {
   if (J->mod && g_drv.ModuleUnload) g_drv.ModuleUnload (J->mod);
   if (J->modV && g_drv.ModuleUnload) g_drv.ModuleUnload (J->modV);
   if (J->modS && g_drv.ModuleUnload) g_drv.ModuleUnload (J->modS);
+  if (J->modR && g_drv.ModuleUnload) g_drv.ModuleUnload (J->modR);
   for (auto& f: J->fit) if (f.mod && g_drv.ModuleUnload) g_drv.ModuleUnload (f.mod);
   if (J->dEmitF) cudaFree (J->dEmitF);
   if (J->dEmitB) cudaFree (J->dEmitB);
@@ -1172,6 +1204,7 @@ struct MBArgsHost {   // must match struct MBArgs in the skeleton
   unsigned* F32; const int64_t* f32Off;
   int32_t* ef; const int64_t* efOff;
   const int64_t* items; const int64_t* itemBnd; int* prog;
+  const int64_t* rowOf;
 };
 
 static std::vector<int64_t> cost_order (const mb_batch* b, const std::vector<int64_t>& pairs) {
@@ -1195,7 +1228,8 @@ static const std::vector<int64_t>& full_order (mb_batch* b) {
 }
 
 struct CountArgs { double* F = nullptr; const int64_t* fOff = nullptr; const double* ll = nullptr; double* counts = nullptr; int32_t* flag = nullptr;
-                   unsigned* F32 = nullptr; const int64_t* f32Off = nullptr; int32_t* ef = nullptr; const int64_t* efOff = nullptr; };
+                   unsigned* F32 = nullptr; const int64_t* f32Off = nullptr; int32_t* ef = nullptr; const int64_t* efOff = nullptr;
+                   const int64_t* rowOf = nullptr; };      // rowOf: the count kernels (4, 8) add pair k's counts into row rowOf[k] of counts
 
 static int launch (mb_machine* m, mb_batch* b, int which, const std::vector<int64_t>& order, double* dResult, uint8_t* dTb, const int64_t* dTbOff,
                    const CountArgs& ca = CountArgs(), int useC = 0) {      // useC: columns per lane of a score kernel (0: the default module's)
@@ -1245,6 +1279,11 @@ static int launch (mb_machine* m, mb_batch* b, int which, const std::vector<int6
     fn = J.kSplit[q];
     grid = (int64_t) J.numSMs * J.blocksPerSMS[q];
   }
+  if (ca.rowOf && (which == 4 || which == 8)) {      // the per-pair variant of a count kernel
+    if (ensure_rows_module (m, J)) return 1;
+    fn = J.kRows[which == 4 ? 0 : 1];
+    grid = (int64_t) J.numSMs * J.blocksPerSMR[which == 4 ? 0 : 1];
+  }
   const int64_t nWorkItems = split ? (int64_t) items.size() : (int64_t) order.size();
   grid = std::min<int64_t> (grid, (nWorkItems + warpsPerBlock - 1) / warpsPerBlock);
   grid = std::max<int64_t> (grid, 1);
@@ -1263,6 +1302,7 @@ static int launch (mb_machine* m, mb_batch* b, int which, const std::vector<int6
   A.x = b->dX; A.xOff = b->dXOff; A.y = b->dY; A.yOff = b->dYOff;
   A.order = dOrder; A.nWork = nWorkItems; A.counter = dCounter;
   A.items = nullptr; A.itemBnd = nullptr; A.prog = nullptr;
+  A.rowOf = ca.rowOf;
   if (split) {
     int64_t* dItems = (int64_t*) ws_reserve (b, WS_ITEMS, items.size() * 8);
     int64_t* dItemBnd = (int64_t*) ws_reserve (b, WS_ITEMBND, itemBnd.size() * 8);
@@ -1569,105 +1609,129 @@ int jit_viterbi (mb_machine* m, mb_batch* b, double* score, int64_t* pathLen) {
 
 // MachineCounts over `pairs` (counts.cpp:37-64) with the log-domain kernels: per pair a Forward sweep
 // that stores its FP64 matrix, then the fused Backward + posterior-count sweep.  Counts are ADDED to
-// hostCounts, log-likelihoods written to loglike[k].  Chunked by free device memory.
+// hostCounts, or with rows (host, [nPairs][nTrans]) written to row k of rows for each pair k; log-likelihoods
+// written to loglike[k].  Chunked by free device memory; a chunk's per-pair rows ([chunk pairs][nTrans]) count
+// against the same budget as its Forward matrices.
 static int counts_log (mb_machine* m, mb_batch* b, const std::vector<int64_t>& pairs, bool wantCounts,
-                       std::vector<double>& hostCounts, double* loglike, int64_t& launches, double& ms) {
+                       std::vector<double>& hostCounts, double* loglike, int64_t& launches, double& ms, double* rows = nullptr) {
   if (pairs.empty()) return 0;
+  const int64_t rowDoubles = rows ? m->T : 0;
   double wanted = 0;
-  for (int64_t k: pairs) wanted += 8.0 * (double) (((((b->xOff[k + 1] - b->xOff[k]) + 1) * ((b->yOff[k + 1] - b->yOff[k]) + 1) * m->S) + 31) & ~(int64_t) 31);
+  for (int64_t k: pairs) wanted += 8.0 * (double) ((((((b->xOff[k + 1] - b->xOff[k]) + 1) * ((b->yOff[k + 1] - b->yOff[k]) + 1) * m->S) + 31) & ~(int64_t) 31) + rowDoubles);
   const double budget = memory_budget (m, b, WS_F, wanted, "jit_f_budget_mb") / 8.0;
   std::vector<std::vector<int64_t>> chunks (1);
-  std::vector<int64_t> fOffHost ((size_t) b->nPairs, 0), chunkDoubles (1, 0);
+  std::vector<int64_t> fOffHost ((size_t) b->nPairs, 0), rowOfHost ((size_t) b->nPairs, 0), chunkDoubles (1, 0);
   for (int64_t k: pairs) {
     const int64_t Li = b->xOff[k + 1] - b->xOff[k], Lo = b->yOff[k + 1] - b->yOff[k];
     const int64_t need = (((Li + 1) * (Lo + 1) * m->S) + 31) & ~(int64_t) 31;
-    if ((double) need > budget) { set_error ("pair " + std::to_string (k) + ": the Forward matrix does not fit in device memory"); return 1; }
-    if (!chunks.back().empty() && (double) (chunkDoubles.back() + need) > budget) { chunks.emplace_back(); chunkDoubles.push_back (0); }
+    if ((double) (need + rowDoubles) > budget) { set_error ("pair " + std::to_string (k) + ": the Forward matrix does not fit in device memory"); return 1; }
+    if (!chunks.back().empty() && (double) (chunkDoubles.back() + need + (int64_t) (chunks.back().size() + 1) * rowDoubles) > budget) { chunks.emplace_back(); chunkDoubles.push_back (0); }
     fOffHost[k] = chunkDoubles.back();
+    rowOfHost[k] = (int64_t) chunks.back().size();
     chunkDoubles.back() += need;
     chunks.back().push_back (k);
   }
   int64_t maxChunk = 0;
+  size_t maxPairs = 0;
   for (int64_t v: chunkDoubles) maxChunk = std::max (maxChunk, v);
+  for (auto& c: chunks) maxPairs = std::max (maxPairs, c.size());
   const size_t T = (size_t) std::max<int64_t> (m->T, 1);
+  const size_t countDoubles = rows ? maxPairs * T : T;
   double* dF = (double*) ws_reserve (b, WS_F, (size_t) maxChunk * 8);
   double* dLL = (double*) ws_reserve (b, WS_RESULT, (size_t) b->nPairs * 8);
   double* dBack = (double*) ws_reserve (b, WS_RESULT2, (size_t) b->nPairs * 8);
   int64_t* dFOff = (int64_t*) ws_reserve (b, WS_FOFF, (size_t) b->nPairs * 8);
-  double* dCounts = (double*) ws_reserve (b, WS_COUNTS, T * 8);
-  if (!dF || !dLL || !dBack || !dFOff || !dCounts) return 1;
+  double* dCounts = (double*) ws_reserve (b, WS_COUNTS, countDoubles * 8);
+  int64_t* dRowOf = rows ? (int64_t*) ws_reserve (b, WS_ROWOF, (size_t) b->nPairs * 8) : nullptr;
+  if (!dF || !dLL || !dBack || !dFOff || !dCounts || (rows && !dRowOf)) return 1;
   MB_CUDA (cudaMemcpyAsync (dFOff, fOffHost.data(), (size_t) b->nPairs * 8, cudaMemcpyHostToDevice, b->stream));
-  MB_CUDA (cudaMemsetAsync (dCounts, 0, T * 8, b->stream));
+  if (rows) MB_CUDA (cudaMemcpyAsync (dRowOf, rowOfHost.data(), (size_t) b->nPairs * 8, cudaMemcpyHostToDevice, b->stream));
+  else MB_CUDA (cudaMemsetAsync (dCounts, 0, T * 8, b->stream));
+  std::vector<double> rowsHere (rows ? countDoubles : 0);
   for (size_t c = 0; c < chunks.size(); ++c) {
     const std::vector<int64_t> order = cost_order (b, chunks[c]);
     CountArgs ca;
-    ca.F = dF; ca.fOff = dFOff; ca.ll = dLL; ca.counts = dCounts;
+    ca.F = dF; ca.fOff = dFOff; ca.ll = dLL; ca.counts = dCounts; ca.rowOf = dRowOf;
     if (timing_begin (b)) return 1;
+    if (rows) MB_CUDA (cudaMemsetAsync (dCounts, 0, chunks[c].size() * T * 8, b->stream));
     if (launch (m, b, 3, order, dLL, nullptr, nullptr, ca)) return 1;
     ++launches;
     if (wantCounts) { if (launch (m, b, 4, order, dBack, nullptr, nullptr, ca)) return 1; ++launches; }
     if (timing_end (b, launches)) return 1;
     ms += b->lastMs;
+    if (rows) {
+      MB_CUDA (cudaMemcpy (rowsHere.data(), dCounts, chunks[c].size() * T * 8, cudaMemcpyDeviceToHost));
+      for (int64_t k: chunks[c]) memcpy (rows + k * m->T, rowsHere.data() + rowOfHost[k] * (int64_t) T, (size_t) m->T * 8);
+    }
   }
   std::vector<double> ll ((size_t) b->nPairs), cnt (T);
   MB_CUDA (cudaMemcpy (ll.data(), dLL, (size_t) b->nPairs * 8, cudaMemcpyDeviceToHost));
   for (int64_t k: pairs) loglike[k] = ll[k];
-  if (wantCounts) {
+  if (wantCounts && !rows) {
     MB_CUDA (cudaMemcpy (cnt.data(), dCounts, T * 8, cudaMemcpyDeviceToHost));
     for (int64_t t = 0; t < m->T; ++t) hostCounts[t] += cnt[t];
   }
   if (ws_bytes (b, WS_F) > kKeepScratchBytes) ws_release (b, WS_F);
+  if (ws_bytes (b, WS_COUNTS) > kKeepScratchBytes) ws_release (b, WS_COUNTS);
   return 0;
 }
 
 // The same E-step with the scaled linear-domain kernels: Forward stores the high words of its values
 // (4 bytes per cell-state) and the frame of every rescale block; Backward multiplies them back in.
-// Pairs the Forward sweep flags, and whole chunks in which the Backward sweep flags a pair, are
-// handed to counts_log.
+// Pairs the Forward sweep flags are handed to counts_log.  Summed counts: a chunk in which the Backward
+// sweep flags a pair is handed over whole (its linear counts are already mixed into one vector).  Per-pair
+// rows: only the flagged pairs are handed over; their chunk-mates keep their linear rows.
 static int counts_lin (mb_machine* m, mb_batch* b, const std::vector<int64_t>& pairs, bool wantCounts,
-                       std::vector<double>& hostCounts, double* loglike, int64_t& launches, double& ms) {
+                       std::vector<double>& hostCounts, double* loglike, int64_t& launches, double& ms, double* rows = nullptr) {
   JitEngine& J = *(JitEngine*) m->jit;
   const int W = 32 * J.C;
+  const int64_t rowWords = rows ? 2 * m->T : 0;      // a pair's row of counts, in 32-bit words
   double wanted = 0;
   for (int64_t k: pairs)
-    wanted += 4.0 * (double) ((((b->xOff[k + 1] - b->xOff[k]) + W) / W) * ((b->yOff[k + 1] - b->yOff[k]) + 32) * (int64_t) (32 * J.C * J.storeQ * 4));
+    wanted += 4.0 * (double) ((((b->xOff[k + 1] - b->xOff[k]) + W) / W) * ((b->yOff[k + 1] - b->yOff[k]) + 32) * (int64_t) (32 * J.C * J.storeQ * 4) + rowWords);
   const double budget = memory_budget (m, b, WS_F, wanted, "jit_f_budget_mb") / 4.0;     // in 32-bit words
   std::vector<std::vector<int64_t>> chunks (1);
-  std::vector<int64_t> fOffHost ((size_t) b->nPairs, 0), efOffHost ((size_t) b->nPairs, 0), chunkWords (1, 0), chunkEf (1, 0);
+  std::vector<int64_t> fOffHost ((size_t) b->nPairs, 0), efOffHost ((size_t) b->nPairs, 0), rowOfHost ((size_t) b->nPairs, 0), chunkWords (1, 0), chunkEf (1, 0);
   for (int64_t k: pairs) {
     const int64_t Li = b->xOff[k + 1] - b->xOff[k], Lo = b->yOff[k + 1] - b->yOff[k];
     // one block of 32 lanes x C cells x ceil(S/4) 16-byte chunks per (strip, step), in the order the sweep produces them
     const int64_t need = ((Li + W) / W) * (Lo + 32) * (int64_t) (32 * J.C * J.storeQ * 4);
     const int64_t needEf = ((Li + W) / W) * ((Lo + 32 + 15) / 16);
-    if ((double) need > budget) { set_error ("pair " + std::to_string (k) + ": the Forward matrix does not fit in device memory"); return 1; }
-    if (!chunks.back().empty() && (double) (chunkWords.back() + need) > budget) { chunks.emplace_back(); chunkWords.push_back (0); chunkEf.push_back (0); }
+    if ((double) (need + rowWords) > budget) { set_error ("pair " + std::to_string (k) + ": the Forward matrix does not fit in device memory"); return 1; }
+    if (!chunks.back().empty() && (double) (chunkWords.back() + need + (int64_t) (chunks.back().size() + 1) * rowWords) > budget) { chunks.emplace_back(); chunkWords.push_back (0); chunkEf.push_back (0); }
     fOffHost[k] = chunkWords.back();
     efOffHost[k] = chunkEf.back();
+    rowOfHost[k] = (int64_t) chunks.back().size();
     chunkWords.back() += need;
     chunkEf.back() += needEf;
     chunks.back().push_back (k);
   }
   int64_t maxChunk = 0, maxEf = 0;
+  size_t maxPairs = 0;
   for (int64_t v: chunkWords) maxChunk = std::max (maxChunk, v);
   for (int64_t v: chunkEf) maxEf = std::max (maxEf, v);
+  for (auto& c: chunks) maxPairs = std::max (maxPairs, c.size());
   const size_t T = (size_t) std::max<int64_t> (m->T, 1);
+  const size_t countDoubles = rows ? maxPairs * T : T;
   unsigned* dF32 = (unsigned*) ws_reserve (b, WS_F, (size_t) maxChunk * 4);
   int32_t* dEf = (int32_t*) ws_reserve (b, WS_EF, (size_t) std::max<int64_t> (maxEf, 1) * 4);
   double* dLL = (double*) ws_reserve (b, WS_RESULT, (size_t) b->nPairs * 8);
   double* dBack = (double*) ws_reserve (b, WS_RESULT2, (size_t) b->nPairs * 8);
   int64_t* dFOff = (int64_t*) ws_reserve (b, WS_FOFF, (size_t) b->nPairs * 8);
   int64_t* dEfOff = (int64_t*) ws_reserve (b, WS_EFOFF, (size_t) b->nPairs * 8);
-  double* dCounts = (double*) ws_reserve (b, WS_COUNTS, T * 8);
+  double* dCounts = (double*) ws_reserve (b, WS_COUNTS, countDoubles * 8);
   int32_t* dFlag = (int32_t*) ws_reserve (b, WS_FLAG, (size_t) b->nPairs * 4);
-  if (!dF32 || !dEf || !dLL || !dBack || !dFOff || !dEfOff || !dCounts || !dFlag) return 1;
+  int64_t* dRowOf = rows ? (int64_t*) ws_reserve (b, WS_ROWOF, (size_t) b->nPairs * 8) : nullptr;
+  if (!dF32 || !dEf || !dLL || !dBack || !dFOff || !dEfOff || !dCounts || !dFlag || (rows && !dRowOf)) return 1;
   MB_CUDA (cudaMemcpyAsync (dFOff, fOffHost.data(), (size_t) b->nPairs * 8, cudaMemcpyHostToDevice, b->stream));
   MB_CUDA (cudaMemcpyAsync (dEfOff, efOffHost.data(), (size_t) b->nPairs * 8, cudaMemcpyHostToDevice, b->stream));
+  if (rows) MB_CUDA (cudaMemcpyAsync (dRowOf, rowOfHost.data(), (size_t) b->nPairs * 8, cudaMemcpyHostToDevice, b->stream));
   std::vector<int64_t> redo;
-  std::vector<double> ll ((size_t) b->nPairs), cnt (T);
+  std::vector<double> ll ((size_t) b->nPairs), cnt (countDoubles);
   std::vector<int32_t> flag ((size_t) b->nPairs);
   for (size_t c = 0; c < chunks.size(); ++c) {
     CountArgs ca;
-    ca.F32 = dF32; ca.f32Off = dFOff; ca.ef = dEf; ca.efOff = dEfOff; ca.ll = dLL; ca.counts = dCounts; ca.flag = dFlag;
+    ca.F32 = dF32; ca.f32Off = dFOff; ca.ef = dEf; ca.efOff = dEfOff; ca.ll = dLL; ca.counts = dCounts; ca.flag = dFlag; ca.rowOf = dRowOf;
     if (timing_begin (b)) return 1;
     MB_CUDA (cudaMemsetAsync (dFlag, 0, (size_t) b->nPairs * 4, b->stream));
     if (launch (m, b, 7, cost_order (b, chunks[c]), dLL, nullptr, nullptr, ca)) return 1;
@@ -1680,39 +1744,51 @@ static int counts_lin (mb_machine* m, mb_batch* b, const std::vector<int64_t>& p
       if (flag[k] || !(ll[k] > -INFINITY)) redo.push_back (k);
       else { good.push_back (k); loglike[k] = ll[k]; }
     }
+    const size_t nCounts = rows ? chunks[c].size() * T : T;
     if (wantCounts && !good.empty()) {
-      MB_CUDA (cudaMemsetAsync (dCounts, 0, T * 8, b->stream));
+      MB_CUDA (cudaMemsetAsync (dCounts, 0, nCounts * 8, b->stream));
       MB_CUDA (cudaMemsetAsync (dFlag, 0, (size_t) b->nPairs * 4, b->stream));
       if (launch (m, b, 8, cost_order (b, good), dBack, nullptr, nullptr, ca)) return 1;
       ++launches;
       MB_CUDA (cudaMemcpyAsync (flag.data(), dFlag, (size_t) b->nPairs * 4, cudaMemcpyDeviceToHost, b->stream));
-      MB_CUDA (cudaMemcpyAsync (cnt.data(), dCounts, T * 8, cudaMemcpyDeviceToHost, b->stream));
+      MB_CUDA (cudaMemcpyAsync (cnt.data(), dCounts, nCounts * 8, cudaMemcpyDeviceToHost, b->stream));
       MB_CUDA (cudaStreamSynchronize (b->stream));
-      bool anyFlag = false;
-      for (int64_t k: good) anyFlag |= flag[k] != 0;
-      if (anyFlag) redo.insert (redo.end(), good.begin(), good.end());     // discard this chunk's linear counts
-      else for (int64_t t = 0; t < m->T; ++t) hostCounts[t] += cnt[t];
+      if (rows) {
+        for (int64_t k: good)
+          if (flag[k]) redo.push_back (k);      // its row is left to the log-domain re-run
+          else memcpy (rows + k * m->T, cnt.data() + rowOfHost[k] * (int64_t) T, (size_t) m->T * 8);
+      } else {
+        bool anyFlag = false;
+        for (int64_t k: good) anyFlag |= flag[k] != 0;
+        if (anyFlag) redo.insert (redo.end(), good.begin(), good.end());     // discard this chunk's linear counts
+        else for (int64_t t = 0; t < m->T; ++t) hostCounts[t] += cnt[t];
+      }
     }
     if (timing_end (b, launches)) return 1;
     ms += b->lastMs;
   }
   if (ws_bytes (b, WS_F) > kKeepScratchBytes) ws_release (b, WS_F);
+  if (ws_bytes (b, WS_COUNTS) > kKeepScratchBytes) ws_release (b, WS_COUNTS);
   b->lastRedo = (int64_t) redo.size();
   std::sort (redo.begin(), redo.end());
-  return counts_log (m, b, redo, wantCounts, hostCounts, loglike, launches, ms);
+  return counts_log (m, b, redo, wantCounts, hostCounts, loglike, launches, ms, rows);
 }
 
-int jit_counts (mb_machine* m, mb_batch* b, double* counts, double* loglike) {
+// rows == nullptr: counts[nTrans] summed over the batch (counts may be null: log-likelihoods only);
+// otherwise rows[nPairs][nTrans], pair k's counts in row k (counts unused)
+int jit_counts (mb_machine* m, mb_batch* b, double* counts, double* loglike, double* rows) {
   JitEngine& J = *(JitEngine*) m->jit;
   if (counts) for (int64_t t = 0; t < m->T; ++t) counts[t] = 0;
+  if (rows) for (int64_t q = 0; q < b->nPairs * m->T; ++q) rows[q] = 0;
   if (b->nPairs == 0) return 0;
   std::vector<int64_t> all ((size_t) b->nPairs);
   for (int64_t k = 0; k < b->nPairs; ++k) all[k] = k;
   std::vector<double> hostCounts ((size_t) std::max<int64_t> (m->T, 1), 0.), ll ((size_t) b->nPairs, 0.);
   int64_t launches = 0;
   double ms = 0;
-  const int rc = J.linearOK ? counts_lin (m, b, all, counts != nullptr, hostCounts, ll.data(), launches, ms)
-                            : counts_log (m, b, all, counts != nullptr, hostCounts, ll.data(), launches, ms);
+  const bool want = counts != nullptr || rows != nullptr;
+  const int rc = J.linearOK ? counts_lin (m, b, all, want, hostCounts, ll.data(), launches, ms, rows)
+                            : counts_log (m, b, all, want, hostCounts, ll.data(), launches, ms, rows);
   if (rc) return rc;
   b->lastMs = ms;
   b->lastLaunches = launches;

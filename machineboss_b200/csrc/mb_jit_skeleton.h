@@ -44,6 +44,7 @@ struct MBArgs {
   // prog[w] how many rows of it are complete, strip s + 1 (item w + 1, claimed later, hence never waited for by
   // its predecessor) waits until the rows it is about to stage are there.  items == 0: a warp takes whole pairs.
   const int64_t* items; const int64_t* itemBnd; int* prog;
+  const int64_t* rowOf;                  // per pair: its row of counts, [row][MB_NTRANS] (per-pair count kernels, MB_PAIR_ROWS)
 };
 
 // Split mode is compiled into a module of its own (MB_SPLIT 1, built the first time a call needs it): in the ordinary
@@ -127,6 +128,15 @@ template<int DIR> __device__ __forceinline__ double mb_res_log (const MBSilN& P)
 
 template<bool B> struct MBBool { static constexpr bool value = B; };
 
+// where a count kernel adds pair k's counts: the summed vector, or (ROWS) the pair's row.  The warps that sweep strips of
+// one pair add into the same row, as they add into the same summed vector.
+template<bool ROWS> __device__ __forceinline__ double* mb_count_row (const MBArgs& A, const int64_t k) {
+#ifdef MB_PAIR_ROWS
+  if (ROWS) return A.counts + A.rowOf[k] * (int64_t) MB_NTRANS;
+#endif
+  return A.counts;
+}
+
 template<int DIR> struct MBDir { };
 template<> struct MBDir<0> { static const int NE = MB_NEMIT_F; static const int RES = MB_S - 1; };
 template<> struct MBDir<1> { static const int NE = MB_NEMIT_B; static const int RES = 0; };
@@ -144,7 +154,8 @@ template<int DIR> __device__ __forceinline__ constexpr bool mb_live (int s) { re
 // MODE 3: Backward fused with the posterior-count accumulation of BackwardMatrix::getCounts
 //         (backward.cpp:62-87): each transition group's term w + B(dest) is formed once and used
 //         both for the Backward log-sum-exp and for exp(F(src) - ll + term).
-template<int MODE, int DIR>
+// ROWS (mode 3): the counts of pair k go to its own row, A.counts + A.rowOf[k] * MB_NTRANS, instead of one summed vector.
+template<int MODE, int DIR, bool ROWS = false>
 __device__ __forceinline__ void mb_run (const MBSil& P, const MBArgs& A) {
   extern __shared__ double mb_smem[];
   double* E = mb_smem;
@@ -393,12 +404,13 @@ __device__ __forceinline__ void mb_run (const MBSil& P, const MBArgs& A) {
         for (; t < nSteps; ++t) { if ((t & 31) == 0) blockStart (t); step (t, MBBool<false>()); }
       }
       if (publishes) mb_publish_rows (A.prog + w, Lo + 1);
-      if (MODE == 3) mb_flush_counts (cs, acc, ta, A.counts, A.idTabB, lane);
+      if (MODE == 3) mb_flush_counts (cs, acc, ta, mb_count_row<ROWS> (A, k), A.idTabB, lane);
       __syncwarp();
     }
   }
 }
 
+#ifndef MB_PAIR_ROWS
 #ifndef MB_SCORE_MODULE
 extern "C" __global__ void __launch_bounds__(MB_THREADS, MB_MINBLOCKS) mb_k_forward (const __grid_constant__ MBSil P, const __grid_constant__ MBArgs A) { mb_run<0, 0> (P, A); }
 extern "C" __global__ void __launch_bounds__(MB_THREADS, MB_MINBLOCKS) mb_k_backward (const __grid_constant__ MBSil P, const __grid_constant__ MBArgs A) { mb_run<0, 1> (P, A); }
@@ -407,6 +419,7 @@ extern "C" __global__ void __launch_bounds__(MB_THREADS, MB_MINBLOCKS_CNT) mb_k_
 #endif
 extern "C" __global__ void __launch_bounds__(MB_THREADS, MB_MINBLOCKS) mb_k_viterbi (const __grid_constant__ MBSil P, const __grid_constant__ MBArgs A) { mb_run<1, 0> (P, A); }
 extern "C" __global__ void __launch_bounds__(MB_THREADS, MB_MINBLOCKS) mb_k_viterbi_score (const __grid_constant__ MBSil P, const __grid_constant__ MBArgs A) { mb_run<4, 0> (P, A); }
+#endif
 
 // ---------------------------------------------------------------------------------------------
 // Scaled linear-domain sweep (Forward for DIR 0, Backward for DIR 1).
@@ -435,7 +448,7 @@ extern "C" __global__ void __launch_bounds__(MB_THREADS, MB_MINBLOCKS) mb_k_vite
 // every rescale block.
 // MODE 3 (DIR 1): Backward fused with the posterior counts: for each transition group the product
 // term = B(dest) * w feeds the Backward sum and, times F(src) * 2^(eF + eB) / Z, the group's count.
-template<int MODE, int DIR, class SIL>
+template<int MODE, int DIR, class SIL, bool ROWS = false>
 __device__ __forceinline__ void mb_run_lin (const SIL& P, const MBArgs& A) {
 #ifdef MB_LANE_FRAMES
   constexpr bool LF = MODE == 0;
@@ -797,13 +810,14 @@ __device__ __forceinline__ void mb_run_lin (const SIL& P, const MBArgs& A) {
       }
       if (publishes) mb_publish_rows (A.prog + w, Lo + 1);
       suspect = (int) __reduce_or_sync (MB_FULL, (unsigned) suspect);      // why: 1 spread, 2 neighbour frame, 4 boundary frame
-      if (MODE == 3) mb_flush_counts_lin (csd, accd, ta, A.counts, A.idTabB, lane);
+      if (MODE == 3) mb_flush_counts_lin (csd, accd, ta, mb_count_row<ROWS> (A, k), A.idTabB, lane);
       __syncwarp();
     }
     if (lane == 0) { if (split) { if (suspect) atomicOr (A.flag + k, suspect); } else A.flag[k] = suspect; }
   }
 }
 
+#ifndef MB_PAIR_ROWS
 #ifdef MB_ROWTAB
 extern "C" __global__ void __launch_bounds__(MB_THREADS, MB_MINBLOCKS_LIN) mb_k_forward_lin (const __grid_constant__ MBSilN P, const __grid_constant__ MBArgs A) { mb_run_lin<0, 0> (P, A); }
 extern "C" __global__ void __launch_bounds__(MB_THREADS, MB_MINBLOCKS_LIN) mb_k_backward_lin (const __grid_constant__ MBSilN P, const __grid_constant__ MBArgs A) { mb_run_lin<0, 1> (P, A); }
@@ -814,6 +828,12 @@ extern "C" __global__ void __launch_bounds__(MB_THREADS, MB_MINBLOCKS_LIN) mb_k_
 #ifndef MB_SCORE_MODULE
 extern "C" __global__ void __launch_bounds__(MB_THREADS, MB_MINBLOCKS_LIN) mb_k_fstore_lin (const __grid_constant__ MBSil P, const __grid_constant__ MBArgs A) { mb_run_lin<2, 0> (P, A); }
 extern "C" __global__ void __launch_bounds__(MB_THREADS, MB_MINBLOCKS_CNT) mb_k_bcounts_lin (const __grid_constant__ MBSil P, const __grid_constant__ MBArgs A) { mb_run_lin<3, 1> (P, A); }
+#endif
+#else
+// the per-pair count module (built the first time a call asks for per-pair counts): only the two count kernels, each
+// flushing into the row of its pair
+extern "C" __global__ void __launch_bounds__(MB_THREADS, MB_MINBLOCKS_CNT) mb_k_bcounts_rows (const __grid_constant__ MBSil P, const __grid_constant__ MBArgs A) { mb_run<3, 1, true> (P, A); }
+extern "C" __global__ void __launch_bounds__(MB_THREADS, MB_MINBLOCKS_CNT) mb_k_bcounts_lin_rows (const __grid_constant__ MBSil P, const __grid_constant__ MBArgs A) { mb_run_lin<3, 1, MBSil, true> (P, A); }
 #endif
 )MBSRC";
 

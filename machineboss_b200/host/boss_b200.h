@@ -606,6 +606,8 @@ public:
     if (gb) mbCheck (mb_group_viterbi_paths_narrow (gb, ids, bytesPerId, off)); else mbCheck (mb_viterbi_paths_narrow (single->handle(), ids, bytesPerId, off));
   }
   void counts (double* c, double* ll) { if (gb) mbCheck (mb_group_counts (gm, gb, c, ll)); else mbCheck (mb_counts (machine.handle(), single->handle(), c, ll)); }
+  // c: [size()][nTransitions], pair k's counts in row k
+  void pairCounts (double* c, double* ll) { if (gb) mbCheck (mb_group_pair_counts (gm, gb, c, ll)); else mbCheck (mb_pair_counts (machine.handle(), single->handle(), c, ll)); }
 private:
   const EvaluatedMachine& machine;
   int64_t n;
@@ -952,6 +954,23 @@ inline vector<vector<MachinePath> > posteriorPaths (const EvaluatedMachine& m, c
     unpack (ids);
   }
   return paths;
+}
+
+// The MachineCounts of each pair of the list on its own, in list order, from one device call (mb_pair_counts; dealt over the
+// box's GPUs like MachineCounts over a list): element k is MachineCounts (m, pair k), its loglike pair k's log-likelihood.
+inline vector<MachineCounts> pairCounts (const EvaluatedMachine& m, const SeqPairList& l) {
+  const size_t n = l.seqPairs.size(), T = (size_t) m.nTransitions;
+  vector<MachineCounts> out (n, MachineCounts (m));
+  if (!n) return out;
+  ListBatch b (m, pairPointers (l));
+  vector<double> c (n * T ? n * T : 1, 0.), ll (n, 0.);
+  b.pairCounts (c.data(), ll.data());
+  for (size_t k = 0; k < n; ++k) {
+    for (StateIndex s = 0; s < m.nStates(); ++s)
+      for (size_t t = 0; t < out[k].count[s].size(); ++t) out[k].count[s][t] = c[k * T + m.state[s].transOffset + t];
+    out[k].loglike = ll[k];
+  }
+  return out;
 }
 
 // api.h:25-31 equivalents taking an already-evaluated machine

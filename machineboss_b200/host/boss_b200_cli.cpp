@@ -16,6 +16,8 @@
 //   -V, --viterbi   Viterbi log-likelihoods, same layout                     (boss.cpp:819-848)
 //   -A, --align     Viterbi alignments as a SeqPairList with meta.path       (boss.cpp:833,843-846)
 //   -C, --counts    raw expected transition counts, MachineCounts::writeJson (counts.cpp:73-78)
+//   -C --per-pair   a JSON array with one counts object per pair, in list order: each is what -C prints for that pair
+//                   alone (pairCounts: the whole list in one device call)
 //   --sample-paths SEED   one path per pair drawn from the posterior, ForwardMatrix::samplePath (forward.cpp:17-23)
 //   --posterior-paths N [--posterior-seed S]   N paths per pair drawn from the posterior for the whole list at once on the
 //                   device (posteriorPaths, default seed 1): [[[transition ids], ...N], ...], [] for a pair without a path
@@ -99,6 +101,7 @@ int main (int argc, char** argv) {
     unsigned rngSeed = 5489u;     // mt19937's default seed
     string kernelCache;           // empty: none
     bool fastIngest = false, ingestOnly = false;
+    bool perPair = false;         // -C: counts of each pair on its own
     string pairedFastaIn, pairedFastaOut;
     for (int a = 1; a < argc; ++a) {
       const string f = argv[a];
@@ -120,6 +123,7 @@ int main (int argc, char** argv) {
       else if (f == "-V" || f == "--viterbi") doV = true;
       else if (f == "-A" || f == "--align") doA = true;
       else if (f == "-C" || f == "--counts") doC = true;
+      else if (f == "--per-pair") perPair = true;
       else if (f == "--envelope") envMode = next();      // full | path | <width>: print each pair's Envelope (t/src/testenv.cpp; no device needed)
       else if (f == "--sample-paths") { doSample = true; sampleSeed = atoll (next().c_str()); }
       else if (f == "--posterior-paths") { posteriorN = atoi (next().c_str()); if (posteriorN < 1) throw runtime_error ("--posterior-paths needs a count of at least 1"); }
@@ -256,6 +260,7 @@ int main (int argc, char** argv) {
     if (data.seqPairs.empty() && inputEmpty && outputEmpty) data.seqPairs.push_back (SeqPair());   // boss.cpp:769-770
     if (data.seqPairs.empty()) throw runtime_error ("no sequence data given");
     if (!(doL || doV || doA || doC || doT || doSample || posteriorN || postTransTop)) throw runtime_error ("nothing to do: give -L, -V, -A, -C or -T");
+    if (perPair && !doC) throw runtime_error ("--per-pair goes with -C");
 
     if (doT) {   // boss.cpp:776-787
       if (constraints.empty() && machine.cons.empty()) throw runtime_error ("To fit parameters, please specify a constraints file and (for machines with input/output) a data file");
@@ -316,14 +321,29 @@ int main (int argc, char** argv) {
     if (doL) printScores (forwardLogLikes (eval, ok));
     if (doC) {
       // ... but -C does not test canTokenize (boss.cpp:811-816): an unknown symbol throws
-      const MachineCounts counts (eval, data);
-      if (symbolic) {   // MachineCounts::writeParamCountsJson (counts.cpp:80-87)
-        cout << "{";
-        size_t np = 0;
-        for (const auto& nc: paramCounts (counts, machine, params)) cout << (np++ ? "," : "") << "\"" << Json::escape (nc.first) << "\":" << nc.second;
-        cout << "}" << endl;
-      } else
-      counts.writeJson (cout);
+      auto writeCounts = [&] (const MachineCounts& counts) {
+        if (symbolic) {   // MachineCounts::writeParamCountsJson (counts.cpp:80-87)
+          cout << "{";
+          size_t np = 0;
+          for (const auto& nc: paramCounts (counts, machine, params)) cout << (np++ ? "," : "") << "\"" << Json::escape (nc.first) << "\":" << nc.second;
+          cout << "}";
+        } else {
+          std::ostringstream os;
+          counts.writeJson (os);
+          string js = os.str();
+          while (js.size() && js.back() == '\n') js.pop_back();
+          cout << js;
+        }
+      };
+      if (perPair) {
+        cout << "[";
+        size_t k = 0;
+        for (const auto& counts: pairCounts (eval, data)) { cout << (k++ ? ",\n " : ""); writeCounts (counts); }
+        cout << "]" << endl;
+      } else {
+        writeCounts (MachineCounts (eval, data));
+        cout << endl;
+      }
     }
     if (postTransTop) {   // BackwardMatrix::postTransQueue (backward.cpp:52-56) and traceFrom (backward.cpp:98-108), per pair
       cout << "[";
