@@ -164,6 +164,34 @@ int mb_sample_paths (mb_machine* m, mb_batch* b, int32_t nSamples, uint64_t seed
  * path r = k * nSamples + j goes to elements pathOff[r] .. pathOff[r] + pathLen[r]. */
 int mb_sampled_paths (mb_batch* b, void* pathTrans, int32_t bytesPerId, const int64_t* pathOff);
 
+/* ---- posterior decoding (BackwardMatrix::postTransQueue / traceFrom, src/backward.cpp:52-56,89-108, for a whole batch) ----
+ * A step of a path takes transition t from cell (i, o), state src, to cell (i + di, o + do), state dst.  Its posterior
+ * probability, the probability that a path drawn from the posterior takes t from that cell, is
+ *     gamma = exp ((F(i, o)[src] - ll) + (B(i + di, o + do)[dst] + w_t))
+ * over the generic engine's log-domain Forward and Backward matrices, ll = B(0, 0)[0] the Backward log-likelihood; bit for bit
+ * the term mb_pair_counts adds to the pair's row (backward.cpp:66); 0 when ll is -inf.  A step is admissible when
+ * F(i, o)[src] + w_t + B(i + di, o + do)[dst] is finite (it lies on a complete path of finite weight).  The gain of a path is the
+ * sum over its steps of c(t) * gamma, c(t) the number of tokens t consumes (2 match, 1 insert or delete, 0 silent): the expected
+ * number of the pair's tokens that a posterior path consumes with the same transition from the same cell, in [0, inLen + outLen].
+ * The maximum expected accuracy (MEA) path is the admissible path from (0, 0, state 0) to (inLen, outLen, end state) of largest
+ * gain: A(0, 0)[0] = 0, A(cell)[s] = max over admissible candidates of A(source cell)[src] + c(t) * gamma, candidates in the
+ * traceback's order (match, delete, insert, silent; each by source state then transition index), the first maximum winning;
+ * cells outside the envelope are -inf.
+ *
+ * mb_mea: the MEA path of every pair.  gain[k] its gain (-inf for an impossible pair, whose path has length 0), loglike[k]
+ * (may be NULL) the Forward log-likelihood, pathLen[k] (may be NULL) its number of steps.  Runs on the generic engine, three
+ * full matrices per pair.  The paths are kept apart from mb_viterbi's and mb_sample_paths'; a failed call leaves none stored. */
+int mb_mea (mb_machine* m, mb_batch* b, double* gain, double* loglike, int64_t* pathLen);
+/* The ids of the last mb_mea on this batch, narrowed to bytesPerId = 1, 2 or 4 as in mb_sampled_paths: pair k's path goes to
+ * pathTrans[pathOff[k] .. pathOff[k] + pathLen[k]); stepPost (may be NULL) receives gamma of each step at the same offsets. */
+int mb_mea_paths (mb_batch* b, void* pathTrans, int32_t bytesPerId, const int64_t* pathOff, double* stepPost);
+/* gamma of each step of caller-supplied paths: path r belongs to pair pairOfPath[r] and holds pathTrans[pathOff[r] ..
+ * pathOff[r] + pathLen[r]); stepPost uses the same offsets.  A path must be a path of its pair: each step leaves the state the
+ * path is in and reads the pair's next tokens, stays in the envelope, and the path ends at (inLen, outLen, end state); the
+ * first path that is not fails the call with a message naming the path and the step.  Runs on the generic engine. */
+int mb_path_posteriors (mb_machine* m, mb_batch* b, int64_t nPaths, const int64_t* pairOfPath,
+                        const int32_t* pathTrans, const int64_t* pathOff, const int64_t* pathLen, double* stepPost);
+
 /* ---- one list of pairs over several GPUs of a box (SURVEY.md 8e) ----
  * Replaces the reference's single-core loops over a SeqPairList: MachineCounts (counts.cpp:37-43) inside
  * MachineFitter::fit (fitter.cpp:23-47), and the -L / -A loops of the CLI (boss.cpp:796,826).  The pairs are

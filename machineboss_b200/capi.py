@@ -21,7 +21,7 @@ _lib = None
 SYMBOLS = ["mb_last_error", "mb_version", "mb_set_kernel_cache_dir", "mb_device_count", "mb_set_device", "mb_set_engine", "mb_set_option", "mb_machine_set_option",
            "mb_machine_create", "mb_machine_update_weights", "mb_machine_info", "mb_machine_destroy",
            "mb_batch_create", "mb_batch_destroy", "mb_batch_trim", "mb_batch_set_envelopes", "mb_forward", "mb_backward", "mb_viterbi",
-           "mb_viterbi_paths", "mb_viterbi_paths_narrow", "mb_viterbi_paths_start", "mb_batch_wait", "mb_counts", "mb_pair_counts", "mb_matrix", "mb_sample_paths", "mb_sampled_paths", "mb_last_kernel_ms", "mb_last_redo", "mb_jit_compile_check", "mb_jit_host_tables", "mb_lane_emulate", "mb_col_emulate",
+           "mb_viterbi_paths", "mb_viterbi_paths_narrow", "mb_viterbi_paths_start", "mb_batch_wait", "mb_counts", "mb_pair_counts", "mb_matrix", "mb_sample_paths", "mb_sampled_paths", "mb_mea", "mb_mea_paths", "mb_path_posteriors", "mb_last_kernel_ms", "mb_last_redo", "mb_jit_compile_check", "mb_jit_host_tables", "mb_lane_emulate", "mb_col_emulate",
            "mb_shard_pairs", "mb_group_create", "mb_group_info", "mb_group_destroy", "mb_group_machine_create", "mb_group_machine_update_weights",
            "mb_group_machine_set_option", "mb_group_machine_info", "mb_group_machine_destroy", "mb_group_batch_create", "mb_group_batch_set_envelopes",
            "mb_group_batch_shard", "mb_group_batch_destroy", "mb_group_forward", "mb_group_backward", "mb_group_viterbi", "mb_group_viterbi_paths",
@@ -69,6 +69,9 @@ def lib():
         L.mb_matrix.argtypes = [P, P, I64, I32, P]
         L.mb_sample_paths.argtypes = [P, P, I32, ctypes.c_uint64, P, P]
         L.mb_sampled_paths.argtypes = [P, P, I32, P]
+        L.mb_mea.argtypes = [P, P, P, P, P]
+        L.mb_mea_paths.argtypes = [P, P, I32, P, P]
+        L.mb_path_posteriors.argtypes = [P, P, I64, P, P, P, P, P]
         L.mb_jit_compile_check.argtypes = [I32, I32, I32, I64, P, P, P, P, ctypes.c_char_p, I64]
         L.mb_jit_host_tables.argtypes = [I32, I32, I32, I64, P, P, P, P, P, I32, P, I64, ctypes.POINTER(I64)]
         L.mb_lane_emulate.argtypes = [I32, I32, I32, I64, P, P, P, P, P, P, I64, I32, ctypes.POINTER(D), P, P]
@@ -406,6 +409,38 @@ def sample_paths(m: Machine, b: Batch, n: int, seed: int, bytes_per_id: int = 4)
     if off[-1]:
         _check(lib().mb_sampled_paths(b.h, _ptr(ids), int(bytes_per_id), _ptr(off)))
     return ll[: b.n_pairs], plen.reshape(b.n_pairs, n), off, ids
+
+
+def mea(m: Machine, b: Batch, bytes_per_id: int = 4):
+    """Maximum expected accuracy path of every pair (mb_mea / mb_mea_paths).  Returns (gain[nPairs], loglike[nPairs],
+    lengths[nPairs], offsets[nPairs + 1], ids, post): pair k's path is ids[offsets[k]:offsets[k + 1]] (int32, or uint8 / uint16
+    with bytes_per_id 1 / 2) and post[offsets[k]:offsets[k + 1]] the posterior probability of each of its steps."""
+    gain = np.empty(max(b.n_pairs, 1), dtype=np.float64)
+    ll = np.empty(max(b.n_pairs, 1), dtype=np.float64)
+    plen = np.zeros(max(b.n_pairs, 1), dtype=np.int64)
+    _check(lib().mb_mea(m.h, b.h, gain.ctypes.data, ll.ctypes.data, plen.ctypes.data))
+    plen = plen[: b.n_pairs]
+    off = np.concatenate([[0], np.cumsum(plen)]).astype(np.int64)
+    ids = np.empty(int(off[-1]), dtype={1: np.uint8, 2: np.uint16, 4: np.int32}[bytes_per_id])
+    post = np.empty(int(off[-1]), dtype=np.float64)
+    if off[-1]:
+        _check(lib().mb_mea_paths(b.h, _ptr(ids), int(bytes_per_id), _ptr(off), _ptr(post)))
+    return gain[: b.n_pairs], ll[: b.n_pairs], plen, off, ids, post
+
+
+def path_posteriors(m: Machine, b: Batch, pair_of_path, offsets, ids) -> np.ndarray:
+    """Posterior probability of each step of given paths (mb_path_posteriors): path r belongs to pair pair_of_path[r] and is
+    ids[offsets[r]:offsets[r + 1]]; the result has the same layout as ids."""
+    pair_of_path = np.ascontiguousarray(pair_of_path, dtype=np.int64)
+    offsets = np.ascontiguousarray(offsets, dtype=np.int64)
+    ids = np.ascontiguousarray(ids, dtype=np.int32)
+    n = int(pair_of_path.shape[0])
+    assert offsets.shape[0] == n + 1
+    lengths = np.ascontiguousarray(np.diff(offsets), dtype=np.int64)
+    starts = np.ascontiguousarray(offsets[:-1])
+    post = np.empty(max(int(offsets[-1]), 1), dtype=np.float64)
+    _check(lib().mb_path_posteriors(m.h, b.h, n, _ptr(pair_of_path), _ptr(ids), _ptr(starts), _ptr(lengths), post.ctypes.data))
+    return post[: int(offsets[-1])]
 
 
 def counts(m: Machine, b: Batch):

@@ -164,22 +164,37 @@ static void pooled_free (int device, void* p, size_t bytes) {
   } else cudaFree (p);
 }
 
-// room for `need` packed path entries in ps.dPaths, keeping what is already there (chunked tracebacks append)
-int paths_reserve (mb_batch* b, PathStore& ps, int64_t need) {
-  if (need <= ps.pathsCapacity) return 0;
-  const int64_t want = std::max<int64_t> (need, 2 * ps.pathsCapacity);
+// room for `need` elements of `elem` bytes in the pooled block *p (capacity *cap elements, *bytes bytes), keeping what is already
+// there (chunked tracebacks append)
+static int grow_keep (mb_batch* b, void** p, int64_t* cap, size_t* bytes, int64_t need, size_t elem) {
+  if (need <= *cap) return 0;
+  const int64_t want = std::max<int64_t> (need, 2 * *cap);
   size_t got = 0;
-  int32_t* p = (int32_t*) pooled_alloc (b->device, (size_t) want * 4, &got);
-  if (!p) return 1;
-  if (ps.dPaths) {
-    MB_CUDA (cudaMemcpyAsync (p, ps.dPaths, (size_t) ps.pathsCapacity * 4, cudaMemcpyDeviceToDevice, b->stream));
+  void* q = pooled_alloc (b->device, (size_t) want * elem, &got);
+  if (!q) return 1;
+  if (*p) {
+    MB_CUDA (cudaMemcpyAsync (q, *p, (size_t) *cap * elem, cudaMemcpyDeviceToDevice, b->stream));
     MB_CUDA (cudaStreamSynchronize (b->stream));
-    pooled_free (b->device, ps.dPaths, ps.pathsBytes);
+    pooled_free (b->device, *p, *bytes);
   }
-  ps.dPaths = p;
-  ps.pathsBytes = got;
-  ps.pathsCapacity = (int64_t) (got / 4);
+  *p = q;
+  *bytes = got;
+  *cap = (int64_t) (got / elem);
   return 0;
+}
+
+int paths_reserve (mb_batch* b, PathStore& ps, int64_t need) {
+  void* p = ps.dPaths;
+  const int rc = grow_keep (b, &p, &ps.pathsCapacity, &ps.pathsBytes, need, 4);
+  ps.dPaths = (int32_t*) p;
+  return rc;
+}
+
+int mea_post_reserve (mb_batch* b, int64_t need) {
+  void* p = b->dMeaPost;
+  const int rc = grow_keep (b, &p, &b->meaPostCapacity, &b->meaPostBytes, need, 8);
+  b->dMeaPost = (double*) p;
+  return rc;
 }
 
 int paths_place (mb_batch* b, PathStore& ps, const int64_t* rows, int64_t n, const int64_t* dLen, int64_t* dOutOff) {
@@ -268,7 +283,9 @@ static int upload_machine (mb_machine* m) {
     oOutOff = blob_reserve (bytes, m->hOut.off), oOutOther = blob_reserve (bytes, m->hOut.other),
     oOutId = blob_reserve (bytes, m->hOut.id), oOutLw = blob_reserve (bytes, m->hOut.lw),
     oFLO = blob_reserve (bytes, m->fwdLevelOff), oFLS = blob_reserve (bytes, m->fwdLevelStates),
-    oBLO = blob_reserve (bytes, m->bwdLevelOff), oBLS = blob_reserve (bytes, m->bwdLevelStates);
+    oBLO = blob_reserve (bytes, m->bwdLevelOff), oBLS = blob_reserve (bytes, m->bwdLevelStates),
+    oSrc = blob_reserve (bytes, m->src), oDst = blob_reserve (bytes, m->dst), oIn = blob_reserve (bytes, m->in),
+    oOut = blob_reserve (bytes, m->out), oLw = blob_reserve (bytes, m->lw);
   std::vector<char> host (bytes, 0);
   auto put = [&] (size_t at, const void* p, size_t n) { if (n) memcpy (host.data() + at, p, n); };
   put (oIncOff, m->hInc.off.data(), m->hInc.off.size() * 8); put (oIncOther, m->hInc.other.data(), m->hInc.other.size() * 4);
@@ -277,12 +294,15 @@ static int upload_machine (mb_machine* m) {
   put (oOutId, m->hOut.id.data(), m->hOut.id.size() * 4); put (oOutLw, m->hOut.lw.data(), m->hOut.lw.size() * 8);
   put (oFLO, m->fwdLevelOff.data(), m->fwdLevelOff.size() * 4); put (oFLS, m->fwdLevelStates.data(), m->fwdLevelStates.size() * 4);
   put (oBLO, m->bwdLevelOff.data(), m->bwdLevelOff.size() * 4); put (oBLS, m->bwdLevelStates.data(), m->bwdLevelStates.size() * 4);
+  put (oSrc, m->src.data(), m->src.size() * 4); put (oDst, m->dst.data(), m->dst.size() * 4);
+  put (oIn, m->in.data(), m->in.size() * 4); put (oOut, m->out.data(), m->out.size() * 4); put (oLw, m->lw.data(), m->lw.size() * 8);
   MB_CUDA (cudaSetDevice (m->device));
   MB_CUDA (cudaMalloc (&m->dBlob, bytes));
   MB_CUDA (cudaMemcpy (m->dBlob, host.data(), bytes, cudaMemcpyHostToDevice));
   m->blobBytes = bytes;
   m->incLwOffset = oIncLw;
   m->outLwOffset = oOutLw;
+  m->lwOffset = oLw;
   char* d = (char*) m->dBlob;
   DevMachine& dm = m->dev;
   dm.S = m->S; dm.nIn1 = m->nIn + 1; dm.nOut1 = m->nOut + 1;
@@ -292,6 +312,9 @@ static int upload_machine (mb_machine* m) {
   dm.nBwdLevels = (int32_t) m->bwdLevelOff.size() - 1;
   dm.fwdLevelOff = (const int32_t*) (d + oFLO); dm.fwdLevelStates = (const int32_t*) (d + oFLS);
   dm.bwdLevelOff = (const int32_t*) (d + oBLO); dm.bwdLevelStates = (const int32_t*) (d + oBLS);
+  dm.nTrans = m->T;
+  dm.tSrc = (const int32_t*) (d + oSrc); dm.tDst = (const int32_t*) (d + oDst);
+  dm.tIn = (const int32_t*) (d + oIn); dm.tOut = (const int32_t*) (d + oOut); dm.tLw = (const double*) (d + oLw);
   return 0;
 }
 
@@ -426,6 +449,7 @@ int mb_machine_update_weights (mb_machine* m, const double* logWeight) {
     MB_CUDA (cudaMemcpy ((char*) m->dBlob + m->incLwOffset, m->hInc.lw.data(), m->hInc.lw.size() * 8, cudaMemcpyHostToDevice));
     MB_CUDA (cudaMemcpy ((char*) m->dBlob + m->outLwOffset, m->hOut.lw.data(), m->hOut.lw.size() * 8, cudaMemcpyHostToDevice));
   }
+  if (m->T) MB_CUDA (cudaMemcpy ((char*) m->dBlob + m->lwOffset, m->lw.data(), (size_t) m->T * 8, cudaMemcpyHostToDevice));
   if (lane_update_weights (m) || col_update_weights (m)) return 1;
   const int rc = big_update_weights (m);
   if (rc == 2) {      // the new weights' ratios changed which insert groups are proportional: generate the big engine again
@@ -557,6 +581,8 @@ void mb_batch_destroy (mb_batch* b) {
   pooled_free (b->device, b->dTokBlock, b->tokBytes);
   pooled_free (b->device, b->viterbiPaths.dPaths, b->viterbiPaths.pathsBytes);
   pooled_free (b->device, b->sampledPaths.dPaths, b->sampledPaths.pathsBytes);
+  pooled_free (b->device, b->meaPaths.dPaths, b->meaPaths.pathsBytes);
+  pooled_free (b->device, b->dMeaPost, b->meaPostBytes);
   ws_release_all (b);
   if (b->copyStream) { cudaStreamSynchronize (b->copyStream); cudaStreamDestroy (b->copyStream); }
   if (b->evCopy) cudaEventDestroy (b->evCopy);
@@ -588,15 +614,15 @@ static int check_call (const mb_machine* m, const mb_batch* b) {
   return 0;
 }
 
-enum Pass { PASS_FORWARD, PASS_VITERBI_PATHS, PASS_VITERBI_SCORES, PASS_BACKWARD, PASS_COUNTS, PASS_MATRIX, PASS_SAMPLE, PASS_PAIR_COUNTS };
+enum Pass { PASS_FORWARD, PASS_VITERBI_PATHS, PASS_VITERBI_SCORES, PASS_BACKWARD, PASS_COUNTS, PASS_MATRIX, PASS_SAMPLE, PASS_PAIR_COUNTS, PASS_MEA, PASS_PATH_POST };
 enum Route { ROUTE_ERROR = -1, ROUTE_NONE, ROUTE_JIT, ROUTE_BIG, ROUTE_COL, ROUTE_LANE, ROUTE_WIDE, ROUTE_GENERIC };
 
 // The engine that serves a call, after any lazy preparation it needs (ROUTE_NONE: nothing to do; ROUTE_ERROR: a preparation
 // failed, error set).  A failed preparation destroys what it built, so the engine's handle is null again.
 static int route_of (mb_machine* m, mb_batch* b, Pass pass) {
   const bool sweep = pass == PASS_FORWARD || pass == PASS_VITERBI_PATHS || pass == PASS_VITERBI_SCORES;
-  // stored matrices (a pair's whole matrix, sampled paths) exist only in the generic engine
-  if (pass == PASS_MATRIX || pass == PASS_SAMPLE || m->engine == MB_ENGINE_GENERIC) return ROUTE_GENERIC;
+  // stored matrices (a pair's whole matrix, sampled paths, posterior decoding) exist only in the generic engine
+  if (pass == PASS_MATRIX || pass == PASS_SAMPLE || pass == PASS_MEA || pass == PASS_PATH_POST || m->engine == MB_ENGINE_GENERIC) return ROUTE_GENERIC;
   if (m->engine == MB_ENGINE_JIT) {
     // the strip kernels sweep full matrices; with envelopes the wide engine takes the sweeps it can, the generic engine the rest
     if (!b->hasEnv) return ROUTE_JIT;
@@ -635,7 +661,7 @@ static int route_of (mb_machine* m, mb_batch* b, Pass pass) {
 static int route (mb_machine* m, mb_batch* b, Pass pass) {
   const int r = route_of (m, b, pass);
   if (r != ROUTE_ERROR && m->opt.get ("verbose", 0)) {
-    static const char* const passNames[] = { "mb_forward", "mb_viterbi", "mb_viterbi (scores)", "mb_backward", "mb_counts", "mb_matrix", "mb_sample_paths", "mb_pair_counts" };
+    static const char* const passNames[] = { "mb_forward", "mb_viterbi", "mb_viterbi (scores)", "mb_backward", "mb_counts", "mb_matrix", "mb_sample_paths", "mb_pair_counts", "mb_mea", "mb_path_posteriors" };
     static const char* const engineNames[] = { "no engine (empty batch)", "jit engine", "big engine", "column engine", "lane engine", "wide engine", "generic engine" };
     fprintf (stderr, "%s: %s\n", passNames[pass], engineNames[r]);
   }
@@ -836,6 +862,69 @@ int mb_sampled_paths (mb_batch* b, void* pathTrans, int32_t bytesPerId, const in
   if (bytesPerId != 1 && bytesPerId != 2 && bytesPerId != 4) { set_error ("mb_sampled_paths: bytesPerId must be 1, 2 or 4"); return 1; }
   if (bytesPerId < 4 && ps.pathIdLimit > (bytesPerId == 1 ? 256 : 65536)) { set_error ("mb_sampled_paths: the machine's transition ids do not fit in " + std::to_string (bytesPerId) + " byte(s)"); return 1; }
   return copy_paths (b, ps, pathTrans, bytesPerId, pathOff);
+}
+
+int mb_mea (mb_machine* m, mb_batch* b, double* gain, double* loglike, int64_t* pathLen) {
+  if (check_call (m, b)) return 1;
+  b->meaStored = false;      // a failed call leaves no MEA paths stored
+  if (!gain) { set_error ("mb_mea: null gain"); return 1; }
+  PathStore& ps = b->meaPaths;
+  ps.pathIdLimit = m->T;
+  ps.pathStart.assign ((size_t) b->nPairs, 0);      // placed by paths_place, a path per pair
+  ps.pathLen.assign ((size_t) b->nPairs, 0);
+  ps.pathsPacked = 0;
+  route (m, b, PASS_MEA);
+  if (generic_mea (m, b, gain, loglike)) { ps.pathStart.clear(); ps.pathLen.clear(); return 1; }
+  b->meaStored = true;
+  if (pathLen) for (int64_t k = 0; k < b->nPairs; ++k) pathLen[k] = ps.pathLen[k];
+  return 0;
+}
+
+int mb_mea_paths (mb_batch* b, void* pathTrans, int32_t bytesPerId, const int64_t* pathOff, double* stepPost) {
+  if (!b) { set_error ("null batch"); return 1; }
+  const PathStore& ps = b->meaPaths;
+  if (!b->meaStored) { set_error ("mb_mea_paths: no MEA paths stored; call mb_mea first"); return 1; }
+  if (bytesPerId != 1 && bytesPerId != 2 && bytesPerId != 4) { set_error ("mb_mea_paths: bytesPerId must be 1, 2 or 4"); return 1; }
+  if (bytesPerId < 4 && ps.pathIdLimit > (bytesPerId == 1 ? 256 : 65536)) { set_error ("mb_mea_paths: the machine's transition ids do not fit in " + std::to_string (bytesPerId) + " byte(s)"); return 1; }
+  int64_t total = 0;
+  for (int64_t k = 0; k < b->nPairs; ++k) total += ps.pathLen[k];
+  if (!total) return 0;
+  if (!pathTrans || !pathOff) { set_error ("mb_mea_paths: null pathTrans or pathOff"); return 1; }
+  if (copy_paths (b, ps, pathTrans, bytesPerId, pathOff)) return 1;
+  if (!stepPost) return 0;
+  std::vector<double> post ((size_t) total);      // packed in pair order, as the ids
+  MB_CUDA (cudaMemcpy (post.data(), b->dMeaPost, (size_t) total * 8, cudaMemcpyDeviceToHost));
+  for (int64_t k = 0; k < b->nPairs; ++k)
+    if (ps.pathLen[k]) memcpy (stepPost + pathOff[k], post.data() + ps.pathStart[k], (size_t) ps.pathLen[k] * 8);
+  return 0;
+}
+
+int mb_path_posteriors (mb_machine* m, mb_batch* b, int64_t nPaths, const int64_t* pairOfPath,
+                        const int32_t* pathTrans, const int64_t* pathOff, const int64_t* pathLen, double* stepPost) {
+  if (check_call (m, b)) return 1;
+  if (nPaths < 0) { set_error ("mb_path_posteriors: negative path count"); return 1; }
+  if (nPaths && (!pairOfPath || !pathOff || !pathLen)) { set_error ("mb_path_posteriors: null pairOfPath, pathOff or pathLen"); return 1; }
+  // the paths come from outside: check them before anything indexes with them, and pack them in path order
+  std::vector<int64_t> off ((size_t) nPaths + 1, 0);
+  for (int64_t r = 0; r < nPaths; ++r) {
+    const std::string path = "mb_path_posteriors: path " + std::to_string (r);
+    if (pairOfPath[r] < 0 || pairOfPath[r] >= b->nPairs) { set_error (path + " belongs to pair " + std::to_string (pairOfPath[r]) + ", which is not in the batch of " + std::to_string (b->nPairs)); return 1; }
+    if (pathLen[r] < 0 || pathOff[r] < 0) { set_error (path + " has a negative length or offset"); return 1; }
+    off[r + 1] = off[r] + pathLen[r];
+  }
+  if (off[nPaths] && (!pathTrans || !stepPost)) { set_error ("mb_path_posteriors: null pathTrans or stepPost"); return 1; }
+  std::vector<int32_t> ids ((size_t) off[nPaths]);
+  for (int64_t r = 0; r < nPaths; ++r)
+    for (int64_t n = 0; n < pathLen[r]; ++n) {
+      const int32_t t = pathTrans[pathOff[r] + n];
+      if (t < 0 || t >= m->T) { set_error ("mb_path_posteriors: path " + std::to_string (r) + ", step " + std::to_string (n) + ": transition " + std::to_string (t) + " is not one of the machine's " + std::to_string (m->T)); return 1; }
+      ids[off[r] + n] = t;
+    }
+  route (m, b, PASS_PATH_POST);
+  std::vector<double> post;
+  if (generic_path_posteriors (m, b, nPaths, pairOfPath, ids, off, post)) return 1;
+  for (int64_t r = 0; r < nPaths; ++r) if (pathLen[r]) memcpy (stepPost + pathOff[r], post.data() + off[r], (size_t) pathLen[r] * 8);
+  return 0;
 }
 
 int mb_jit_compile_check (int32_t nStates, int32_t nInTok, int32_t nOutTok, int64_t nTrans,

@@ -16,6 +16,9 @@
 //   DPMatrix::traceBack        dpmatrix.defs.h:82-110 traceback_kernel
 //   ForwardMatrix::samplePath  forward.cpp:17-23      sample_kernel
 //   BackwardMatrix::getCounts  backward.cpp:62-87     counts_kernel
+//   postTransQueue / traceFrom backward.cpp:52-56,89-108  posterior decoding over stored Forward and Backward matrices:
+//                                                     mea_fill_kernel (the MEA DP), mea_traceback_kernel (its path and each
+//                                                     step's posterior), path_post_kernel (the posterior of each step of a given path)
 #include <algorithm>
 #include <cmath>
 #include <cstdio>
@@ -309,6 +312,160 @@ __global__ void __launch_bounds__(256) counts_kernel (DevMachine m, DevBatch b, 
 }
 
 // ---------------------------------------------------------------------------------------------
+// posterior decoding (definitions: include/machineboss_b200.h, mb_mea)
+// ---------------------------------------------------------------------------------------------
+// The candidates into state s at cell (i, o), a = x[i-1] (0 at i == 0), c = y[o-1] (0 at o == 0): f (incoming list entry p,
+// source inPos, source outPos, tokens consumed) in the reference's order (match, delete, insert, silent; each by source state
+// then transition index), as traceback_kernel and sample_kernel walk them.
+template<class Fn>
+__device__ __forceinline__ void for_each_incoming (const DevMachine& m, int64_t i, int64_t o, int s, int a, int c, Fn&& f) {
+  const int64_t ks = (int64_t) s * m.nIn1;
+  auto list = [&] (int64_t key, int64_t si, int64_t so, int tokens) {
+    for (int64_t p = m.inc.off[key], e = m.inc.off[key + 1]; p < e; ++p) f (p, si, so, tokens);
+  };
+  if (i && o) list ((ks + a) * m.nOut1 + c, i - 1, o - 1, 2);
+  if (i) list ((ks + a) * m.nOut1, i - 1, o, 1);
+  if (o) list (ks * m.nOut1 + c, i, o - 1, 1);
+  list (ks * m.nOut1, i, o, 0);
+}
+
+// A step's posterior gamma = exp ((F - ll) + (B + w)) from f = F(source cell)[src] and bw = B(destination cell)[dst] + w: the
+// bracketing of counts_kernel, so that gamma is bit for bit the term it adds.  Returns whether the step is admissible.
+__device__ __forceinline__ bool step_post (double f, double ll, double bw, double& gamma) {
+  const double e = (f - ll) + bw;
+  gamma = exp (e);
+  return e > neg_inf();
+}
+
+// The MEA DP over a chunk's stored Forward (wsF) and Backward (wsB) matrices, A into wsA: fill_kernel's forward wavefront and
+// silent-level sweep, one CTA per pair, cells outside the envelope -inf.  gain[k] = A(Li, Lo)[end state].
+__global__ void __launch_bounds__(256) mea_fill_kernel (DevMachine m, DevBatch b, const int64_t* __restrict__ pairs,
+                                                        const int64_t* __restrict__ wsOff, const double* __restrict__ wsF,
+                                                        const double* __restrict__ wsB, const double* __restrict__ backLL,
+                                                        double* __restrict__ wsA, double* __restrict__ gain) {
+  const int64_t k = pairs[blockIdx.x];
+  const uint8_t* x = b.x + b.xOff[k];
+  const uint8_t* y = b.y + b.yOff[k];
+  const int64_t Li = b.xOff[k + 1] - b.xOff[k], Lo = b.yOff[k + 1] - b.yOff[k];
+  const int S = m.S;
+  const Cells F = { const_cast<double*> (wsF) + wsOff[blockIdx.x], Li, S, 0 }, B = { const_cast<double*> (wsB) + wsOff[blockIdx.x], Li, S, 0 },
+              A = { wsA + wsOff[blockIdx.x], Li, S, 0 };
+  const double ninf = neg_inf(), ll = backLL[k];
+  const Env env = pair_env (b, k);
+  for (int64_t d = 0; d <= Li + Lo; ++d) {
+    const int64_t lo = d > Lo ? d - Lo : 0, hi = d < Li ? d : Li;
+    const int64_t nc = hi - lo + 1;
+    for (int l = 0; l < m.nFwdLevels; ++l) {
+      const int l0 = m.fwdLevelOff[l], ns = m.fwdLevelOff[l + 1] - l0;
+      for (int64_t item = threadIdx.x; item < nc * ns; item += blockDim.x) {
+        const int64_t i = lo + item / ns, o = d - i;
+        const int s = m.fwdLevelStates[l0 + (int) (item % ns)];
+        double acc = (i || o || s) ? ninf : 0.;
+        const double bs = B.at (i, o)[s];
+        if (env.contains (i, o) && ll > ninf && bs > ninf)
+          for_each_incoming (m, i, o, s, i ? x[i - 1] : 0, o ? y[o - 1] : 0, [&] (int64_t p, int64_t si, int64_t so, int tokens) {
+            const int src = m.inc.other[p];
+            double g;
+            if (!step_post (F.at (si, so)[src], ll, bs + m.inc.lw[p], g)) return;
+            const double v = A.at (si, so)[src] + tokens * g;
+            if (acc < v) acc = v;
+          });
+        A.at (i, o)[s] = env.contains (i, o) ? acc : ninf;
+      }
+      __syncthreads();
+    }
+  }
+  if (threadIdx.x == 0) gain[k] = env.contains (Li, Lo) ? A.at (Li, Lo)[S - 1] : ninf;
+}
+
+// The MEA path over the stored A, F and B matrices, one thread per pair of the chunk: each step rebuilds the candidates with the
+// fill's arithmetic and takes the first maximum, as the fill did.  With out == nullptr only the length is computed; otherwise the
+// path is written start -> end into out[outOff[slot] ..) and each step's gamma into outPost at the same place.
+__global__ void mea_traceback_kernel (DevMachine m, DevBatch b, const int64_t* __restrict__ pairs, int64_t nSlots, const int64_t* __restrict__ wsOff,
+                                      const double* __restrict__ wsF, const double* __restrict__ wsB, const double* __restrict__ wsA,
+                                      const double* __restrict__ backLL, const double* __restrict__ gain, int64_t* __restrict__ lenOut,
+                                      int32_t* __restrict__ out, double* __restrict__ outPost, const int64_t* __restrict__ outOff) {
+  const int64_t slot = (int64_t) blockIdx.x * blockDim.x + threadIdx.x;
+  if (slot >= nSlots) return;
+  const int64_t k = pairs[slot];
+  const uint8_t* x = b.x + b.xOff[k];
+  const uint8_t* y = b.y + b.yOff[k];
+  const int64_t Li = b.xOff[k + 1] - b.xOff[k], Lo = b.yOff[k + 1] - b.yOff[k];
+  const int S = m.S;
+  const Cells F = { const_cast<double*> (wsF) + wsOff[slot], Li, S, 0 }, B = { const_cast<double*> (wsB) + wsOff[slot], Li, S, 0 },
+              A = { const_cast<double*> (wsA) + wsOff[slot], Li, S, 0 };
+  const double ninf = neg_inf(), ll = backLL[k];
+  int64_t n = 0;
+  if (gain[k] > ninf) {
+    const int64_t total = out ? lenOut[slot] : 0;
+    int64_t i = Li, o = Lo;
+    int s = S - 1;
+    while (i > 0 || o > 0 || s != 0) {
+      const double bs = B.at (i, o)[s];
+      double best = ninf, bestG = 0;
+      int64_t bestP = -1, bi = 0, bo = 0;
+      for_each_incoming (m, i, o, s, i ? x[i - 1] : 0, o ? y[o - 1] : 0, [&] (int64_t p, int64_t si, int64_t so, int tokens) {
+        const int src = m.inc.other[p];
+        double g;
+        if (!step_post (F.at (si, so)[src], ll, bs + m.inc.lw[p], g)) return;
+        const double v = A.at (si, so)[src] + tokens * g;
+        if (best < v) { best = v; bestG = g; bestP = p; bi = si; bo = so; }
+      });
+      if (bestP < 0) break;   // cannot happen for a finite gain
+      if (out) {
+        if (n >= total) break;   // cannot happen: the walk replays the length pass's
+        out[outOff[slot] + total - 1 - n] = m.inc.id[bestP];
+        outPost[outOff[slot] + total - 1 - n] = bestG;
+      }
+      ++n;
+      i = bi; o = bo; s = m.inc.other[bestP];
+    }
+  }
+  if (!out) lenOut[slot] = n;
+}
+
+// per-path outcome of path_post_kernel (the first check a step fails)
+enum { PP_OK = 0, PP_SOURCE, PP_INPUT, PP_OUTPUT, PP_ENVELOPE, PP_END };
+
+// The posterior of each step of given paths, one thread per path of the chunk: path r (pair pairOfPath[r], the chunk's pair
+// slotOfPath[r]) is ids[off[r] .. off[r + 1]), its gammas go to post at the same places.  The walk checks each step and records
+// the first one that is not a step of the pair (err[r], errStep[r]; PP_END with errStep = length when the path stops early).
+__global__ void path_post_kernel (DevMachine m, DevBatch b, const int64_t* __restrict__ chunkPaths, int64_t nChunkPaths,
+                                  const int64_t* __restrict__ slotOfPath, const int64_t* __restrict__ pairOfPath,
+                                  const int32_t* __restrict__ ids, const int64_t* __restrict__ off, const int64_t* __restrict__ wsOff,
+                                  const double* __restrict__ wsF, const double* __restrict__ wsB, const double* __restrict__ backLL,
+                                  double* __restrict__ post, int32_t* __restrict__ err, int64_t* __restrict__ errStep) {
+  const int64_t q = (int64_t) blockIdx.x * blockDim.x + threadIdx.x;
+  if (q >= nChunkPaths) return;
+  const int64_t r = chunkPaths[q], slot = slotOfPath[r], k = pairOfPath[r];
+  const uint8_t* x = b.x + b.xOff[k];
+  const uint8_t* y = b.y + b.yOff[k];
+  const int64_t Li = b.xOff[k + 1] - b.xOff[k], Lo = b.yOff[k + 1] - b.yOff[k];
+  const int S = m.S;
+  const Cells F = { const_cast<double*> (wsF) + wsOff[slot], Li, S, 0 }, B = { const_cast<double*> (wsB) + wsOff[slot], Li, S, 0 };
+  const double ninf = neg_inf(), ll = backLL[k];
+  const Env env = pair_env (b, k);
+  int64_t i = 0, o = 0, n = off[r];
+  int s = 0, code = PP_OK;
+  for (; n < off[r + 1]; ++n) {
+    const int t = ids[n], a = m.tIn[t], c = m.tOut[t], dst = m.tDst[t];
+    if (m.tSrc[t] != s) { code = PP_SOURCE; break; }
+    if (a && (i >= Li || x[i] != a)) { code = PP_INPUT; break; }
+    if (c && (o >= Lo || y[o] != c)) { code = PP_OUTPUT; break; }
+    const int64_t ni = i + (a ? 1 : 0), no = o + (c ? 1 : 0);
+    if (!env.contains (ni, no)) { code = PP_ENVELOPE; break; }
+    // a silent transition that does not advance (only possible on state 0) never contributes to the DP (build_csr): gamma 0
+    double g = 0;
+    if (ll > ninf && (a || c || dst > s)) step_post (F.at (i, o)[s], ll, B.at (ni, no)[dst] + m.tLw[t], g);
+    post[n] = g;
+    i = ni; o = no; s = dst;
+  }
+  if (code == PP_OK && !(i == Li && o == Lo && s == S - 1)) code = PP_END;
+  err[r] = code;
+  errStep[r] = n - off[r];
+}
+
+// ---------------------------------------------------------------------------------------------
 // host side: chunk the batch so that the cell storage of a chunk fits in free device memory
 // ---------------------------------------------------------------------------------------------
 struct Chunk {
@@ -498,6 +655,111 @@ int generic_counts (mb_machine* m, mb_batch* b, double* counts, double* loglike,
   b->lastLaunches = launches;
   if (loglike) MB_CUDA (cudaMemcpy (loglike, dF.p, (size_t) b->nPairs * 8, cudaMemcpyDeviceToHost));
   if (counts && !rows) MB_CUDA (cudaMemcpy (counts, dCounts.p, (size_t) m->T * 8, cudaMemcpyDeviceToHost));
+  return 0;
+}
+
+// Per chunk: the Forward and Backward fills into full storage, the MEA fill into a third matrix, then generic_viterbi's length
+// pass / placement / id pass, the id pass also writing each step's gamma into b->dMeaPost.
+int generic_mea (mb_machine* m, mb_batch* b, double* gain, double* loglike) {
+  b->lastMs = 0;
+  b->lastLaunches = 0;
+  if (b->nPairs == 0) return 0;
+  std::vector<Chunk> chunks;
+  if (plan_chunks (b, m->S, false, 3, chunks)) return 1;
+  DevBuf dF, dB, dGain;
+  if (dF.alloc ((size_t) b->nPairs * 8) || dB.alloc ((size_t) b->nPairs * 8) || dGain.alloc ((size_t) b->nPairs * 8)) return 1;
+  int64_t launches = 0;
+  double ms = 0;
+  for (auto& ch: chunks) {
+    const int64_t nSlots = (int64_t) ch.pairs.size();
+    DevBuf dPairs, dOff, dWsF, dWsB, dWsA, dLen, dOutOff;
+    if (upload (dPairs, ch.pairs, b->stream) || upload (dOff, ch.wsOff, b->stream) || dWsF.alloc ((size_t) ch.doubles * 8)
+        || dWsB.alloc ((size_t) ch.doubles * 8) || dWsA.alloc ((size_t) ch.doubles * 8) || dLen.alloc ((size_t) nSlots * 8)
+        || dOutOff.alloc ((size_t) nSlots * 8)) return 1;
+    const unsigned grid = (unsigned) nSlots, tg = (unsigned) ((nSlots + 63) / 64);
+    if (timing_begin (b)) return 1;
+    fill_kernel<OP_SUM, false><<<grid, 256, 0, b->stream>>> (m->dev, b->dev, dPairs.as<int64_t>(), dOff.as<int64_t>(), dWsF.as<double>(), 0, dF.as<double>());
+    fill_kernel<OP_SUM, true><<<grid, 256, 0, b->stream>>> (m->dev, b->dev, dPairs.as<int64_t>(), dOff.as<int64_t>(), dWsB.as<double>(), 0, dB.as<double>());
+    mea_fill_kernel<<<grid, 256, 0, b->stream>>> (m->dev, b->dev, dPairs.as<int64_t>(), dOff.as<int64_t>(), dWsF.as<double>(), dWsB.as<double>(), dB.as<double>(),
+                                                  dWsA.as<double>(), dGain.as<double>());
+    mea_traceback_kernel<<<tg, 64, 0, b->stream>>> (m->dev, b->dev, dPairs.as<int64_t>(), nSlots, dOff.as<int64_t>(), dWsF.as<double>(), dWsB.as<double>(),
+                                                    dWsA.as<double>(), dB.as<double>(), dGain.as<double>(), dLen.as<int64_t>(), nullptr, nullptr, nullptr);
+    MB_CUDA (cudaGetLastError());
+    if (paths_place (b, b->meaPaths, ch.pairs.data(), nSlots, dLen.as<int64_t>(), dOutOff.as<int64_t>()) || mea_post_reserve (b, b->meaPaths.pathsPacked)) return 1;
+    mea_traceback_kernel<<<tg, 64, 0, b->stream>>> (m->dev, b->dev, dPairs.as<int64_t>(), nSlots, dOff.as<int64_t>(), dWsF.as<double>(), dWsB.as<double>(),
+                                                    dWsA.as<double>(), dB.as<double>(), dGain.as<double>(), dLen.as<int64_t>(), b->meaPaths.dPaths, b->dMeaPost,
+                                                    dOutOff.as<int64_t>());
+    MB_CUDA (cudaGetLastError());
+    launches += 5;
+    if (timing_end (b, launches)) return 1;
+    ms += b->lastMs;
+  }
+  b->lastMs = ms;
+  b->lastLaunches = launches;
+  MB_CUDA (cudaMemcpy (gain, dGain.p, (size_t) b->nPairs * 8, cudaMemcpyDeviceToHost));
+  if (loglike) MB_CUDA (cudaMemcpy (loglike, dF.p, (size_t) b->nPairs * 8, cudaMemcpyDeviceToHost));
+  return 0;
+}
+
+// Per chunk that holds the pair of some path: the Forward and Backward fills into full storage, then path_post_kernel over that
+// chunk's paths.
+int generic_path_posteriors (mb_machine* m, mb_batch* b, int64_t nPaths, const int64_t* pairOfPath, const std::vector<int32_t>& ids,
+                             const std::vector<int64_t>& off, std::vector<double>& post) {
+  b->lastMs = 0;
+  b->lastLaunches = 0;
+  post.assign ((size_t) off[nPaths], 0.);
+  if (nPaths == 0) return 0;
+  std::vector<Chunk> chunks;
+  if (plan_chunks (b, m->S, false, 2, chunks)) return 1;
+  std::vector<int64_t> chunkOf ((size_t) b->nPairs), slotOf ((size_t) b->nPairs), slotOfPath ((size_t) nPaths), pairs (pairOfPath, pairOfPath + nPaths);
+  for (size_t c = 0; c < chunks.size(); ++c)
+    for (size_t q = 0; q < chunks[c].pairs.size(); ++q) { chunkOf[chunks[c].pairs[q]] = (int64_t) c; slotOf[chunks[c].pairs[q]] = (int64_t) q; }
+  std::vector<std::vector<int64_t>> pathsOf (chunks.size());
+  for (int64_t r = 0; r < nPaths; ++r) { pathsOf[chunkOf[pairs[r]]].push_back (r); slotOfPath[r] = slotOf[pairs[r]]; }
+  DevBuf dLL, dFLL, dSlotOfPath, dPairOfPath, dIds, dPathOff, dPost, dErr, dErrStep;
+  if (dLL.alloc ((size_t) b->nPairs * 8) || dFLL.alloc ((size_t) b->nPairs * 8) || upload (dSlotOfPath, slotOfPath, b->stream)
+      || upload (dPairOfPath, pairs, b->stream) || upload (dPathOff, off, b->stream) || dIds.alloc (ids.size() * 4)
+      || dPost.alloc (post.size() * 8) || dErr.alloc ((size_t) nPaths * 4) || dErrStep.alloc ((size_t) nPaths * 8)) return 1;
+  if (!ids.empty()) MB_CUDA (cudaMemcpyAsync (dIds.p, ids.data(), ids.size() * 4, cudaMemcpyHostToDevice, b->stream));
+  int64_t launches = 0;
+  double ms = 0;
+  for (size_t c = 0; c < chunks.size(); ++c) {
+    if (pathsOf[c].empty()) continue;
+    const Chunk& ch = chunks[c];
+    const int64_t nChunkPaths = (int64_t) pathsOf[c].size();
+    DevBuf dPairs, dOff, dWsF, dWsB, dChunkPaths;
+    if (upload (dPairs, ch.pairs, b->stream) || upload (dOff, ch.wsOff, b->stream) || upload (dChunkPaths, pathsOf[c], b->stream)
+        || dWsF.alloc ((size_t) ch.doubles * 8) || dWsB.alloc ((size_t) ch.doubles * 8)) return 1;
+    const unsigned grid = (unsigned) ch.pairs.size();
+    if (timing_begin (b)) return 1;
+    fill_kernel<OP_SUM, false><<<grid, 256, 0, b->stream>>> (m->dev, b->dev, dPairs.as<int64_t>(), dOff.as<int64_t>(), dWsF.as<double>(), 0, dFLL.as<double>());
+    fill_kernel<OP_SUM, true><<<grid, 256, 0, b->stream>>> (m->dev, b->dev, dPairs.as<int64_t>(), dOff.as<int64_t>(), dWsB.as<double>(), 0, dLL.as<double>());
+    path_post_kernel<<<(unsigned) ((nChunkPaths + 63) / 64), 64, 0, b->stream>>> (m->dev, b->dev, dChunkPaths.as<int64_t>(), nChunkPaths, dSlotOfPath.as<int64_t>(),
+                                                                                 dPairOfPath.as<int64_t>(), dIds.as<int32_t>(), dPathOff.as<int64_t>(), dOff.as<int64_t>(),
+                                                                                 dWsF.as<double>(), dWsB.as<double>(), dLL.as<double>(), dPost.as<double>(),
+                                                                                 dErr.as<int32_t>(), dErrStep.as<int64_t>());
+    MB_CUDA (cudaGetLastError());
+    launches += 3;
+    if (timing_end (b, launches)) return 1;
+    ms += b->lastMs;
+  }
+  b->lastMs = ms;
+  b->lastLaunches = launches;
+  std::vector<int32_t> err ((size_t) nPaths);
+  std::vector<int64_t> errStep ((size_t) nPaths);
+  MB_CUDA (cudaMemcpy (err.data(), dErr.p, (size_t) nPaths * 4, cudaMemcpyDeviceToHost));
+  MB_CUDA (cudaMemcpy (errStep.data(), dErrStep.p, (size_t) nPaths * 8, cudaMemcpyDeviceToHost));
+  for (int64_t r = 0; r < nPaths; ++r) {
+    if (err[r] == PP_OK) continue;
+    static const char* const what[] = { "", "transition %d does not leave the state the path is in", "transition %d does not read the pair's next input token",
+                                        "transition %d does not write the pair's next output token", "transition %d leaves the pair's envelope",
+                                        "the path ends before the end state at the end of both sequences" };
+    char msg[160];
+    snprintf (msg, sizeof msg, what[err[r]], err[r] == PP_END ? 0 : ids[off[r] + errStep[r]]);
+    set_error ("mb_path_posteriors: path " + std::to_string (r) + " (pair " + std::to_string (pairs[r]) + "), step " + std::to_string (errStep[r]) + ": " + msg);
+    return 1;
+  }
+  if (!post.empty()) MB_CUDA (cudaMemcpy (post.data(), dPost.p, post.size() * 8, cudaMemcpyDeviceToHost));
   return 0;
 }
 

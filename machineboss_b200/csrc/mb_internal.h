@@ -39,6 +39,13 @@ struct DevMachine {
   const int32_t* fwdLevelStates;
   const int32_t* bwdLevelOff;
   const int32_t* bwdLevelStates;
+  // every transition by id (mb_path_posteriors walks caller-supplied paths): source, destination, tokens, log-weight
+  int64_t nTrans;
+  const int32_t* tSrc;
+  const int32_t* tDst;
+  const int32_t* tIn;
+  const int32_t* tOut;
+  const double* tLw;
 };
 
 struct DevBatch {
@@ -116,7 +123,7 @@ struct mb_machine {
   std::vector<int32_t> fwdLevelOff, fwdLevelStates, bwdLevelOff, bwdLevelStates;
   void* dBlob = nullptr;   // one device allocation holding everything below
   size_t blobBytes = 0;
-  size_t incLwOffset = 0, outLwOffset = 0;   // byte offsets of the two weight arrays inside the blob
+  size_t incLwOffset = 0, outLwOffset = 0, lwOffset = 0;   // byte offsets of the three weight arrays inside the blob
   mb::DevMachine dev {};
 
   // jit engine (mb_jit.cu)
@@ -163,6 +170,11 @@ struct mb_batch {
   mb::PathStore viterbiPaths;          // result of the last mb_viterbi with traceback, a path per pair
   mb::PathStore sampledPaths;          // result of the last mb_sample_paths, path k * nSamples + j
   int32_t samplesPerPair = 0;          // nSamples of that call (0: no samples stored)
+  mb::PathStore meaPaths;              // result of the last mb_mea, a path per pair
+  double* dMeaPost = nullptr;          // posterior of each step of meaPaths, at the same offsets (pooled; meaPostCapacity entries)
+  int64_t meaPostCapacity = 0;
+  size_t meaPostBytes = 0;
+  bool meaStored = false;              // the last mb_mea succeeded
 };
 
 namespace mb {
@@ -176,6 +188,13 @@ int generic_counts (mb_machine* m, mb_batch* b, double* counts, double* loglike,
 int generic_matrix (mb_machine* m, mb_batch* b, int64_t pair, int kind, double* cells);
 // nSamples paths per pair drawn from the stored Forward matrices into b->sampledPaths (pathLen / pathStart set by the caller's size)
 int generic_sample_paths (mb_machine* m, mb_batch* b, int32_t nSamples, uint64_t seed, double* loglike);
+// the maximum expected accuracy path of every pair into b->meaPaths and its step posteriors into b->dMeaPost (pathLen / pathStart
+// set by the caller's size); gain[k] its gain, loglike[k] (may be null) the Forward log-likelihood
+int generic_mea (mb_machine* m, mb_batch* b, double* gain, double* loglike);
+// posterior of each step of nPaths given paths: path r of pair pairOfPath[r] is ids[off[r] .. off[r + 1]) (packed), its step
+// posteriors go to post[off[r] ..); a path that is not a path of its pair is an error naming the path and the step
+int generic_path_posteriors (mb_machine* m, mb_batch* b, int64_t nPaths, const int64_t* pairOfPath, const std::vector<int32_t>& ids,
+                             const std::vector<int64_t>& off, std::vector<double>& post);
 
 // ---- jit engine (mb_jit.cu) ----
 bool jit_supported (const mb_machine* m, std::string* why);
@@ -254,6 +273,7 @@ size_t ws_bytes (const mb_batch* b, int slot);
 size_t ws_pool_bytes (int device);
 bool ws_pool_fits (int device, size_t bytes);   // a pooled block would serve this request   // freed blocks kept for reuse; released when an allocation fails
 int paths_reserve (mb_batch* b, PathStore& ps, int64_t need);   // room for `need` packed path entries in ps.dPaths (pooled; keeps the content)
+int mea_post_reserve (mb_batch* b, int64_t need);   // room for `need` step posteriors in b->dMeaPost (pooled; keeps the content)
 // paths rows[0..n) of the store (a pair's index for Viterbi paths), after those the call has placed so far: copies their lengths
 // (dLen, device) to the host, sets pathStart / pathLen, grows dPaths to hold them and writes each path's start into dOutOff
 // (device) for the id pass

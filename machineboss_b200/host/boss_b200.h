@@ -956,6 +956,55 @@ inline vector<vector<MachinePath> > posteriorPaths (const EvaluatedMachine& m, c
   return paths;
 }
 
+// The maximum expected accuracy path of each pair, computed for the whole list on the device (mb_mea; definitions in
+// include/machineboss_b200.h): (*gain)[k] its gain (-inf, with an empty path, for a pair without a path), (*stepPost)[k] the
+// posterior probability of each of its steps, (*loglike)[k] the Forward log-likelihood.  One device, like posteriorPaths.
+inline vector<MachinePath> meaPaths (const EvaluatedMachine& m, const SeqPairList& l, vector<double>* gain = nullptr,
+                                     vector<vector<double> >* stepPost = nullptr, vector<double>* loglike = nullptr) {
+  const size_t n = l.seqPairs.size();
+  DeviceBatch b (m, pairPointers (l));
+  vector<double> g (n ? n : 1), ll (n ? n : 1);
+  vector<int64_t> len (n ? n : 1), off (n + 1, 0);
+  mbCheck (mb_mea (m.handle(), b.handle(), g.data(), ll.data(), len.data()));
+  for (size_t k = 0; k < n; ++k) off[k + 1] = off[k] + len[k];
+  vector<int32_t> ids ((size_t) off[n] ? (size_t) off[n] : 1);
+  vector<double> post (ids.size());
+  if (off[n]) mbCheck (mb_mea_paths (b.handle(), ids.data(), 4, off.data(), post.data()));
+  if (gain) gain->assign (g.begin(), g.begin() + n);
+  if (loglike) loglike->assign (ll.begin(), ll.begin() + n);
+  if (stepPost) stepPost->assign (n, vector<double>());
+  vector<MachinePath> paths (n);
+  for (size_t k = 0; k < n; ++k)
+    for (int64_t q = off[k]; q < off[k + 1]; ++q) {
+      paths[k].trans.push_back (m.transition (ids[q]));
+      if (stepPost) (*stepPost)[k].push_back (post[q]);
+    }
+  return paths;
+}
+
+// The posterior probability of each step of paths[k], a path of pair k of the list (mb_path_posteriors), one vector per path.
+// One device.
+inline vector<vector<double> > pathPosteriors (const EvaluatedMachine& m, const SeqPairList& l, const vector<MachinePath>& paths) {
+  if (paths.size() != l.seqPairs.size()) throw runtime_error ("pathPosteriors: one path per pair of the list");
+  const size_t n = paths.size();
+  vector<vector<double> > out (n);
+  if (!n) return out;
+  DeviceBatch b (m, pairPointers (l));
+  vector<int64_t> pairOf (n), off (n), len (n);
+  vector<int32_t> ids;
+  for (size_t k = 0; k < n; ++k) {
+    pairOf[k] = (int64_t) k;
+    off[k] = (int64_t) ids.size();
+    for (const auto& t: paths[k].trans) ids.push_back ((int32_t) t.id);
+    len[k] = (int64_t) ids.size() - off[k];
+  }
+  vector<double> post (ids.size() ? ids.size() : 1);
+  if (ids.empty()) ids.push_back (0);
+  mbCheck (mb_path_posteriors (m.handle(), b.handle(), (int64_t) n, pairOf.data(), ids.data(), off.data(), len.data(), post.data()));
+  for (size_t k = 0; k < n; ++k) out[k].assign (post.begin() + off[k], post.begin() + off[k] + len[k]);
+  return out;
+}
+
 // The MachineCounts of each pair of the list on its own, in list order, from one device call (mb_pair_counts; dealt over the
 // box's GPUs like MachineCounts over a list): element k is MachineCounts (m, pair k), its loglike pair k's log-likelihood.
 inline vector<MachineCounts> pairCounts (const EvaluatedMachine& m, const SeqPairList& l) {

@@ -21,6 +21,11 @@
 //   --sample-paths SEED   one path per pair drawn from the posterior, ForwardMatrix::samplePath (forward.cpp:17-23)
 //   --posterior-paths N [--posterior-seed S]   N paths per pair drawn from the posterior for the whole list at once on the
 //                   device (posteriorPaths, default seed 1): [[[transition ids], ...N], ...], [] for a pair without a path
+//   --mea           maximum expected accuracy paths for the whole list on the device (meaPaths), one object per pair in list
+//                   order: {"input":..,"output":..,"gain":g,"path":[transition ids],"postProb":[posterior of each step]};
+//                   "gain":"-Infinity" and empty arrays for a pair that cannot be tokenised or has no path
+//   --viterbi-post-prob   per pair, the posterior probability of each step of its Viterbi path (pathPosteriors):
+//                   [[p, ...], ...], [] for a pair without one
 //                   (boss -C prints PARAMETER counts, which needs the symbolic weight derivatives
 //                   of the Machine -- outside this path; see INTEGRATION.md)
 //   data: -D/--data pairs.json (a SeqPairList) | --input-fasta X --output-fasta Y |
@@ -93,6 +98,7 @@ int main (int argc, char** argv) {
     string envMode;
     long long sampleSeed = 1;
     int posteriorN = 0;
+    bool doMea = false, doViterbiPost = false;
     unsigned long long posteriorSeed = 1;
     int postTransTop = 0;
     bool doDownsample = false;
@@ -128,6 +134,8 @@ int main (int argc, char** argv) {
       else if (f == "--sample-paths") { doSample = true; sampleSeed = atoll (next().c_str()); }
       else if (f == "--posterior-paths") { posteriorN = atoi (next().c_str()); if (posteriorN < 1) throw runtime_error ("--posterior-paths needs a count of at least 1"); }
       else if (f == "--posterior-seed") posteriorSeed = strtoull (next().c_str(), nullptr, 10);
+      else if (f == "--mea") doMea = true;
+      else if (f == "--viterbi-post-prob") doViterbiPost = true;
       else if (f == "--downsample-size") { doDownsample = true; downsampleSize = atof (next().c_str()); }      // boss.cpp:487-490: which transitions Machine::downsample keeps
       else if (f == "--downsample-prob") { doDownsample = true; downsampleProb = atof (next().c_str()); }
       else if (f == "--downsample-path") { doDownsample = true; downsamplePaths = atoi (next().c_str()); }      // boss.cpp:491-493: sample this many paths (seed: --seed)
@@ -259,7 +267,7 @@ int main (int argc, char** argv) {
     for (const auto& i: inSeqs) for (const auto& o: outSeqs) { SeqPair sp; sp.input = i; sp.output = o; data.seqPairs.push_back (sp); }
     if (data.seqPairs.empty() && inputEmpty && outputEmpty) data.seqPairs.push_back (SeqPair());   // boss.cpp:769-770
     if (data.seqPairs.empty()) throw runtime_error ("no sequence data given");
-    if (!(doL || doV || doA || doC || doT || doSample || posteriorN || postTransTop)) throw runtime_error ("nothing to do: give -L, -V, -A, -C or -T");
+    if (!(doL || doV || doA || doC || doT || doSample || posteriorN || doMea || doViterbiPost || postTransTop)) throw runtime_error ("nothing to do: give -L, -V, -A, -C or -T");
     if (perPair && !doC) throw runtime_error ("--per-pair goes with -C");
 
     if (doT) {   // boss.cpp:776-787
@@ -414,6 +422,54 @@ int main (int argc, char** argv) {
         cout << "]";
       }
       cout << "]\n";
+    }
+    if (doMea || doViterbiPost) {   // the whole list in one device call; pairs that cannot be tokenised have no path
+      vector<int> okAt (data.seqPairs.size(), -1);
+      for (size_t q = 0; q < okIndex.size(); ++q) okAt[okIndex[q]] = (int) q;
+      cout.precision (17);
+      auto printList = [&] (const vector<double>& v) { cout << "["; size_t n = 0; for (double p: v) cout << (n++ ? "," : "") << p; cout << "]"; };
+      if (doMea) {
+        vector<double> gain;
+        vector<vector<double> > post;
+        const vector<MachinePath> paths = meaPaths (eval, ok, &gain, &post);
+        cout << "[";
+        size_t k = 0;
+        for (const auto& sp: data.seqPairs) {
+          const int q = okAt[k];
+          const bool has = q >= 0 && gain[q] > ninf;
+          cout << (k++ ? ",\n " : "") << "{\"input\":\"" << Json::escape (sp.input.name) << "\",\"output\":\"" << Json::escape (sp.output.name)
+               << "\",\"gain\":";
+          if (has) cout << gain[q]; else cout << toInfinitySafeString (ninf);
+          cout << ",\"path\":[";
+          size_t n = 0;
+          if (has) for (const auto& t: paths[q].trans) cout << (n++ ? "," : "") << t.id;
+          cout << "],\"postProb\":";
+          printList (has ? post[q] : vector<double>());
+          cout << "}";
+        }
+        cout << "]\n";
+      }
+      if (doViterbiPost) {
+        vector<MachinePath> vpaths;
+        const vector<double> sc = viterbiLogLikes (eval, ok, &vpaths);
+        SeqPairList withPath;      // pairs without a Viterbi path have no steps to score
+        vector<MachinePath> found;
+        vector<int> foundAt (ok.seqPairs.size(), -1);
+        size_t q = 0;
+        for (const auto& sp: ok.seqPairs) {
+          if (sc[q] > ninf) { foundAt[q] = (int) found.size(); withPath.seqPairs.push_back (sp); found.push_back (vpaths[q]); }
+          ++q;
+        }
+        const vector<vector<double> > post = pathPosteriors (eval, withPath, found);
+        cout << "[";
+        for (size_t k = 0; k < data.seqPairs.size(); ++k) {
+          const int f = okAt[k] >= 0 ? foundAt[okAt[k]] : -1;
+          cout << (k ? ",\n " : "");
+          printList (f >= 0 ? post[f] : vector<double>());
+        }
+        cout << "]\n";
+      }
+      cout.precision (6);
     }
     if (doA || doV) {
       vector<MachinePath> paths;
